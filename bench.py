@@ -14,6 +14,12 @@ Prints ONE JSON line (rank 0).  `value` is measured with the batch already resid
 measurement through the public API with HOST (pinned) inputs: host->device copies and the device->host read of the
 loss sit inside the timed region.  `--impl reference` times the CPU reference implementation (the torch / C oracle,
 all host threads) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step computed (the training step's predictions, losses, gradient and
+updated parameters; the heatmap grids) as DIR/<name>.npy.  Every input is seeded, so two builds run with the same
+arguments can be compared output for output.  Each timed training step starts from the same parameters and optimizer
+state (TrainLeg.step_resident), so from run to run the predictions repeat and the losses, gradient and parameters differ
+only by the summation order of fp32 atomics; the heatmap grids are exact.
 """
 from __future__ import annotations
 
@@ -234,6 +240,7 @@ class TrainLeg:
         self.flat = FlatParams(self.model)
         self.reducer = GradReducer(self.flat)
         self.opt = FusedAdamW(self.flat, lr=1e-3, max_grad_norm=1.0)
+        self.start = self.flat.flat.clone()
         x_host, tgt_host = synth.make_sample(batch, seq_len, MAX_OBJECTS, seed=seed_base + rank)
         self.x_host = x_host.pin_memory()
         self.tgt_host = {k: v.pin_memory() for k, v in tgt_host.items()}
@@ -242,17 +249,30 @@ class TrainLeg:
         self.loss_host = torch.zeros(6).pin_memory()
         self.prefetch = HostBatchPrefetcher("cuda")
         self.h2d_bytes = self.x_host.numel() * 4 + sum(v.numel() * v.element_size() for v in self.tgt_host.values())
+        self.keep_outputs = False          # True: self.last holds the predictions and losses of the latest step
+        self.last = None
 
     def step(self, x, tgt):
         self.flat.zero_grad()
         self.reducer.prepare()
-        losses = self.model.compute_loss(self.model(x), tgt)
+        pred = self.model(x)
+        losses = self.model.compute_loss(pred, tgt)
         losses["total"].backward()
         self.reducer.finish()
         self.opt.step(grad_scale=1.0 / self.world)
+        if self.keep_outputs:
+            self.last = {"pred": {k: v.detach() for k, v in pred.items()}, "loss": {k: v.detach() for k, v in losses.items()}}
         return losses["total"]
 
     def step_resident(self):
+        # Every resident step starts from the initial parameters and optimizer state: it runs a training step's kernels on
+        # the same shapes, and what it computes depends on the seeded inputs alone.  Chained steps would not be reproducible:
+        # the weight gradients end in fp32 atomic sums, and a few steps later the bf16 forward pass has turned that
+        # summation-order noise in the parameters into visibly different predictions.
+        self.flat.flat.copy_(self.start)
+        self.opt.m.zero_()
+        self.opt.v.zero_()
+        self.opt.t = 0
         self.step(self.x_dev, self.tgt_dev)
 
     def step_e2e(self):
@@ -327,6 +347,34 @@ def invariance_check(world, rank):
     return out
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_TRACES = 65536                    # per-trace outputs of a larger batch: a fixed, seeded sample of this many traces
+
+
+def train_outputs(leg):
+    """What the last timed training step computed, as float32 arrays: the predictions and losses its caller receives,
+    the gradient it produced and the parameters after its optimizer update."""
+    import numpy as np
+    rows = None
+    if leg.batch > DUMP_TRACES:
+        rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(leg.batch, DUMP_TRACES, replace=False))).cuda()
+    out = {f"train_{k}": v if rows is None else v[rows] for k, v in leg.last["pred"].items()}
+    out.update({f"train_loss_{k}": v for k, v in leg.last["loss"].items()})
+    out["train_grad"] = leg.flat.grad
+    out["train_params"] = leg.flat.flat
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def run_ours(args):
     import torch.distributed as dist
     from roomslam_b200 import OccupancyHeatmapBaseline, synth, _lib
@@ -352,12 +400,17 @@ def run_ours(args):
 
     # ---- training step: headline leg -----------------------------------------------------------------------
     leg = TrainLeg(B, rank, world, precision)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    leg.keep_outputs = dump is not None
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
     n0 = lib.rs_launch_count()
     ms_train = timed(leg.step_resident, args.steps, args.warmup, dist_on)
     launches_train = (lib.rs_launch_count() - n0) // (args.steps + args.warmup) * args.steps
+    if dump is not None:
+        dump.update(train_outputs(leg))
+        leg.keep_outputs, leg.last = False, None
     ms_train_e2e = timed(leg.step_e2e, args.steps, max(1, args.warmup // 2), dist_on)
     h2d_train = leg.h2d_bytes
     final_loss = float(leg.loss_host[0])
@@ -377,7 +430,7 @@ def run_ours(args):
         B_o, n_tr_o = shard_sizes(args_o, world)
         leg_o = TrainLeg(B_o, rank, world, precision)
         ms_o = timed(leg_o.step_resident, args.steps, args.warmup, dist_on)
-        ms_o_e2e = timed(leg_o.step_e2e, max(2, args.steps // 2), 2, dist_on)
+        ms_o_e2e = timed(leg_o.step_e2e, args.steps, 2, dist_on)
         leg_o.free()
         del leg_o
         other_leg = {"scaling": other, "global_batch": B_o * world, "batch_per_gpu": B_o, "value": B_o * world / (ms_o / 1e3),
@@ -387,7 +440,7 @@ def run_ours(args):
     c1 = drop = None
     if not dist_on:
         c1_leg = TrainLeg(32, 0, 1, "fp32")
-        ms_c1 = timed(c1_leg.step_resident, max(args.steps, 10), 3, False)
+        ms_c1 = timed(c1_leg.step_resident, args.steps, 3, False)
         c1_leg.free()
         del c1_leg
         c1 = {"workload": "BASELINE config 1: batch 32 x 500 steps, fp32 kernels (1e-4 parity mode), fwd+loss+bwd+clip+AdamW",
@@ -404,7 +457,7 @@ def run_ours(args):
     c4 = None
     if not dist_on and not args.skip_c4:
         c4_leg = TrainLeg(1024, 0, 1, "bf16", hidden=256, seq_len=4000)
-        ms_c4 = timed(c4_leg.step_resident, 3, 2, False)
+        ms_c4 = timed(c4_leg.step_resident, args.steps, 2, False)
         F_.enable_kernel_timing(True)
         c4_leg.step_resident()
         torch.cuda.synchronize()
@@ -415,7 +468,7 @@ def run_ours(args):
         c4_flops = gru_flops_per_trace(T=4000, H=256)
         c4 = {"workload": "BASELINE config 4: bi-GRU H=256 L=2 seq_len=4000, batch 1024, bf16, fwd+loss+bwd+clip+AdamW "
                           "(W_hh streamed from L2 by the recurrence kernels, csrc/rec_wide.cu)",
-              "value": 1024 / (ms_c4 / 1e3), "unit": "traces/s", "ms_per_step": ms_c4, "steps": 3, "warmup": 2,
+              "value": 1024 / (ms_c4 / 1e3), "unit": "traces/s", "ms_per_step": ms_c4, "steps": args.steps, "warmup": 2,
               "algorithmic_gflop_per_trace": c4_flops / 1e9, "flop_bound_ms": c4_flops * 1024 / (pk["tflops_sustained"] * 1e12) * 1e3,
               "frac_of_flop_bound": c4_flops * 1024 / (pk["tflops_sustained"] * 1e12) * 1e3 / ms_c4,
               "kernel_ms": {k: v[0] for k, v in c4_kernels.items()}}
@@ -438,6 +491,11 @@ def run_ours(args):
     n1 = lib.rs_launch_count()
     ms_heat = timed(heat_resident, args.steps, args.warmup, dist_on)
     launches_heat = (lib.rs_launch_count() - n1) // (args.steps + args.warmup) * args.steps
+    if dump is not None:              # int32 counts: float64 holds every value exactly
+        grids = packed.view(2, hm.gy, hm.gx) if dist_on else torch.stack([occ, stat])
+        dump["heatmap_occupancy"] = grids[0].double().cpu().numpy()
+        dump["heatmap_stationary"] = grids[1].double().cpu().numpy()
+        dump["heatmap_dropped"] = dropped.double().cpu().numpy()
     # the binning kernel alone (events around the single launch, same stream)
     ms_kernel = timed(lambda: hm.bin_into(pts, occ, stat, dropped), args.steps, 1, False)
     conserved = int(occ.sum().item()) + int(dropped.item()) == n_tr * SEQ_LEN
@@ -453,7 +511,7 @@ def run_ours(args):
             dist.all_reduce(both, op=dist.ReduceOp.SUM)
             both.cpu()
 
-    ms_heat_e2e = timed(heat_e2e, max(1, min(args.steps, 3)), 1, dist_on)
+    ms_heat_e2e = timed(heat_e2e, args.steps, 1, dist_on)
     del pts_host
     heat_other = None
     if dist_on:
@@ -520,6 +578,8 @@ def run_ours(args):
             line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")}
             line["c1"]["cpu_same_config"] = {"value": cb["value"], "unit": "traces/s", "ratio": line["c1"]["value"] / cb["value"]}
             line["heatmap"]["cpu_baseline"] = cpu_heatmap_baseline()
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if dist_on:
         dist.barrier()
@@ -739,7 +799,14 @@ def main():
     ap.add_argument("--skip-c4", action="store_true", help="skip the BASELINE config 4 leg (H 256, T 4000; ~63 GB of HBM)")
     ap.add_argument("--suite", default="headline", choices=["headline", "next"],
                     help="'next': one JSON line per SURVEY.md 8(f) row instead of the headline line (single GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed training step and heatmap pass computed to DIR/<name>.npy (rank 0's "
+                         "shard; float32, float64 for the heatmap counts; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.suite != "headline"):
+        ap.error("--dump-outputs applies to the GPU headline run (--impl ours --suite headline)")
     # Native libraries write banners to file descriptor 1 (NCCL prints its version at the first communicator init).
     # The contract is ONE JSON line on stdout: keep Python's stdout on the real descriptor and point fd 1 at stderr.
     sys.stdout.flush()
