@@ -27,6 +27,12 @@ const char* rs_last_error(void);       /* thread-local message of the last faili
 int rs_abi_version(void);              /* bumped on any signature change */
 int rs_device_ok(void);                /* 1 when the current CUDA device is sm_100 (B200), else 0 */
 int64_t rs_launch_count(void);         /* kernels launched by this library so far (process-wide) */
+/* Deterministic mode (process-wide, default off).  On: every reduction the library splits over CTAs stores per-split
+ * partials into a workspace allocated in stream order on the call's stream (cudaMallocAsync) and adds them onto the output
+ * in a fixed order, and the split depends on the shape only, so repeated calls on the same inputs give the same bits.
+ * Off: split reductions end in floating-point atomics.  The Python binding follows torch.use_deterministic_algorithms. */
+int rs_set_deterministic(int on);      /* returns 0 */
+int rs_deterministic(void);            /* 1 when deterministic mode is on, else 0 */
 
 /* ---- occupancy heatmap + stationary time (replaces README.md:15,163-164 `src/models/baseline.py`) ------- */
 /* points: float32 [n_traces, seq_len, 2].  occ, stat: int32 [gy, gx].  n_dropped: one uint64.
@@ -100,7 +106,8 @@ int rs_loss_bwd_f32(const double* sums6, const float* d_losses6, int B, int N, i
 /* ---- bf16 tensor-core GEMMs (tcgen05 + TMEM accumulators, TMA-fed): the time-parallel work of the bf16 mode ---- */
 /* C[M,N] (ldc) = act(A[M,K] (bf16, lda) . B[N,K]^T (bf16, ldb) + bias[N] (fp32, optional)).  K % 64 == 0, N % 128 == 0,
  * leading dimensions in elements and multiples of 8.  flags: RS_GEMM_RELU, RS_GEMM_OUT_F32 (C is fp32 and written
- * with direct row stores; default: bf16 through TMA stores).  TMA-fed tcgen05: the decoder MLP of the bf16 mode. */
+ * with direct row stores; default: bf16 through TMA stores).  TMA-fed tcgen05: the decoder MLP of the bf16 mode.
+ * With RS_GEMM_OUT_F32, C and bias are accessed as float4: both 16-byte aligned, ldc % 4 == 0. */
 int rs_gemm_bf16_nt(const void* A, int64_t lda, const void* B, int64_t ldb, void* C, int64_t ldc, const float* bias,
                     int64_t M, int N, int K, int flags, void* stream);
 /* C[M,N] (fp32, ldc) += A[:, a_col0:a_col0+M]^T . B[:, b_col0:b_col0+N], reduction over `rows` row pairs
@@ -112,7 +119,8 @@ int rs_gemm_bf16_tn_acc(const void* A, int64_t lda, int64_t a_rows, int a_col0, 
 
 /* fp32 [rows, cols] (ld) -> bf16 [rows, 6 * kpad] (ld_out): sixths [lo | hi | mid | mid | hi | hi] (role_b = 0, A operand) or
  * [hi | lo | mid | hi | mid | hi] (role_b = 1, B operand; smallest partial products first); hi + mid + lo = x to 24 mantissa bits, zero padded to kpad columns.
- * One rs_gemm_bf16_nt over K = 6 * kpad then yields A . B^T at fp32 accuracy ("bf16x6") at tensor-core speed. */
+ * One rs_gemm_bf16_nt over K = 6 * kpad then yields A . B^T at fp32 accuracy ("bf16x6") at tensor-core speed.
+ * With ld % 4 == 0 the rows are read as float4: x must then be 16-byte aligned. */
 int rs_split_bf16x6(const float* x, int64_t ld, int64_t rows, int cols, int kpad, int role_b, void* out, int64_t ld_out,
                     void* stream);
 

@@ -66,7 +66,26 @@ def check(rc: int, what: str) -> None:
         raise RoomSlamError(f"{what} failed (code {rc}): {msg.decode() if msg else 'unknown error'}")
 
 
+_det_flag = None     # torch.are_deterministic_algorithms_enabled, bound on the first call
+_det_mode = None     # the library's deterministic mode as last set from it
+
+
+def sync_deterministic() -> None:
+    """Brings the library's process-wide deterministic mode (rs_set_deterministic) in line with
+    torch.use_deterministic_algorithms (warn_only included): split reductions then sum per-split partials in a fixed order
+    instead of ending in floating-point atomics.  Runs before every library call, on whichever thread makes it."""
+    global _det_flag, _det_mode
+    if _det_flag is None:
+        import torch
+        _det_flag = torch.are_deterministic_algorithms_enabled
+    on = _det_flag()
+    if on != _det_mode:
+        check(load().rs_set_deterministic(int(on)), "rs_set_deterministic")
+        _det_mode = on
+
+
 def call(name: str, *args) -> None:
+    sync_deterministic()
     check(getattr(load(), name)(*args), name)
 
 

@@ -1,4 +1,4 @@
-// Library-level pieces of the C ABI: error text, device check, tensor-map encoding.
+// Library-level pieces of the C ABI: error text, device check, deterministic mode, tensor-map encoding.
 #include <stdarg.h>
 #include <string.h>
 
@@ -9,6 +9,9 @@ namespace rs {
 
 static thread_local char g_error[1024] = "";
 static unsigned long long g_launches = 0;
+static int g_deterministic = 0;
+
+bool deterministic() { return __atomic_load_n(&g_deterministic, __ATOMIC_RELAXED) != 0; }
 
 void count_launch(int n) { __atomic_fetch_add(&g_launches, (unsigned long long)n, __ATOMIC_RELAXED); }
 
@@ -83,3 +86,8 @@ extern "C" const char* rs_last_error(void) { return rs::g_error; }
 extern "C" int rs_abi_version(void) { return 1; }
 extern "C" int64_t rs_launch_count(void) { return (int64_t)__atomic_load_n(&rs::g_launches, __ATOMIC_RELAXED); }
 extern "C" int rs_device_ok(void) { return rs::check_device_sm100() == 0 ? 1 : 0; }
+extern "C" int rs_set_deterministic(int on) {
+    __atomic_store_n(&rs::g_deterministic, on ? 1 : 0, __ATOMIC_RELAXED);
+    return 0;
+}
+extern "C" int rs_deterministic(void) { return rs::deterministic() ? 1 : 0; }

@@ -38,6 +38,36 @@ int make_tmap_2d(CUtensorMap* out, const void* base, CUtensorMapDataType dtype, 
                  uint64_t inner, uint64_t outer, uint64_t row_stride_bytes, uint32_t box_inner,
                  uint32_t box_outer, CUtensorMapSwizzle swizzle);
 
+// ---- deterministic mode (rs_set_deterministic) ----------------------------------------------
+// A reduction split over CTAs then stores one partial per split into a workspace instead of adding it to the output with
+// atomics, and slot_sum adds the partials in ascending split order.  The split of a reduction may depend on the shape
+// only: kDetSplitSms stands in for the SM count wherever the default path sizes a split by num_sms().
+bool deterministic();
+constexpr int kDetSplitSms = 148;
+
+// out[r * ldo + c] = (accumulate ? out[r * ldo + c] : 0) + parts[0][r * cols + c] + parts[1][...] + ..., slot s at
+// parts + s * part_stride.  Up to kMaxSlotSums outputs of different shapes in one launch.
+template <typename T>
+struct SlotSum {
+    const T* parts;
+    T* out;
+    long long ldo;
+    int rows, cols;
+};
+constexpr int kMaxSlotSums = 64;
+template <typename T>
+int slot_sum(const SlotSum<T>* jobs, int n_jobs, int n_parts, long long part_stride, bool accumulate, cudaStream_t stream);
+
+// Workspace allocated in stream order on the call's stream and freed in stream order when it goes out of scope.
+struct StreamScratch {
+    void* p = nullptr;
+    cudaStream_t stream;
+    explicit StreamScratch(cudaStream_t s) : stream(s) {}
+    ~StreamScratch() { if (p) cudaFreeAsync(p, stream); }
+    cudaError_t alloc(size_t bytes) { return cudaMallocAsync(&p, bytes, stream); }
+    template <typename T> T* as() const { return static_cast<T*>(p); }
+};
+
 // ---- device-side PTX ------------------------------------------------------------------------
 #ifdef __CUDACC__
 

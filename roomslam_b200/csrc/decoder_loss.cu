@@ -75,6 +75,8 @@ __global__ void relu_bwd_bf16_kernel(const __nv_bfloat16* __restrict__ dy, const
 __device__ __forceinline__ float sgn(float d) { return (d > 0.0f) - (d < 0.0f); }
 
 // sums: [0] n_valid, [1] ce, [2] |dpos|, [3] |dsize|, [4] |dorient|, [5] bce   (double accumulators)
+// kDet: block b stores its six sums to sums + 6 b (summed in block order by rs::slot_sum)
+template <bool kDet>
 __global__ void __launch_bounds__(256)
 loss_fwd_kernel(const float* __restrict__ cls, const float* __restrict__ pos, const float* __restrict__ size,
                 const float* __restrict__ orient, const float* __restrict__ vlogit, const long long* __restrict__ t_cls,
@@ -125,7 +127,8 @@ loss_fwd_kernel(const float* __restrict__ cls, const float* __restrict__ pos, co
     if (threadIdx.x < 6) {
         double t = 0.0;
         for (int w = 0; w < 8; ++w) t += (double)red[threadIdx.x][w];
-        atomicAdd(&sums[threadIdx.x], t);
+        if (kDet) sums[blockIdx.x * 6 + threadIdx.x] = t;
+        else atomicAdd(&sums[threadIdx.x], t);
     }
 }
 
@@ -236,12 +239,23 @@ extern "C" int rs_loss_fwd_f32(const float* cls, const float* pos, const float* 
     RS_REQUIRE(C >= 1 && C <= kMaxClasses, "rs_loss_fwd_f32: 1 <= num_classes <= %d", kMaxClasses);
     const long long slots = (long long)B * N;
     RS_CUDA_OK(cudaMemsetAsync(sums6, 0, 6 * sizeof(double), stream));
-    if (slots > 0)
-        loss_fwd_kernel<<<blocks_for(slots), 256, 0, stream>>>(cls, pos, size, orient, vlogit,
+    rs::StreamScratch ws(stream);
+    if (slots > 0 && rs::deterministic()) {
+        const int blocks = blocks_for(slots);
+        RS_CUDA_OK(ws.alloc(sizeof(double) * 6 * blocks));
+        loss_fwd_kernel<true><<<blocks, 256, 0, stream>>>(cls, pos, size, orient, vlogit, reinterpret_cast<const long long*>(t_cls),
+                                                          t_pos, t_size, t_orient, t_valid, slots, C, ws.as<double>(), g_cls,
+                                                          g_pos, g_size, g_orient, g_valid);
+        rs::count_launch();
+        const rs::SlotSum<double> job = {ws.as<double>(), sums6, 6, 1, 6};
+        if (int rc = rs::slot_sum(&job, 1, blocks, 6, false, stream)) return rc;
+    } else if (slots > 0) {
+        loss_fwd_kernel<false><<<blocks_for(slots), 256, 0, stream>>>(cls, pos, size, orient, vlogit,
                                                               reinterpret_cast<const long long*>(t_cls), t_pos, t_size,
                                                               t_orient, t_valid, slots, C, sums6, g_cls, g_pos, g_size,
                                                               g_orient, g_valid);
                                                               rs::count_launch();
+    }
     loss_finalize_kernel<<<1, 32, 0, stream>>>(sums6, slots, losses6, weights5[0], weights5[1], weights5[2], weights5[3],
                                                weights5[4]);
                                                rs::count_launch();

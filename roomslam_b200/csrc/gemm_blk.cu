@@ -11,6 +11,8 @@
 //   blk_gemm_nt : per block m:  C_blk[:, n] = A_blk[:, kchunks] . W[n, :]^T + bias      (bf16 out, direct stores)
 //                 -> input projection P = X W_ih^T + b  and  dX = dG W_ih
 //   blk_gemm_tn : C[M, N] += sum over blocks  A_blk[:, mchunks]^T . B_blk'[:, nchunks]   (fp32 out, split over blocks)
+//                 (the split reductions end in fp32 atomics; deterministic mode stores per-split partials into a workspace
+//                 and rs::slot_sum adds them in split order, here and in blk_wgrad)
 //                 -> dW_ih, dW_hh (block of dG at t' paired with the block of h at t' -/+ 1), bias gradients (ones column)
 //
 // Warp roles: warp 0 = bulk-copy producer, warp 1 = tcgen05.mma issuer (one lane), warps 2..5 = TMEM epilogue.
@@ -340,6 +342,8 @@ struct TnParams {
     int splits, blocks_per_split;
 };
 
+// kDet: item (split, mt) stores its tile to p.C + ((split * m_tiles + mt) * 128 + row) * ldc (workspace, ldc = n_cols)
+template <bool kDet>
 __global__ void __launch_bounds__(NUM_THREADS, 1) blk_gemm_tn_kernel(const TnParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const int b_bytes = p.n_cols * 256;
@@ -409,13 +413,16 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) blk_gemm_tn_kernel(const TnPar
             rs::mbar_wait(acc_full, acc_phase);
             rs::tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-            float* crow = p.C + (long long)(p.c_row0[mt] + row) * p.ldc;
+            float* crow = p.C + (long long)((kDet ? (split * p.m_tiles + mt) * 128 : p.c_row0[mt]) + row) * p.ldc;
             for (int c0 = 0; c0 < p.n_cols; c0 += 16) {
                 uint32_t r[16];
                 rs::tmem_ld_32x32b_x16(taddr + c0, r);
                 rs::tmem_ld_wait();
 #pragma unroll
-                for (int j = 0; j < 16; ++j) atomicAdd(crow + c0 + j, __uint_as_float(r[j]));
+                for (int j = 0; j < 16; ++j) {
+                    if (kDet) crow[c0 + j] = __uint_as_float(r[j]);
+                    else atomicAdd(crow + c0 + j, __uint_as_float(r[j]));
+                }
             }
             rs::tc_fence_before();
         }
@@ -454,6 +461,7 @@ struct WgParams {
     // paired launch (cluster of 2 CTAs = roles 2 j, 2 j + 1 of a split): bit j set = the two roles read the SAME dG block, the
     // even CTA bulk-copies it once with cluster multicast into both CTAs' stages
     int paired; unsigned int share_mask;
+    long long ws_split;                 // deterministic mode: floats per split slot (role outputs point into slot 0)
 };
 
 // Paired mode.  A dG block feeds two roles (its ih role against X, its hh role against h); as single CTAs they move 96 and 64 KB
@@ -461,6 +469,8 @@ struct WgParams {
 // 12.6 GB of operands, ncu).  As a cluster of two the even CTA's producer loads the block ONCE and multicasts it into both
 // stages; it waits for both CTAs' MMAs to retire before it refills a stage (the odd CTA's tcgen05.commit arrives on both
 // empty barriers), each CTA streams its own B operand.  The shared ring keeps the pair in lockstep by construction.
+// kDet: the outputs of role r point into slot 0 of a workspace; item (split, r) stores to slot `split` (+ split * ws_split)
+template <bool kDet>
 __global__ void __launch_bounds__(NUM_THREADS, 1) blk_wgrad_kernel(const WgParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
     const int stage_bytes = 2 * PIECE_BYTES + p.max_b_bytes + 2 * CHUNK_BYTES;   // A | B | B2 (16 columns)
@@ -564,27 +574,35 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) blk_wgrad_kernel(const WgParam
             rs::mbar_wait(acc_full, acc_phase);
             rs::tc_fence_after();
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-            float* crow = R.C + (long long)row * R.ldc;
+            const long long slot = kDet ? split * p.ws_split : 0;
+            float* crow = R.C + slot + (long long)row * R.ldc;
             for (int c0 = 0; c0 < R.n_cols; c0 += 16) {
                 uint32_t r[16];
                 rs::tmem_ld_32x32b_x16(taddr + c0, r);
                 rs::tmem_ld_wait();
 #pragma unroll
-                for (int j = 0; j < 16; ++j) atomicAdd(crow + c0 + j, __uint_as_float(r[j]));
+                for (int j = 0; j < 16; ++j) {
+                    if (kDet) crow[c0 + j] = __uint_as_float(r[j]);
+                    else atomicAdd(crow + c0 + j, __uint_as_float(r[j]));
+                }
             }
             if (R.bias) {
                 uint32_t r[8];
                 rs::tmem_ld_32x32b_x8(taddr + 256, r);
                 rs::tmem_ld_wait();
-                atomicAdd(R.bias + row, __uint_as_float(r[0]));
+                if (kDet) R.bias[slot + row] = __uint_as_float(r[0]);
+                else atomicAdd(R.bias + row, __uint_as_float(r[0]));
             }
             if (R.B2) {
                 uint32_t r[16];
                 rs::tmem_ld_32x32b_x16(taddr + 272, r);
                 rs::tmem_ld_wait();
-                float* c2 = R.C2 + (long long)row * R.ldc2;
+                float* c2 = R.C2 + slot + (long long)row * R.ldc2;
 #pragma unroll
-                for (int j = 0; j < 16; ++j) atomicAdd(c2 + j, __uint_as_float(r[j]));
+                for (int j = 0; j < 16; ++j) {
+                    if (kDet) c2[j] = __uint_as_float(r[j]);
+                    else atomicAdd(c2 + j, __uint_as_float(r[j]));
+                }
             }
             rs::tc_fence_before();
         }
@@ -698,15 +716,30 @@ extern "C" int rs_blk_gemm_tn_acc(const void* A, int64_t a_cols, const int* a_mc
     }
     p.B = static_cast<const uint8_t*>(B); p.b_block_bytes = b_broadcast ? 0 : b_cols * 256; p.b_chunk0 = b_chunk0; p.n_cols = n_cols; p.b_shift = b_shift;
     p.C = C; p.ldc = ldc; p.m_tiles = m_tiles; p.tiles = tiles; p.T = T; p.Tp = T + 2;
-    int splits = num_sms() / m_tiles;
+    const bool det = rs::deterministic();
+    int splits = (det ? rs::kDetSplitSms : num_sms()) / m_tiles;
     if (splits < 1) splits = 1;
     if (splits > total) splits = (int)total;
     p.blocks_per_split = (int)((total + splits - 1) / splits);
     p.splits = (int)((total + p.blocks_per_split - 1) / p.blocks_per_split);
     const int smem = 2 * (2 * PIECE_BYTES + n_cols * 256) + 256;
-    RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_tn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const int items = p.m_tiles * p.splits;
-    blk_gemm_tn_kernel<<<items < num_sms() ? items : num_sms(), NUM_THREADS, smem, stream>>>(p);
+    const int grid = items < num_sms() ? items : num_sms();
+    if (det) {
+        rs::StreamScratch ws(stream);
+        const long long slot = (long long)m_tiles * 128 * n_cols;
+        RS_CUDA_OK(ws.alloc(sizeof(float) * p.splits * slot));
+        p.C = ws.as<float>(); p.ldc = n_cols;
+        RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_tn_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        blk_gemm_tn_kernel<true><<<grid, NUM_THREADS, smem, stream>>>(p);
+        rs::count_launch();
+        RS_CUDA_OK(cudaGetLastError());
+        rs::SlotSum<float> jobs[TN_MAX_MT];
+        for (int i = 0; i < m_tiles; ++i) jobs[i] = {ws.as<float>() + (long long)i * 128 * n_cols, C + (long long)c_row0[i] * ldc, ldc, 128, n_cols};
+        return rs::slot_sum(jobs, m_tiles, p.splits, slot, true, stream);
+    }
+    RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_tn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    blk_gemm_tn_kernel<false><<<grid, NUM_THREADS, smem, stream>>>(p);
     rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());
     return 0;
@@ -746,13 +779,37 @@ extern "C" int rs_blk_wgrad(const void* dG, int64_t a_cols, const void* ones_blo
         if (n_cols[r] > max_n) max_n = n_cols[r];
     }
     p.max_b_bytes = max_n * 256;
-    int splits = num_sms() / n_roles;
+    const bool det = rs::deterministic();
+    int splits = (det ? rs::kDetSplitSms : num_sms()) / n_roles;
     if (splits < 1) splits = 1;
     if (splits > total) splits = (int)total;
     p.blocks_per_split = (int)((total + splits - 1) / splits);
     p.splits = (int)((total + p.blocks_per_split - 1) / p.blocks_per_split);
     const int smem = 2 * (2 * PIECE_BYTES + p.max_b_bytes + 2 * CHUNK_BYTES) + 2 * CHUNK_BYTES + 256;
-    RS_CUDA_OK(cudaFuncSetAttribute(blk_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    // deterministic mode: every role output gets a dense image in each split's workspace slot; after the launch one slot_sum
+    // adds the slots onto the outputs in split order
+    rs::StreamScratch ws(stream);
+    rs::SlotSum<float> jobs[3 * WG_MAX_ROLES];
+    int n_jobs = 0;
+    if (det) {
+        long long off[3 * WG_MAX_ROLES];
+        for (int r = 0; r < n_roles; ++r) {
+            const WgRole& R = p.role[r];
+            if (R.n_cols) { off[n_jobs] = p.ws_split; jobs[n_jobs++] = {nullptr, R.C, R.ldc, 128, R.n_cols}; p.ws_split += 128LL * R.n_cols; }
+            if (R.bias) { off[n_jobs] = p.ws_split; jobs[n_jobs++] = {nullptr, R.bias, 1, 128, 1}; p.ws_split += 128; }
+            if (R.B2) { off[n_jobs] = p.ws_split; jobs[n_jobs++] = {nullptr, R.C2, R.ldc2, 128, 16}; p.ws_split += 128 * 16; }
+        }
+        RS_CUDA_OK(ws.alloc(sizeof(float) * p.splits * p.ws_split));
+        for (int j = 0; j < n_jobs; ++j) jobs[j].parts = ws.as<float>() + off[j];
+        for (int r = 0, j = 0; r < n_roles; ++r) {
+            WgRole& R = p.role[r];
+            if (R.n_cols) { R.C = ws.as<float>() + off[j++]; R.ldc = R.n_cols; }
+            if (R.bias) R.bias = ws.as<float>() + off[j++];
+            if (R.B2) R.C2 = ws.as<float>() + off[j++];
+        }
+    }
+    const auto kernel = det ? blk_wgrad_kernel<true> : blk_wgrad_kernel<false>;
+    RS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const int items = n_roles * p.splits;
     int grid = items < num_sms() ? items : num_sms();
     // paired mode: roles 2 j and 2 j + 1 form a cluster; where they name the same dG columns the block is loaded once (multicast)
@@ -770,11 +827,12 @@ extern "C" int rs_blk_wgrad(const void* dG, int64_t a_cols, const void* ones_blo
         attr[0].id = cudaLaunchAttributeClusterDimension;
         attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
         cfg.attrs = attr; cfg.numAttrs = 1;
-        RS_CUDA_OK(cudaLaunchKernelEx(&cfg, blk_wgrad_kernel, p));
+        RS_CUDA_OK(cudaLaunchKernelEx(&cfg, kernel, p));
     } else {
-        blk_wgrad_kernel<<<grid, NUM_THREADS, smem, stream>>>(p);
+        kernel<<<grid, NUM_THREADS, smem, stream>>>(p);
     }
     rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());
+    if (det) return rs::slot_sum(jobs, n_jobs, p.splits, p.ws_split, true, stream);
     return 0;
 }

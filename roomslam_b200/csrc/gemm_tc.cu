@@ -6,7 +6,8 @@
 //              written with TMA stores.  M is huge (B*(T+2) rows), N and K are small multiples of 128 / 64.
 //              -> layer input projection  P = X . W_ih^T + b_ih   and   dX = dG . W_ih
 //   mode TN  : C[M,N] += A[Kr,M]^T . B[Kr,N], reduction over the ROWS of A and B (both "MN-major" operands),
-//              split over CTAs along Kr, fp32 result added to C with red.global.add.f32.  A rows and B rows may be
+//              split over CTAs along Kr, fp32 result added to C with red.global.add.f32 (deterministic mode: per-split
+//              partials in a workspace, summed in split order by rs::slot_sum).  A rows and B rows may be
 //              shifted against each other by one (dW_hh pairs dGh_t with h_{t-1}).
 //              -> dW_ih = dGx^T . X,  dW_hh = dGh^T . H_prev
 //
@@ -43,7 +44,9 @@ struct GemmParams {
     long long ldc;          // TN: leading dimension of C (floats)
 };
 
-template <bool kTN>
+// kDet (TN only): the tile of split s is stored to slot s of the workspace p.c_f32 ([splits][M][ldc = N]) instead of being
+// added to C with atomics
+template <bool kTN, bool kDet = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_c, const GemmParams p) {
@@ -236,16 +239,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
                 }
             } else {
                 const int gm = m_blk * BM + row;
+                float* cbase = kDet ? p.c_f32 + static_cast<long long>(tile / (p.m_tiles * p.n_tiles)) * p.M * p.ldc : p.c_f32;
 #pragma unroll
                 for (int c0 = 0; c0 < BN; c0 += 32) {
                     uint32_t r[32];
                     rs::tmem_ld_32x32b_x32(taddr + c0, r);
                     rs::tmem_ld_wait();
                     if (gm < p.M) {
-                        float* crow = p.c_f32 + static_cast<long long>(gm) * p.ldc + n_blk * BN + c0;
+                        float* crow = cbase + static_cast<long long>(gm) * p.ldc + n_blk * BN + c0;
 #pragma unroll
-                        for (int j = 0; j < 32; ++j)
-                            if (n_blk * BN + c0 + j < p.N) atomicAdd(crow + j, __uint_as_float(r[j]));
+                        for (int j = 0; j < 32; ++j) {
+                            if (n_blk * BN + c0 + j >= p.N) continue;
+                            if (kDet) crow[j] = __uint_as_float(r[j]);
+                            else atomicAdd(crow + j, __uint_as_float(r[j]));
+                        }
                     }
                 }
                 rs::tc_fence_before();
@@ -285,6 +292,8 @@ extern "C" int rs_gemm_bf16_nt(const void* A, int64_t lda, const void* B, int64_
     RS_REQUIRE(K % BK == 0 && N % BN == 0, "rs_gemm_bf16_nt: need K %% 64 == 0 and N %% 128 == 0 (got N=%d K=%d)", N, K);
     RS_REQUIRE(lda % 8 == 0 && ldb % 8 == 0 && ldc % 8 == 0, "rs_gemm_bf16_nt: leading dimensions must be multiples of 8");
     const bool out_f32 = flags & RS_GEMM_OUT_F32;
+    RS_REQUIRE(!out_f32 || ((reinterpret_cast<uintptr_t>(C) & 15) == 0 && ldc % 4 == 0 && (reinterpret_cast<uintptr_t>(bias) & 15) == 0),
+               "rs_gemm_bf16_nt: with RS_GEMM_OUT_F32, C and bias are accessed as float4 and must be 16-byte aligned");
     RS_REQUIRE(M < (1ll << 31), "rs_gemm_bf16_nt: M too large");
     CUtensorMap ta, tb, tc;
     if (rs::make_tmap_2d(&ta, A, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, K, M, lda * 2, BK, BM, CU_TENSOR_MAP_SWIZZLE_128B)) return 2;
@@ -333,7 +342,8 @@ static int tn_launch(const void* A, int64_t lda, int64_t a_rows, int a_col0, int
     const int out_tiles = p.m_tiles * p.n_tiles;
     const long long kb_per_seg = (rows + BK - 1) / BK;
     const long long kblocks_total = kb_per_seg * n_seg;
-    int splits = num_sms() / out_tiles;
+    const bool det = rs::deterministic();
+    int splits = (det ? rs::kDetSplitSms : num_sms()) / out_tiles;
     if (splits < 1) splits = 1;
     if (splits > kblocks_total) splits = (int)kblocks_total;
     const long long kb_per_split = (kblocks_total + splits - 1) / splits;
@@ -346,9 +356,20 @@ static int tn_launch(const void* A, int64_t lda, int64_t a_rows, int a_col0, int
     p.a_row_shift = a_row_shift; p.b_row_shift = b_row_shift;
     p.a_col0 = a_col0; p.b_col0 = b_col0;
     p.c_f32 = C; p.ldc = ldc;
-    RS_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     const int total = out_tiles * splits;
     int grid = total < num_sms() ? total : num_sms();
+    if (det && splits > 1) {
+        rs::StreamScratch ws(stream);
+        RS_CUDA_OK(ws.alloc(sizeof(float) * (size_t)splits * M * N));
+        p.c_f32 = ws.as<float>(); p.ldc = N;
+        RS_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        gemm_tc_kernel<true, true><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(ta, tb, ta, p);
+        rs::count_launch();
+        RS_CUDA_OK(cudaGetLastError());
+        const rs::SlotSum<float> job = {ws.as<float>(), C, ldc, M, N};
+        return rs::slot_sum(&job, 1, splits, (long long)M * N, true, stream);
+    }
+    RS_CUDA_OK(cudaFuncSetAttribute(gemm_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     gemm_tc_kernel<true><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(ta, tb, ta, p);
     rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());

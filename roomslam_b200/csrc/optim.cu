@@ -5,6 +5,8 @@
 
 namespace {
 
+// kDet: block b stores its sum to out[b] (summed in block order by rs::slot_sum) instead of adding it to out[0]
+template <bool kDet>
 __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g, long long n, float scale, double* out) {
     float s = 0.0f;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
@@ -18,7 +20,8 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float* __restrict__ g,
     if (threadIdx.x == 0) {
         double t = 0.0;
         for (int w = 0; w < 8; ++w) t += (double)red[w];
-        atomicAdd(out, t);
+        if (kDet) out[blockIdx.x] = t;
+        else atomicAdd(out, t);
     }
 }
 
@@ -56,9 +59,16 @@ extern "C" int rs_adamw_step_f32(float* p, const float* g, float* m, float* v, i
     RS_REQUIRE(p && g && m && v && sumsq_scratch && n >= 0 && step >= 1, "rs_adamw_step_f32: bad arguments");
     int blocks = (int)((n + 255) / 256);
     if (blocks > 148 * 4) blocks = 148 * 4;
-    if (max_norm > 0.0f) {
+    rs::StreamScratch ws(stream);
+    if (max_norm > 0.0f && rs::deterministic()) {
+        RS_CUDA_OK(ws.alloc(sizeof(double) * blocks));
+        sumsq_kernel<true><<<blocks, 256, 0, stream>>>(g, n, grad_scale, ws.as<double>());
+        rs::count_launch();
+        const rs::SlotSum<double> job = {ws.as<double>(), sumsq_scratch, 1, 1, 1};
+        if (int rc = rs::slot_sum(&job, 1, blocks, 1, false, stream)) return rc;
+    } else if (max_norm > 0.0f) {
         RS_CUDA_OK(cudaMemsetAsync(sumsq_scratch, 0, sizeof(double), stream));
-        sumsq_kernel<<<blocks, 256, 0, stream>>>(g, n, grad_scale, sumsq_scratch);
+        sumsq_kernel<false><<<blocks, 256, 0, stream>>>(g, n, grad_scale, sumsq_scratch);
         rs::count_launch();
     }
     const float bc1 = 1.0f - powf(beta1, (float)step), bc2 = 1.0f - powf(beta2, (float)step);

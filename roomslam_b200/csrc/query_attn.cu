@@ -253,6 +253,11 @@ __global__ void query_attn_combine_kernel(const float* __restrict__ part, int Q,
 // backward: recompute p from (max, sum); dP = d_ctx . m + d_anchor . nc; dS = p (dP - delta);
 //   d_memory[n] (+)= sum_q p d_ctx_q + dS qk_q  (+ d_summary / count on valid tokens)
 //   dqk partial[b, split][q] = sum_n dS m_n ; dqb partial = sum_n dS
+// Several query tiles add into the same d_memory rows: with atomics (atomic_dm) in one launch, or (kDet) one launch per
+// tile, qt = qt_det, each adding onto what the launches of the tiles before it wrote -- a fixed order, one writer per element
+// and launch.  A launch per tile was chosen over per-tile partial buffers: no workspace (B N D floats per tile) and no
+// extra reduction kernel.
+template <bool kDet>
 __global__ void __launch_bounds__(NT)
 query_attn_bwd_kernel(SeqC mem, const float* __restrict__ traces, int F, const unsigned char* __restrict__ mask,
                       const float* __restrict__ mean, const float* __restrict__ rms, const float* __restrict__ count,
@@ -260,7 +265,7 @@ query_attn_bwd_kernel(SeqC mem, const float* __restrict__ traces, int F, const u
                       const float* __restrict__ anchor, const float* __restrict__ stats, const float* __restrict__ d_ctx,
                       const float* __restrict__ d_anchor, const float* __restrict__ d_summary, int N, int Q, int D,
                       int tokens_per_split, float* __restrict__ d_mem, long long dm_ld, long long dm_rows, long long dm_row0,
-                      int atomic_dm, float* __restrict__ dq_part) {
+                      int atomic_dm, float* __restrict__ dq_part, int qt_det) {
     extern __shared__ __align__(16) float sm[];
     const int Dp = D + 1, J = D / 8;
     float* qk_s = sm;                       // [QT][Dp]
@@ -272,7 +277,7 @@ query_attn_bwd_kernel(SeqC mem, const float* __restrict__ traces, int F, const u
     float* qv_s = nc_s + TC * 4;            // [QT][8]: qb, max, 1/sum, delta, d_anchor x3, -
     __shared__ float mu[3];
     const long long b = blockIdx.x;
-    const int split = blockIdx.y, qt = blockIdx.z, splits = gridDim.y;
+    const int split = blockIdx.y, qt = kDet ? qt_det : blockIdx.z, splits = gridDim.y;
     const int q = threadIdx.x >> 3, g8 = threadIdx.x & 7;
     const int qg = qt * QT + q;
     for (int e = threadIdx.x; e < QT * D; e += NT) {
@@ -374,7 +379,8 @@ query_attn_bwd_kernel(SeqC mem, const float* __restrict__ traces, int F, const u
 #pragma unroll
                 for (int j = 0; j < MAXJ; ++j) {
                     if (j < J) {
-                        if (atomic_dm) atomicAdd(dst + 8 * j, dm[j]);
+                        if (kDet) dst[8 * j] = qt == 0 ? dm[j] : dst[8 * j] + dm[j];
+                        else if (atomic_dm) atomicAdd(dst + 8 * j, dm[j]);
                         else dst[8 * j] = dm[j];
                     }
                 }
@@ -455,10 +461,21 @@ extern "C" int rs_query_attn_bwd_f32(const float* memory, int64_t m_ld, int64_t 
     const int tps = ((chunks + splits - 1) / splits) * TC;
     const int qtiles = (Q + QT - 1) / QT;
     const size_t smem = ((size_t)3 * QT * (D + 1) + 2 * QT * (TC + 1) + TC * 4 + QT * 8) * sizeof(float);
-    RS_CUDA_OK(cudaFuncSetAttribute(query_attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    query_attn_bwd_kernel<<<dim3(B, splits, qtiles), NT, smem, stream>>>(
+    if (qtiles > 1 && rs::deterministic()) {
+        RS_CUDA_OK(cudaFuncSetAttribute(query_attn_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        for (int qt = 0; qt < qtiles; ++qt) {
+            query_attn_bwd_kernel<true><<<dim3(B, splits, 1), NT, smem, stream>>>(
+                mkc(memory, m_ld, m_rows, m_row0), traces, F, mask, mean, rms, count, qk, qb, ctx, anchor, stats, d_ctx, d_anchor,
+                d_summary, N, Q, D, tps, d_memory, dm_ld, dm_rows, dm_row0, 0, dq_part, qt);
+            rs::count_launch();
+        }
+        RS_CUDA_OK(cudaGetLastError());
+        return 0;
+    }
+    RS_CUDA_OK(cudaFuncSetAttribute(query_attn_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    query_attn_bwd_kernel<false><<<dim3(B, splits, qtiles), NT, smem, stream>>>(
         mkc(memory, m_ld, m_rows, m_row0), traces, F, mask, mean, rms, count, qk, qb, ctx, anchor, stats, d_ctx, d_anchor,
-        d_summary, N, Q, D, tps, d_memory, dm_ld, dm_rows, dm_row0, qtiles > 1 ? 1 : 0, dq_part);
+        d_summary, N, Q, D, tps, d_memory, dm_ld, dm_rows, dm_row0, qtiles > 1 ? 1 : 0, dq_part, 0);
     rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());
     return 0;

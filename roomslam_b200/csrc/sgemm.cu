@@ -2,7 +2,8 @@
 // projections, weight gradients and the decoder MLP.  The bf16 mode uses the tcgen05 kernel (gemm_tc.cu).
 //   C[m,n] = act( sum_k A(m,k) * B(k,n) + bias[n] ) (+ C[m,n] when accumulate)
 // A(m,k) = A[m*a_sm + k*a_sk], B(k,n) = B[k*b_sk + n*b_sn], C row-major with leading dimension ldc.
-// 64x64x16 tiles, 256 threads, 4x4 register micro-tiles; optional split-K over gridDim.z with fp32 atomics.
+// 64x64x16 tiles, 256 threads, 4x4 register micro-tiles; optional split-K over gridDim.z with fp32 atomics (deterministic
+// mode: per-split partials in a workspace, summed in split order by rs::slot_sum).
 #include "common.cuh"
 #include "../../include/roomslam_b200.h"
 
@@ -10,6 +11,8 @@ namespace {
 
 constexpr int BM = 64, BN = 64, BK = 16;
 
+// kDet: split z stores its partial (bias added by split 0) to C + z * M * N, a dense [M][N] slot (ldc = N)
+template <bool kDet>
 __global__ void __launch_bounds__(256)
 sgemm_kernel(const float* __restrict__ A, long long a_sm, long long a_sk, const float* __restrict__ B, long long b_sk,
              long long b_sn, float* __restrict__ C, long long ldc, const float* __restrict__ bias, int M, int N, int K,
@@ -67,7 +70,10 @@ sgemm_kernel(const float* __restrict__ A, long long a_sm, long long a_sk, const 
             if (gn >= N) continue;
             float v = acc[i][j];
             float* c = &C[gm * ldc + gn];
-            if (split) {
+            if (kDet) {
+                if (bias && blockIdx.z == 0) v += bias[gn];
+                C[(long long)blockIdx.z * M * N + gm * ldc + gn] = v;
+            } else if (split) {
                 if (bias && blockIdx.z == 0) v += bias[gn];
                 atomicAdd(c, v);  // C was zeroed (or holds the value to accumulate onto) before the launch
             } else {
@@ -80,6 +86,8 @@ sgemm_kernel(const float* __restrict__ A, long long a_sm, long long a_sk, const 
     }
 }
 
+// kDet: slab y stores its sums to out + y * N instead
+template <bool kDet>
 __global__ void colsum_kernel(const float* __restrict__ A, long long lda, int M, int N, int rows_per_block,
                               float* __restrict__ out) {
     // block = 32 columns x 8 row-lanes over a slab of rows; slabs are combined with fp32 atomics
@@ -95,7 +103,8 @@ __global__ void colsum_kernel(const float* __restrict__ A, long long lda, int M,
         float t = 0.0f;
 #pragma unroll
         for (int i = 0; i < 8; ++i) t += part[i][threadIdx.x];
-        atomicAdd(&out[col], t);
+        if (kDet) out[(long long)blockIdx.y * N + col] = t;
+        else atomicAdd(&out[col], t);
     }
 }
 
@@ -119,6 +128,16 @@ extern "C" int rs_sgemm(const float* A, int64_t a_sm, int64_t a_sk, const float*
             grid.z = (K + k_per_split - 1) / k_per_split;
         }
     }
+    if (grid.z > 1 && rs::deterministic()) {
+        rs::StreamScratch ws(stream);
+        RS_CUDA_OK(ws.alloc(sizeof(float) * (size_t)grid.z * M * N));
+        sgemm_kernel<true><<<grid, 256, 0, stream>>>(A, a_sm, a_sk, B, b_sk, b_sn, ws.as<float>(), N, bias, M, N, K, k_per_split,
+                                                     flags);
+        rs::count_launch();
+        RS_CUDA_OK(cudaGetLastError());
+        const rs::SlotSum<float> job = {ws.as<float>(), C, ldc, M, N};
+        return rs::slot_sum(&job, 1, (int)grid.z, (long long)M * N, flags & RS_GEMM_ACCUMULATE, stream);
+    }
     if (grid.z > 1 && !(flags & RS_GEMM_ACCUMULATE)) {
         if (ldc == N) {
             RS_CUDA_OK(cudaMemsetAsync(C, 0, sizeof(float) * (size_t)M * N, stream));
@@ -126,7 +145,7 @@ extern "C" int rs_sgemm(const float* A, int64_t a_sm, int64_t a_sk, const float*
             RS_CUDA_OK(cudaMemset2DAsync(C, sizeof(float) * ldc, 0, sizeof(float) * N, M, stream));
         }
     }
-    sgemm_kernel<<<grid, 256, 0, stream>>>(A, a_sm, a_sk, B, b_sk, b_sn, C, ldc, bias, M, N, K, k_per_split, flags);
+    sgemm_kernel<false><<<grid, 256, 0, stream>>>(A, a_sm, a_sk, B, b_sk, b_sn, C, ldc, bias, M, N, K, k_per_split, flags);
     rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());
     return 0;
@@ -141,7 +160,16 @@ extern "C" int rs_colsum_f32(const float* A, int64_t lda, int M, int N, float* o
     int slabs = (M + 2047) / 2048;
     if (slabs > 128) slabs = 128;
     const int rows_per_block = (M + slabs - 1) / slabs;
-    colsum_kernel<<<dim3((N + 31) / 32, slabs), dim3(32, 8), 0, stream>>>(A, lda, M, N, rows_per_block, out);
+    if (slabs > 1 && rs::deterministic()) {
+        rs::StreamScratch ws(stream);
+        RS_CUDA_OK(ws.alloc(sizeof(float) * (size_t)slabs * N));
+        colsum_kernel<true><<<dim3((N + 31) / 32, slabs), dim3(32, 8), 0, stream>>>(A, lda, M, N, rows_per_block, ws.as<float>());
+        rs::count_launch();
+        RS_CUDA_OK(cudaGetLastError());
+        const rs::SlotSum<float> job = {ws.as<float>(), out, N, 1, N};
+        return rs::slot_sum(&job, 1, slabs, N, true, stream);     // onto the zeroed or accumulated output
+    }
+    colsum_kernel<false><<<dim3((N + 31) / 32, slabs), dim3(32, 8), 0, stream>>>(A, lda, M, N, rows_per_block, out);
     rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());
     return 0;

@@ -77,6 +77,8 @@ extern "C" int rs_split_bf16x6(const float* x, int64_t ld, int64_t rows, int col
     RS_REQUIRE(kpad % 8 == 0 && kpad >= cols && ld_out >= 6 * (int64_t)kpad && ld_out % 8 == 0,
                "rs_split_bf16x6: kpad must be a multiple of 8 >= cols and ld_out >= 6 * kpad (multiple of 8)");
     RS_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "rs_split_bf16x6: output must be 16-byte aligned");
+    RS_REQUIRE((ld & 3) || (reinterpret_cast<uintptr_t>(x) & 15) == 0,
+               "rs_split_bf16x6: with ld %% 4 == 0 the rows are read as float4, so x must be 16-byte aligned");
     const long long total = rows * (kpad / 8);
     long long blocks = (total + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;

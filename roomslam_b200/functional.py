@@ -130,6 +130,8 @@ def split3(x2d: torch.Tensor, role_b: bool = False):
     x2d = x2d.float()
     if x2d.stride(1) != 1:
         x2d = x2d.contiguous()
+    if x2d.data_ptr() % 16:             # rows are read as float4; a parameter may be a view at any offset of a flat buffer
+        x2d = x2d.clone()
     rows, cols = x2d.shape
     kp = _kpad(cols)
     out = torch.empty(rows, 6 * kp, dtype=torch.bfloat16, device=x2d.device)
@@ -139,6 +141,8 @@ def split3(x2d: torch.Tensor, role_b: bool = False):
 
 def nt_tc(a3: torch.Tensor, b3: torch.Tensor, bias, out: torch.Tensor):
     """out[M, N] (fp32) = A . B^T + bias from split operands (a3: [M, 6kp] A role, b3: [N, 6kp] B role); N % 128 == 0."""
+    if bias is not None and bias.data_ptr() % 16:    # read as float4 (FlatParams views sit at any offset)
+        bias = bias.clone()
     _lib.call("rs_gemm_bf16_nt", _p(a3), a3.stride(0), _p(b3), b3.stride(0), _p(out), out.stride(0), _p(bias), a3.shape[0],
               b3.shape[0], a3.shape[1], OUT_F32, _stream(out))
 

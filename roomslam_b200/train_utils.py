@@ -6,6 +6,7 @@ clip_grad_norm_(1.0), optimizer.step with AdamW :440-444), for one process per G
 """
 from __future__ import annotations
 
+import os
 import re
 from typing import List, Optional
 
@@ -14,6 +15,19 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from . import _lib
+
+
+def seed_everything(seed: int) -> None:
+    """Seeds Python, numpy and torch (host and every GPU) and turns on torch.use_deterministic_algorithms, which the
+    library follows with fixed-order split reductions: a rerun with the same seed, data and GPU model gives the same bits."""
+    import random
+
+    import numpy as np
+    os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")     # torch's condition for deterministic cuBLAS calls
+    random.seed(seed)
+    np.random.seed(seed)
+    torch.manual_seed(seed)
+    torch.use_deterministic_algorithms(True)
 
 
 class FlatParams:

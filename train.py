@@ -10,7 +10,7 @@ import os
 import torch
 
 from roomslam_b200 import RoomSLAM, data
-from roomslam_b200.train_utils import FlatParams, FusedAdamW
+from roomslam_b200.train_utils import FlatParams, FusedAdamW, seed_everything
 
 # README.md:147-157
 BATCH_SIZE, LEARNING_RATE, HIDDEN_SIZE, SEQUENCE_LENGTH, MAX_OBJECTS, NUM_EPOCHS = 32, 1e-3, 128, 500, 10, 100
@@ -26,11 +26,15 @@ def main():
     ap.add_argument("--create_sample_data", action="store_true")
     ap.add_argument("--checkpoint_dir", default="checkpoints")
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--deterministic", action="store_true",
+                    help="seed everything and turn on torch.use_deterministic_algorithms: bit-identical reruns")
     args = ap.parse_args()
     if args.create_sample_data:
         data.create_sample_data(args.data_dir, seq_len=SEQUENCE_LENGTH, max_objects=MAX_OBJECTS, seed=args.seed)
         print(f"wrote sample data to {args.data_dir}")
         return
+    if args.deterministic:
+        seed_everything(args.seed)
     torch.manual_seed(args.seed)
     x, tgt = data.load_dir(args.data_dir, SEQUENCE_LENGTH, MAX_OBJECTS)
     n_val = max(1, len(x) // 10)

@@ -19,6 +19,7 @@ from roomslam_b200 import data, preprocess
 from roomslam_b200.evaluation import MetricAccumulator
 from roomslam_b200.lstm_model import build_model
 from roomslam_b200.set_loss import SetCriterion
+from roomslam_b200.train_utils import seed_everything
 
 WEIGHTS = {"class_loss": 2.0, "l1_loss": 5.0, "giou_loss": 2.0}                 # train.py:433-437
 
@@ -55,10 +56,14 @@ def main():
     ap.add_argument("--max_trace_len", type=int, default=3000)
     ap.add_argument("--iou_thresh", type=float, default=0.5)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--deterministic", action="store_true",
+                    help="seed everything and turn on torch.use_deterministic_algorithms: bit-identical reruns")
     args = ap.parse_args()
     config = dict(vars(args), model_type="lstm")
     os.makedirs(args.save_dir, exist_ok=True)
     json.dump(config, open(os.path.join(args.save_dir, "config.json"), "w"), indent=2)
+    if args.deterministic:
+        seed_everything(args.seed)
     torch.manual_seed(args.seed)
     gen = torch.Generator().manual_seed(args.seed)
     train_pts, train_tgt = load_split(args.data_dir)
