@@ -171,10 +171,10 @@ int rs_blk_wgrad(const void* dG, int64_t a_cols, const void* ones_block, int n_r
                  int tiles, int T, void* stream);
 /* ---- bf16 mode: every bf16 operand image of one bidirectional layer from its fp32 master weights, one launch -------
  * w: HOST array of 8 DEVICE pointers (weight_ih, weight_hh, bias_ih, bias_hh, then the _reverse twins; torch.nn.GRU's
- * names, shapes and r|z|n gate order).  Outputs (device): whh_img [2][H/8 (+2 for layer 0)][3H][8] bf16 (the image
- * rs_rec_fwd_bf16 documents), b_hn [2][H], bias_x [2][3H] (b_ih + b_hh of r, z; scaled like the rows), wt_proj
- * [6H/128][I/64][8][128][8] bf16 (B pieces of rs_blk_gemm_nt for P = X W_ih^T; NULL for layer 0 whose I <= 2 columns ride
- * in whh_img), whhT_img [2][3H/8][H][8] bf16 (rs_rec_bwd_bf16), wt_dgrad [I/128][6H/64][8][128][8] bf16 (dX = dG W_ih) or
+ * names, shapes and r|z|n gate order).  I <= 16 is layer 0, deeper layers take a multiple of 128.  Outputs (device):
+ * whh_img [2][H/8 (+2 x_steps(I) for layer 0, +2 with wih_img)][3H][8] bf16 (the image rs_rec_fwd_bf16 documents), b_hn
+ * [2][H], bias_x [2][3H] (b_ih + b_hh of r, z; scaled like the rows), wt_proj [6H/128][I/64][8][128][8] bf16 (B pieces of
+ * rs_blk_gemm_nt for P = X W_ih^T; NULL for layer 0 whose I <= 16 columns ride in whh_img), whhT_img [2][3H/8][H][8] bf16 (rs_rec_bwd_bf16), wt_dgrad [I/128][6H/64][8][128][8] bf16 (dX = dG W_ih) or
  * NULL.
  * split = 1: every weight image holds a bf16 PAIR per weight, hi = bf16(w) then lo = bf16(w - hi), stacked along K
  * (whh_img: chunks [0, H/8) hi, [H/8, H/4) lo, then the layer-0 input chunks; whhT_img, wt_proj, wt_dgrad: K blocks hi
@@ -184,9 +184,11 @@ int rs_blk_wgrad(const void* dG, int64_t a_cols, const void* ones_block, int n_r
 int rs_gru_pack_weights_bf16(const float* const* w, int H, int I, int split, void* whh_img, float* b_hn, float* bias_x,
                              void* wt_proj, void* whhT_img, void* wt_dgrad, void* wih_img, void* stream);
 /* ---- bf16 mode: persistent tcgen05 GRU recurrence (H = 128), tile-major activations --------------------------- */
-/* Forward of one bidirectional layer.  Layer 0: x (B, T, I <= 2) fp32, its projection rides on the tensor core:
- * Whh is then [2][18][384][8] bf16 with chunk 16 = per gate row (w_hi, w_hi, w_lo) per input and (b_hi, b_lo), chunk
- * 17 = 0.  Deeper layers, either: P tile-major (6H columns, bias folded in) and Whh [2][16][384][8]; or, with the
+/* Forward of one bidirectional layer.  Layer 0: x (B, T, 1 <= I <= 16) fp32, its projection rides on the tensor core as
+ * s = x_steps(I) = ceil((3 I + 2) / 16) more K = 16 steps: Whh is then [2][16 + 2 s][384][8] bf16 whose chunks 16 .. 15 + 2 s
+ * hold the input columns: input i at columns 3 i + k (i < 2) or 8 + 3 (i - 2) + k (i >= 2), k = 0, 1, 2 = per gate row
+ * (w_hi, w_hi, w_lo); the bias (b_hi, b_lo) at columns 6, 7; every other column 0 (I <= 2: chunk 16 as always, chunk
+ * 17 = 0).  Any other I is rejected with an error.  Deeper layers, either: P tile-major (6H columns, bias folded in) and Whh [2][16][384][8]; or, with the
  * projection FUSED into the recurrence (unsplit weights): X = the layer's tile-major input (2H columns), Wih
  * [2][32][384][8] and Whh [2][18][384][8] whose chunk 16 holds only the bias (rs_gru_pack_weights_bf16 with wih_img) --
  * P and the projection GEMM are then not needed at all.  The r and z rows of all
@@ -208,10 +210,10 @@ int rs_rec_bwd_bf16(const void* d_out, const float* d_h_n, const void* gates, co
 /* The same two kernels for hidden_size = 256 (BASELINE config 4: H 256, T 4000), where W_hh no longer fits in shared memory:
  * each CTA of the pair streams its half of the weights from L2 through a ring of bulk copies once per time step
  * (csrc/rec_wide.cu).  Tile-major operands as above with H = 256 (P 6H, out 2H, dG 8H columns; gates
- * [tiles][T][2][128][128][8] fp16).  Wst: [2 dirs][2 ranks][9 (layer 0) or 8 stages][2 K steps][2 chunks][384 rows][8]
- * bf16, rows = r | z | n gate rows of hidden units [128 rank, 128 rank + 128) (r, z scaled by 1/2), K step k = hidden
- * units [16 k, 16 k + 16); layer 0: K step 16 = the input chunk (w_hi, w_hi, w_lo per input column, b_hi, b_lo) and a zero
- * chunk, K step 17 = 0.  WTst: [2][2][8 stages][6 K steps][2 chunks][128 rows][8] bf16 = W_hh^T with rows = hidden units
+ * [tiles][T][2][128][128][8] fp16).  Wst: [2 dirs][2 ranks][8 + ceil(s / 2) (layer 0, s = x_steps(I), 1 <= I <= 16) or 8
+ * stages][2 K steps][2 chunks][384 rows][8] bf16, rows = r | z | n gate rows of hidden units [128 rank, 128 rank + 128) (r, z
+ * scaled by 1/2), K step k = hidden units [16 k, 16 k + 16); layer 0: K steps 16 .. 15 + s = the input columns of
+ * rs_rec_fwd_bf16's Whh (same column map), then zero K steps up to the whole stage.  WTst: [2][2][8 stages][6 K steps][2 chunks][128 rows][8] bf16 = W_hh^T with rows = hidden units
  * [128 rank, +128) and K = the 768 gate rows in r | z | n order. */
 int rs_rec_fwd_bf16_wide(const float* x, int I, const void* P, const void* Wst, const float* b_hn, void* out, void* gates,
                          float* h_n, const int* lengths, const void* drop_bits, const float* drop_scale, void* out_drop,

@@ -1,7 +1,8 @@
 // One launch builds every bf16 operand image a bidirectional GRU layer needs from its fp32 master weights
 // (torch.nn.GRU's weight_ih / weight_hh / bias_ih / bias_hh and their _reverse twins, rnn.py:1290-1297 gate order r|z|n):
-//   whh_img   [2][16 (+2)][3H][8]  B operand of the recurrence forward (r, z rows scaled by 1/2: sigma(a) = tanh(a/2)/2 + 1/2);
-//                                  layer 0: chunk 16 = per gate row (w_hi, w_hi, w_lo) per input column and (b_hi, b_lo)
+//   whh_img   [2][16 (+2 s)][3H][8]  B operand of the recurrence forward (r, z rows scaled by 1/2: sigma(a) = tanh(a/2)/2 + 1/2);
+//                                  layer 0 (I <= 16): chunks 16 .. 15 + 2 s, s = x_steps(I) = the input columns: per gate row
+//                                  (w_hi, w_hi, w_lo) per input and (b_hi, b_lo) at the columns of rec_common.cuh's map
 //   b_hn      [2][H]               bias of the hidden side of the n gate
 //   bias_x    [2][3H]              b_ih (+ b_hh for r, z), scaled like the rows: folded into the projection / the input chunk
 //   wt_proj   [6H/128][I/64][8][128][8]   W_ih (scaled) as B pieces of the projection GEMM            (deeper layers)
@@ -29,7 +30,7 @@ struct PackWParams {
     const float* b_hh[2];
     int H, I, nck, split;                      // split: every weight as a bf16 pair hi + lo (see rs_gru_pack_weights_bf16)
     uint4* whh_img; float* b_hn; float* bias_x; uint4* wt_proj; uint4* whhT_img; uint4* wt_dgrad; uint4* wih_img;
-    int bias_chunk;                            // whh_img carries the input chunk (layer 0: input weights + bias; fused projection: bias only)
+    int layer0;                                // whh_img's input chunks hold the input weights and the bias (else: the bias only)
     long long n_a, n_e, n_d, n_f, n_g, n_b;    // pieces per region
 };
 
@@ -66,15 +67,20 @@ __global__ void pack_w_kernel(const PackWParams p) {
             } else {
 #pragma unroll
                 for (int j = 0; j < 8; ++j) v[j] = 0.0f;
-                if (c == nh) {                             // input chunk: layer-0 input weights (hi, hi, lo) and the bias (hi, lo)
-                    for (int ci = 0; ci < I && ci < 2 && I <= 2; ++ci) {
-                        const float w = __ldg(p.w_ih[d] + (long long)row * I + ci) * s;
+                // input chunks (rec_common.cuh's column map): layer-0 input weights (hi, hi, lo) and the bias (hi, lo);
+                // with the fused projection the bias only
+#pragma unroll
+                for (int j = 0; j < 8; ++j) {
+                    const int col = (c - nh) * 8 + j, i = x_col_input(col), k = x_col_part(col);
+                    if (i < 0) {
+                        const float b = bias_x_of(p, d, row);
+                        const float bhi = __bfloat162float(__float2bfloat16_rn(b));
+                        v[j] = k == 0 ? bhi : b - bhi;
+                    } else if (p.layer0 && i < I) {
+                        const float w = __ldg(p.w_ih[d] + (long long)row * I + i) * s;
                         const float hi = __bfloat162float(__float2bfloat16_rn(w));
-                        v[3 * ci] = hi; v[3 * ci + 1] = hi; v[3 * ci + 2] = w - hi;
+                        v[j] = k == 2 ? w - hi : hi;
                     }
-                    const float b = bias_x_of(p, d, row);
-                    const float bhi = __bfloat162float(__float2bfloat16_rn(b));
-                    v[6] = bhi; v[7] = b - bhi;
                 }
             }
             p.whh_img[e] = pack8(v);
@@ -159,9 +165,9 @@ extern "C" int rs_gru_pack_weights_bf16(const float* const* w, int H, int I, int
     if (rs::check_device_sm100()) return 3;
     RS_REQUIRE(w && whh_img && b_hn && bias_x && whhT_img, "rs_gru_pack_weights_bf16: bad arguments");
     RS_REQUIRE(H % 128 == 0 && H >= 128, "rs_gru_pack_weights_bf16: H must be a multiple of 128");
-    const bool layer0 = (I <= 2);
+    const bool layer0 = (I <= rs::kMaxXInputs);            // deeper layers take a multiple of 128: unambiguous
     RS_REQUIRE(layer0 ? (I >= 1 && !wt_dgrad && !wt_proj && !wih_img) : (I % 128 == 0 && (wt_proj || wih_img)),
-               "rs_gru_pack_weights_bf16: layer 0 takes 1-2 input columns (no projection images); deeper layers a multiple of 128 "
+               "rs_gru_pack_weights_bf16: layer 0 takes 1-16 input columns (no projection images); deeper layers a multiple of 128 "
                "and wt_proj (projection GEMM) or wih_img (projection fused into the recurrence)");
     RS_REQUIRE(!(wih_img && split), "rs_gru_pack_weights_bf16: the fused projection takes plain (unsplit) weights");
     PackWParams p = {};
@@ -170,8 +176,8 @@ extern "C" int rs_gru_pack_weights_bf16(const float* const* w, int H, int I, int
         RS_REQUIRE(p.w_ih[d] && p.w_hh[d] && p.b_ih[d] && p.b_hh[d], "rs_gru_pack_weights_bf16: null weight pointer");
     }
     split = split ? 1 : 0;
-    p.bias_chunk = (layer0 || wih_img) ? 1 : 0;
-    p.H = H; p.I = I; p.split = split; p.nck = (H / 8) * (1 + split) + (p.bias_chunk ? 2 : 0);
+    p.layer0 = layer0 ? 1 : 0;
+    p.H = H; p.I = I; p.split = split; p.nck = (H / 8) * (1 + split) + (layer0 ? 2 * rs::x_steps(I) : (wih_img ? 2 : 0));
     p.whh_img = static_cast<uint4*>(whh_img); p.b_hn = b_hn; p.bias_x = bias_x;
     p.wt_proj = static_cast<uint4*>(wt_proj); p.whhT_img = static_cast<uint4*>(whhT_img); p.wt_dgrad = static_cast<uint4*>(wt_dgrad);
     p.wih_img = static_cast<uint4*>(wih_img);

@@ -58,7 +58,8 @@ extern "C" int rs_rec_fwd_bf16(const float* x, int I, const void* P, int64_t p_c
     RS_REQUIRE((x != nullptr) + (P != nullptr) + (X != nullptr) == 1,
                "rs_rec_fwd_bf16: exactly one of x (layer 0), P (deeper layers, projected) and X (deeper layers, projection fused) must be given");
     RS_REQUIRE(!X || (Wih && !split), "rs_rec_fwd_bf16: the fused projection needs Wih and plain (unsplit) weights");
-    RS_REQUIRE(!x || (I >= 1 && I <= 2), "rs_rec_fwd_bf16: the MMA-fused input projection takes 1 or 2 input columns");
+    RS_REQUIRE(!x || (I >= 1 && I <= rs::kMaxXInputs), "rs_rec_fwd_bf16: the MMA-fused input projection takes 1 to %d input columns (got %d)",
+               rs::kMaxXInputs, I);
     RS_REQUIRE(!P || p_cols == 6 * H, "rs_rec_fwd_bf16: P must have 6H = %d columns", 6 * H);
     RS_REQUIRE(Whh && b_hn && out && h_n && B >= 0 && T >= 0, "rs_rec_fwd_bf16: bad arguments");
     if (T == 0) {

@@ -46,8 +46,33 @@ __device__ __forceinline__ void unpack8h(const uint4& v, float* f) {
 __device__ __forceinline__ uint4 ldg16(const uint8_t* p) { return __ldg(reinterpret_cast<const uint4*>(p)); }
 __device__ __forceinline__ void stg16(uint8_t* p, const uint4& v) { *reinterpret_cast<uint4*>(p) = v; }
 
-// Layer-0 input columns of one trace row: per input c the triple (hi, lo, hi) with hi = bf16(x_c), lo = bf16(x_c - hi),
-// then (1, 1); at most 2 inputs fit the 8 columns of one 16-byte chunk.
+// Layer-0 input columns: W_ih x + b rides on the recurrence MMA as extra K = 16 steps of hi / lo split operands.  The column
+// map (A operand = the trace row, built here; B operand = the weight image, built by pack_w.cu for H = 128 and by
+// functional_bf16.py for H = 256):
+//   input i < 2 : columns 3 i + k        k = 0, 1, 2:  x (hi, lo, hi)  against  W_ih (hi, hi, lo)
+//   bias        : columns 6, 7                         (1, 1)          against  b (hi, lo)
+//   input i >= 2: columns 8 + 3 (i - 2) + k            as inputs 0 and 1
+//   every other column of the input K steps is zero.
+// Inputs 0, 1 and the bias fill the first 16-byte chunk exactly as the 2-input layout always did; I inputs take 3 I + 2
+// columns, so x_steps(I) = ceil((3 I + 2) / 16) K steps: 1 up to 4 inputs, 2 up to 10, 3 up to 15, 4 for 16.
+constexpr int kMaxXInputs = 16;
+__host__ __device__ constexpr int x_col(int i, int k) { return i < 2 ? 3 * i + k : 8 + 3 * (i - 2) + k; }
+__host__ __device__ constexpr int x_col_input(int c) { return c < 6 ? c / 3 : (c < 8 ? -1 : 2 + (c - 8) / 3); }  // -1: bias
+__host__ __device__ constexpr int x_col_part(int c) { return c < 6 ? c % 3 : (c < 8 ? c - 6 : (c - 8) % 3); }
+__host__ __device__ constexpr int x_steps(int I) { return (3 * I + 2 + 15) / 16; }
+// 16-byte chunks per row of the input columns a recurrence kernel writes: 1 for I <= 2 (the second chunk of the one K step
+// stays zero), else every chunk of the x_steps(I) K steps
+__host__ __device__ constexpr int x_chunks(int I) { return I <= 2 ? 1 : 2 * x_steps(I); }
+constexpr bool x_map_ok() {
+    for (int i = 0; i < kMaxXInputs; ++i)
+        for (int k = 0; k < 3; ++k)
+            if (x_col_input(x_col(i, k)) != i || x_col_part(x_col(i, k)) != k || x_col(i, k) >= 16 * x_steps(i + 1)) return false;
+    return x_col_input(6) == -1 && x_col_input(7) == -1 && x_steps(2) == 1 && x_steps(kMaxXInputs) == 4;
+}
+static_assert(x_map_ok(), "layer-0 input column map");
+
+// Chunk 0 of the input columns of one trace row: per input c < 2 the triple (hi, lo, hi) with hi = bf16(x_c),
+// lo = bf16(x_c - hi), then (1, 1).  Everything a row with at most 2 inputs needs.
 __device__ __forceinline__ uint4 pack_x(const float* xp, int I) {
     float c[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     if (xp) {
@@ -62,6 +87,26 @@ __device__ __forceinline__ uint4 pack_x(const float* xp, int I) {
     }
     c[6] = 1.0f; c[7] = 1.0f;
     return pack8(c);
+}
+// Chunk ch (any of the x_chunks(I)) of the input columns of one trace row; xp = NULL (pad row): the bias columns only.
+__device__ __forceinline__ uint4 pack_x_chunk(const float* xp, int I, int ch) {
+    uint32_t w[4];
+#pragma unroll
+    for (int jp = 0; jp < 4; ++jp) {                   // two columns at a time keeps the live set small
+        float v[2];
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const int i = x_col_input(ch * 8 + 2 * jp + e), k = x_col_part(ch * 8 + 2 * jp + e);
+            v[e] = i < 0 ? 1.0f : 0.0f;
+            if (xp && i >= 0 && i < I) {
+                const float x = __ldg(xp + i);
+                const float hi = __bfloat162float(__float2bfloat16_rn(x));
+                v[e] = k == 1 ? x - hi : hi;
+            }
+        }
+        w[jp] = f2_to_bf2(v[0], v[1]);
+    }
+    return make_uint4(w[0], w[1], w[2], w[3]);
 }
 
 

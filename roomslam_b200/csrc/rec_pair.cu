@@ -30,8 +30,7 @@ constexpr int ROWS = 64;                        // traces of a tile held by one 
 constexpr int CHUNK_G = 2048;                   // global: one 16-byte chunk column over the 128 rows of a tile
 constexpr int CHUNK_S = ROWS * 16;              // shared: the same over this CTA's 64 rows
 constexpr int W_CHUNK = 192 * 16;               // shared: one chunk column of this CTA's W_hh rows (r | z | hn of 64 units)
-constexpr int W_FWD_BYTES = 18 * W_CHUNK;       // 54 KB (16 hidden chunks + 2 layer-0 input chunks)
-constexpr int A_FWD_BYTES = 18 * CHUNK_S;       // 18 KB per tile in flight
+constexpr int A_FWD_BYTES = 18 * CHUNK_S;       // 18 KB per tile in flight (16 hidden chunks + one K step of input chunks)
 constexpr int H32_BYTES = (H / 4) * CHUNK_S;    // 32 KB per tile in flight (fp32 master copy of h)
 constexpr int W_BWD_BYTES = 48 * CHUNK_S;       // 48 KB: W_hh^T rows of this CTA's 64 hidden units, K = 384 gate rows
 constexpr int A_BWD_BYTES = 48 * CHUNK_S;       // 48 KB per tile in flight (dGh)
@@ -44,6 +43,7 @@ template <int NT> struct EpiShape {
     static constexpr int NGRP = UPT / 8;                // 16-byte chunks (8 units) per thread and step
 };
 constexpr int NUM_THREADS = 64 + 512;
+constexpr int X_CHUNKS_USED = x_col(kMaxXInputs - 1, 2) / 8 + 1;   // 7 of the 8 chunks of 4 input K steps (the last is padding)
 
 struct FwdPairParams {
     const float* x; int I;
@@ -65,7 +65,12 @@ struct FwdPairParams {
 };
 
 // kMode 0: the input-side pre-activations come from HBM (P, written by the projection GEMM).
-// kMode 1: layer 0, the K = 2 input projection rides on the recurrence MMA as one more K = 16 step (hi / lo split operands).
+// kMode 1: layer 0, the K = I input projection rides on the recurrence MMA as (kXC + 1) / 2 more K = 16 steps of hi / lo
+//   split operands (rec_common.cuh has the column map).  kXC = the 16-byte input chunks per row the epilogue writes each step:
+//   1 (I <= 2: the one K step's second chunk stays zero; written after the epilogue from registers loaded before the wait
+//   for the accumulator), else x_chunks(I), spread over the threads of a row and double-buffered in the A tile: the chunks
+//   of step t+1 go into the buffer the MMA of step t does not read, BEFORE the wait, so no packed input is held in
+//   registers across it (the 96-register cap left no room for that without spills).
 // kMode 2 (NT = 1): the K = 256 input projection of a deeper layer is FUSED: W_ih's rows of this CTA's hidden units stay in
 //   shared memory next to W_hh (96 + 54 KB; the master state is in registers in this mode), warp 1 bulk-copies the layer
 //   input X_t of the CTA's 64 rows one step ahead (32 KB, one buffer), and the issuer runs X_{t+1} . W_ih^T (+ the bias via the
@@ -75,18 +80,23 @@ struct FwdPairParams {
 //   loads left at all.
 // kDrop: inter-layer dropout on this layer's output (drop_bits / out_drop given).  A template parameter, not a run-time
 // flag: the mask test, the scaled copy and its bf16 pack are ~3.5 of the epilogue's 24 instructions per (row, hidden unit).
-template <int NT, bool kVarLen, int kMode, bool kDrop>
+template <int NT, bool kVarLen, int kMode, bool kDrop, int kXC = 1>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_fwd_pair_kernel(const FwdPairParams p) {
     constexpr bool kFusedX = (kMode != 0);                 // the n gate's input part arrives in its own accumulator columns
     constexpr bool kProj = (kMode == 2);
     static_assert(!kProj || NT == 1, "the fused projection needs the double-buffered accumulator of the one-tile mode");
+    static_assert(kXC == 1 || (kMode == 1 && kXC % 2 == 0 && kXC <= 2 * x_steps(kMaxXInputs)), "input chunks per row");
+    constexpr int kXS = (kXC + 1) / 2;                     // input K steps
+    constexpr int kXB = kXC == 1 ? 1 : 2;                  // input column buffers
+    constexpr int kXCW = kXC < X_CHUNKS_USED ? kXC : X_CHUNKS_USED;   // chunks that can hold a nonzero column
+    constexpr int A_BYTES = (16 + 2 * kXS * kXB) * CHUNK_S;     // A tile per tile in flight: h_{t-1} | input columns
     extern __shared__ __align__(1024) uint8_t smem[];
-    uint8_t* w_s = smem;                                   // [18 chunks][192 rows][16 B]
+    uint8_t* w_s = smem;                                   // [16 (x2 split) + 2 kXS chunks][192 rows][16 B]
     const int n_hid = 16 * (1 + p.split);                  // hidden-state chunks of W: hi parts, then (split) lo parts
-    const int n_chunks = n_hid + (kFusedX ? 2 : 0);
+    const int n_chunks = n_hid + (kFusedX ? 2 * kXS : 0);
     uint8_t* wih_s = w_s + n_chunks * W_CHUNK;             // [32 chunks][192 rows][16 B]   (kProj)
-    uint8_t* a_s = wih_s + (kProj ? 32 * W_CHUNK : 0);     // [NT][18 chunks][64 rows][16 B]  h_{t-1} | input columns
-    uint8_t* h32_s = a_s + NT * A_FWD_BYTES;               // [NT][32 chunks of 4 floats][64 rows][16 B]   (NT = 2 only)
+    uint8_t* a_s = wih_s + (kProj ? 32 * W_CHUNK : 0);     // [NT][16 + 2 kXS kXB chunks][64 rows][16 B]  h_{t-1} | input columns
+    uint8_t* h32_s = a_s + NT * A_BYTES;                   // [NT][32 chunks of 4 floats][64 rows][16 B]   (NT = 2 only)
     uint8_t* x_s = h32_s + (NT == 1 ? 0 : NT * H32_BYTES); // [32 chunks][64 rows][16 B]  X_t of this CTA's rows (kProj)
     float* bhn_s = reinterpret_cast<float*>(x_s + (kProj ? 32 * CHUNK_S : 0));
     uint64_t* bars = reinterpret_cast<uint64_t*>(bhn_s + H);
@@ -138,14 +148,23 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
         }
     }
     for (int i = threadIdx.x; i < H; i += blockDim.x) bhn_s[i] = p.b_hn[dir * H + i];
-    for (int i = threadIdx.x; i < NT * (A_FWD_BYTES + (NT == 1 ? 0 : H32_BYTES)) / 16; i += blockDim.x)
+    for (int i = threadIdx.x; i < NT * (A_BYTES + (NT == 1 ? 0 : H32_BYTES)) / 16; i += blockDim.x)
         reinterpret_cast<uint4*>(a_s)[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
-    if (fused_x && threadIdx.x < ROWS * NT) {           // input columns of the first step
-        const int s = threadIdx.x / ROWS, rl = threadIdx.x % ROWS;
-        const long long b = (long long)(tile0 + s) * 128 + rank * ROWS + rl;
-        *reinterpret_cast<uint4*>(a_s + s * A_FWD_BYTES + 16 * CHUNK_S + rl * 16) =      // kProj: the constant (1, 1) bias column only
-            pack_x((!kProj && s < n_slots && b < p.B) ? p.x + (b * T + (dir ? T - 1 : 0)) * p.I : nullptr, p.I);
+    if (kXC == 1) {
+        if (fused_x && threadIdx.x < ROWS * NT) {       // input columns of the first step
+            const int s = threadIdx.x / ROWS, rl = threadIdx.x % ROWS;
+            const long long b = (long long)(tile0 + s) * 128 + rank * ROWS + rl;
+            *reinterpret_cast<uint4*>(a_s + s * A_BYTES + 16 * CHUNK_S + rl * 16) =      // kProj: the constant (1, 1) bias column only
+                pack_x((!kProj && s < n_slots && b < p.B) ? p.x + (b * T + (dir ? T - 1 : 0)) * p.I : nullptr, p.I);
+        }
+    } else {
+        for (int i = threadIdx.x; i < NT * kXCW * ROWS; i += blockDim.x) {      // buffer 0: the input columns of the first step
+            const int rl = i % ROWS, ch = (i / ROWS) % kXCW, s = i / (ROWS * kXCW);
+            const long long b = (long long)(tile0 + s) * 128 + rank * ROWS + rl;
+            *reinterpret_cast<uint4*>(a_s + s * A_BYTES + (16 + ch) * CHUNK_S + rl * 16) =
+                pack_x_chunk((s < n_slots && b < p.B) ? p.x + (b * T + (dir ? T - 1 : 0)) * p.I : nullptr, p.I, ch);
+        }
     }
     fence_proxy_async();
     if (warp == 0) mbar_wait(w_full, 0);
@@ -221,7 +240,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                         tc_fence_after();
                     }
                     if (elect_one()) {
-                        const uint32_t a_addr = smem_u32(a_s + s * A_FWD_BYTES);
+                        const uint32_t a_addr = smem_u32(a_s + s * A_BYTES);
                         const uint32_t d = tmem_base + s * 256;
                         for (int part = 0; part <= p.split; ++part) {     // split weights: h . W_hi^T + h . W_lo^T, same A tile
 #pragma unroll
@@ -234,12 +253,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                                 tc_mma_bf16_pair(d + 128, da, db1, idesc128, (k | part) != 0);     // W_hn h -> columns [128, 192)
                             }
                         }
-                        if (fused_x) {      // layer 0: W_ih x + b as one more K = 16 step of hi / lo split operands
-                            const uint64_t da = umma_desc_noswz(a_addr + 16 * CHUNK_S, CHUNK_S, 128);
-                            const uint64_t db0 = umma_desc_noswz(w_addr + n_hid * W_CHUNK, W_CHUNK, 128);
-                            const uint64_t db1 = umma_desc_noswz(w_addr + n_hid * W_CHUNK + 128 * 16, W_CHUNK, 128);
-                            tc_mma_bf16_pair(d, da, db0, idesc256, 1u);
-                            tc_mma_bf16_pair(d + 192, da, db1, idesc128, 0u);         // W_in x + b_in -> columns [192, 256)
+                        if (fused_x) {      // layer 0: W_ih x + b as kXS more K = 16 steps of hi / lo split operands
+#pragma unroll
+                            for (int k = 0; k < kXS; ++k) {
+                                const uint64_t da = umma_desc_noswz(a_addr + (16 + 2 * kXS * (kXB == 2 ? (step & 1) : 0) + 2 * k) * CHUNK_S, CHUNK_S, 128);
+                                const uint64_t db0 = umma_desc_noswz(w_addr + (n_hid + 2 * k) * W_CHUNK, W_CHUNK, 128);
+                                const uint64_t db1 = umma_desc_noswz(w_addr + (n_hid + 2 * k) * W_CHUNK + 128 * 16, W_CHUNK, 128);
+                                tc_mma_bf16_pair(d, da, db0, idesc256, 1u);
+                                tc_mma_bf16_pair(d + 192, da, db1, idesc128, k != 0);     // W_in x + b_in -> columns [192, 256)
+                            }
                         }
                         tc_commit_pair(&acc_full[s]);
                     }
@@ -295,10 +317,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
         const bool live = b < p.B;
         const int ub = uh * 64 + wg * UPT;                 // first hidden unit of this thread
         const uint32_t taddr0 = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + s * 256 + wg * UPT;
-        uint8_t* a_row = a_s + s * A_FWD_BYTES + rl * 16;
+        uint8_t* a_row = a_s + s * A_BYTES + rl * 16;
         uint8_t* h32_row = h32_s + s * H32_BYTES + rl * 16;
         const uint32_t hr_remote = mapa_cluster(smem_u32(&h_ready[s]), 0);
         const float* xrow = (kMode == 1 && p.x) ? p.x + b * T * p.I : nullptr;
+        constexpr int X_NTH = 128 / UPT;                   // threads per row (both lane halves)
+        const int x_ui = ub / UPT;                         // this thread's place among them
         const int len = (kVarLen && live) ? p.lengths[b] : T;
         const float dscale = kDrop ? __ldg(p.drop_scale) : 1.0f;
         float hreg[kRegState ? UPT : 1];
@@ -340,10 +364,25 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
             o_cur += o_step;
             if (!kFusedX) p_cur += p_step;
             if (g_cur) g_cur += g_step;
+            // input columns of step t+1, loaded and packed before the wait.  I <= 2: one chunk, by the row's thread of units
+            // 0.., stored after the epilogue; else chunk ch by the row's thread ch % X_NTH (a warp-uniform test: every chunk
+            // index stays a compile-time constant, and so does its column map), stored at once into the other buffer
             uint4 xnext = make_uint4(0, 0, 0, 0);
             const bool write_x = kMode == 1 && ub == 0 && step + 1 < T;
             const uint32_t taddr = taddr0 + (kProj ? (step & 1) * 256 : 0);
-            if (write_x) xnext = pack_x(live ? xrow + (long long)(dir ? t - 1 : t + 1) * p.I : nullptr, p.I);
+            if (kXC == 1) {
+                if (write_x) xnext = pack_x(live ? xrow + (long long)(dir ? t - 1 : t + 1) * p.I : nullptr, p.I);
+            } else if (step + 1 < T) {
+                const float* xp = live ? xrow + (long long)(dir ? t - 1 : t + 1) * p.I : nullptr;
+                uint8_t* xbuf = a_row + (16 + 2 * kXS * ((step + 1) & 1)) * CHUNK_S;
+#define RS_PUT_X(U)                                                                                                     \
+    case U:                                                                                                             \
+        if (U < kXCW) *reinterpret_cast<uint4*>(xbuf + (U) * CHUNK_S) = pack_x_chunk(xp, p.I, U);                      \
+        if (U + X_NTH < kXCW) *reinterpret_cast<uint4*>(xbuf + (U + X_NTH) * CHUNK_S) = pack_x_chunk(xp, p.I, U + X_NTH); \
+        break
+                switch (x_ui) { RS_PUT_X(0); RS_PUT_X(1); RS_PUT_X(2); RS_PUT_X(3); RS_PUT_X(4); RS_PUT_X(5); RS_PUT_X(6); RS_PUT_X(7); }
+#undef RS_PUT_X
+            }
             if (!kFusedX) load_p(pblk, 0);
             mbar_wait(&acc_full[s], step & 1);
             tc_fence_after();
@@ -423,7 +462,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                     last_n[grp - kDefer0] = sn;
                 }
             }
-            if (write_x) *reinterpret_cast<uint4*>(a_row + 16 * CHUNK_S) = xnext;
+            if (kXC == 1 && write_x) *reinterpret_cast<uint4*>(a_row + 16 * CHUNK_S) = xnext;
             fence_proxy_async();        // h_t written with ordinary stores -> visible to the tensor core of this SM
             tc_fence_before();          // TMEM reads done before the next MMA overwrites the accumulator
             __syncwarp();
@@ -842,28 +881,42 @@ int rec_fwd_pair(const float* x, int I, const void* P, const void* X, const void
     p.B = B; p.T = T; p.n_tiles = (B + 127) / 128; p.pf_dist = pf_dist; p.split = split ? 1 : 0;
     const int mode = X ? 2 : (x ? 1 : 0);
     if (mode == 2) nt = 1;                  // the fused projection runs one tile per pair (two waves above 37 tiles)
+    const int xc = mode == 1 ? x_chunks(I) : 1;     // layer 0: 16-byte input chunks per row (kXC of the kernel)
+    const int xs = (xc + 1) / 2;                    // input K steps
+    auto smem_of = [&](int nt_) {
+        return (16 * (1 + p.split) + (mode ? 2 * xs : 0)) * W_CHUNK + (mode == 2 ? 32 * W_CHUNK + 32 * CHUNK_S : 0)
+               + nt_ * (16 + 2 * xs * (xc == 1 ? 1 : 2)) * CHUNK_S + (nt_ == 1 ? 0 : nt_ * H32_BYTES) + H * 4 + 256;
+    };
+    // split weights with 3 or 4 input K steps (I >= 11) and two tiles in flight need 235 / 245 KB: one tile per pair then
+    if (nt == 2 && smem_of(2) > 227 * 1024) nt = 1;
     const int pairs = (p.n_tiles + nt - 1) / nt;
-    const int smem = (16 * (1 + p.split) + (mode ? 2 : 0)) * W_CHUNK + (mode == 2 ? 32 * W_CHUNK + 32 * CHUNK_S : 0) + nt * A_FWD_BYTES
-                     + (nt == 1 ? 0 : nt * H32_BYTES) + H * 4 + 256;
+    const int smem = smem_of(nt);
     const dim3 grid(2 * pairs, 2);
-#define RS_LAUNCH_FWD_D(NT_, VL_, MODE_, DROP_)                                                                         \
+#define RS_LAUNCH_FWD_D(NT_, VL_, MODE_, DROP_, XC_)                                                                    \
     do {                                                                                                                \
-        RS_CUDA_OK(cudaFuncSetAttribute(rec_fwd_pair_kernel<NT_, VL_, MODE_, DROP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        rec_fwd_pair_kernel<NT_, VL_, MODE_, DROP_><<<grid, NUM_THREADS, smem, stream>>>(p);                            \
+        RS_CUDA_OK(cudaFuncSetAttribute(rec_fwd_pair_kernel<NT_, VL_, MODE_, DROP_, XC_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+        rec_fwd_pair_kernel<NT_, VL_, MODE_, DROP_, XC_><<<grid, NUM_THREADS, smem, stream>>>(p);                       \
     } while (0)
-#define RS_LAUNCH_FWD(NT_, VL_, MODE_)                                                                                  \
+#define RS_LAUNCH_FWD_X(NT_, VL_, MODE_, XC_)                                                                           \
     do {                                                                                                                \
-        if (p.drop_bits) RS_LAUNCH_FWD_D(NT_, VL_, MODE_, true); else RS_LAUNCH_FWD_D(NT_, VL_, MODE_, false);          \
+        if (p.drop_bits) RS_LAUNCH_FWD_D(NT_, VL_, MODE_, true, XC_); else RS_LAUNCH_FWD_D(NT_, VL_, MODE_, false, XC_); \
     } while (0)
+#define RS_LAUNCH_FWD(NT_, VL_, MODE_) RS_LAUNCH_FWD_X(NT_, VL_, MODE_, 1)
 #define RS_LAUNCH_FWD_M(NT_, VL_)                                                                                       \
     do {                                                                                                                \
-        if (mode == 1) RS_LAUNCH_FWD(NT_, VL_, 1); else RS_LAUNCH_FWD(NT_, VL_, 0);                                     \
+        if (mode != 1) RS_LAUNCH_FWD(NT_, VL_, 0);                                                                      \
+        else if (xc == 1) RS_LAUNCH_FWD(NT_, VL_, 1);                                                                   \
+        else if (xc == 2) RS_LAUNCH_FWD_X(NT_, VL_, 1, 2);                                                              \
+        else if (xc == 4) RS_LAUNCH_FWD_X(NT_, VL_, 1, 4);                                                              \
+        else if (xc == 6) RS_LAUNCH_FWD_X(NT_, VL_, 1, 6);                                                              \
+        else RS_LAUNCH_FWD_X(NT_, VL_, 1, 8);                                                                           \
     } while (0)
     if (mode == 2) { if (lengths) RS_LAUNCH_FWD(1, true, 2); else RS_LAUNCH_FWD(1, false, 2); }
     else if (nt == 1) { if (lengths) RS_LAUNCH_FWD_M(1, true); else RS_LAUNCH_FWD_M(1, false); }
     else { if (lengths) RS_LAUNCH_FWD_M(2, true); else RS_LAUNCH_FWD_M(2, false); }
 #undef RS_LAUNCH_FWD_M
 #undef RS_LAUNCH_FWD
+#undef RS_LAUNCH_FWD_X
 #undef RS_LAUNCH_FWD_D
     count_launch();
     RS_CUDA_OK(cudaGetLastError());

@@ -26,7 +26,7 @@ constexpr int CHUNK_G = 2048;
 constexpr int CHUNK_S = ROWS * 16;
 constexpr int WSTAGE = 24576;                   // one ring stage: fwd 2 K steps x [2 chunks][384 rows][16 B], bwd 6 x [2][128][16 B]
 constexpr int NSTAGE_MAX = 7;                  // ring depth: 5 stages next to the fp32 master state in shared memory, 7 when it lives in TMEM
-constexpr int A_FWD_BYTES = (HW / 8 + 2) * CHUNK_S;     // 34 KB: h tile + the layer-0 input chunks
+constexpr int A_FWD_BYTES = (HW / 8 + 2) * CHUNK_S;     // 34 KB: h tile + the layer-0 input chunks of one K step
 constexpr int H32_BYTES = (HW / 4) * CHUNK_S;           // 64 KB: fp32 master copy of h
 constexpr int A_BWD_BYTES = (3 * HW / 8) * CHUNK_S;     // 96 KB: dGh tile
 constexpr int NUM_THREADS = 64 + 512;                   // warp 0: MMA issuer (even CTA) / ring relay (odd CTA), warp 1: ring producer
@@ -79,8 +79,15 @@ __device__ __forceinline__ void ring_relay(RingBars* rb, long long total, int NS
 
 // kVarLen / kDrop: packed variable-length traces / inter-layer dropout as template parameters (their selects, mask tests and the
 // masked copy cost instructions in the epilogue chain that bounds a time step even when unused)
-template <bool kFusedX, bool kVarLen, bool kDrop>
+// kXC (layer 0): the 16-byte input chunks per row of the (kXC + 1) / 2 input K steps (rec_common.cuh has the column map): 1
+// for I <= 2 (the one K step's second chunk stays zero), else x_chunks(I); the chunk ch is loaded and packed by the row's
+// thread ch (8 per row) before the wait for the accumulator and stored into the A tile after the epilogue.
+template <bool kFusedX, bool kVarLen, bool kDrop, int kXC = 1>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_fwd_wide_kernel(const FwdWideParams p) {
+    static_assert(kXC == 1 || (kFusedX && kXC % 2 == 0 && kXC <= 2 * x_steps(kMaxXInputs)), "input chunks per row");
+    constexpr int kXS = (kXC + 1) / 2;                     // input K steps
+    constexpr int A_BYTES = (HW / 8 + 2 * kXS) * CHUNK_S;  // h tile + the input chunks
+    constexpr int kXCW = kXC < x_col(kMaxXInputs - 1, 2) / 8 + 1 ? kXC : x_col(kMaxXInputs - 1, 2) / 8 + 1;  // chunks that can be nonzero
     // fp32 master copy of h: layer 0 needs all 512 TMEM columns for its accumulators (r | z | W_hn h | W_in x), so the state
     // lives in shared memory; deeper layers keep it in the 128 spare TMEM columns (64 KB of shared memory less: the L1 cache
     // that backs the epilogue's global loads grows by as much)
@@ -88,15 +95,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
     const int NSTAGE = p.nstage;
     extern __shared__ __align__(1024) uint8_t smem[];
     uint8_t* ring = smem;                                  // [NSTAGE][WSTAGE]
-    uint8_t* a_s = ring + NSTAGE * WSTAGE;                 // [34 chunks][64 rows][16 B]
-    uint8_t* h32_s = a_s + A_FWD_BYTES;                    // [64 chunks of 4 floats][64 rows][16 B]  (layer 0 only)
+    uint8_t* a_s = ring + NSTAGE * WSTAGE;                 // [32 + 2 kXS chunks][64 rows][16 B]
+    uint8_t* h32_s = a_s + A_BYTES;                        // [64 chunks of 4 floats][64 rows][16 B]  (layer 0 only)
     float* bhn_s = reinterpret_cast<float*>(h32_s + (kTmemState ? 0 : H32_BYTES));
     RingBars* rb = reinterpret_cast<RingBars*>(bhn_s + HW);
     uint64_t* h_ready = reinterpret_cast<uint64_t*>(rb + 1);
     uint64_t* acc_full = h_ready + 1;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 1);
 
-    constexpr int KS = HW / 16 + (kFusedX ? 1 : 0);        // K = 16 steps per time step
+    constexpr int KS = HW / 16 + (kFusedX ? kXS : 0);      // K = 16 steps per time step
     constexpr int SPS = (KS + 1) / 2;                      // ring stages per time step (2 K steps each)
     const uint32_t rank = cluster_ctarank();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -113,13 +120,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
     }
     if (warp == 0) tmem_alloc_pair<512>(tmem_slot);
     for (int i = threadIdx.x; i < HW; i += blockDim.x) bhn_s[i] = p.b_hn[dir * HW + i];
-    for (int i = threadIdx.x; i < (A_FWD_BYTES + (kTmemState ? 0 : H32_BYTES)) / 16; i += blockDim.x)
+    for (int i = threadIdx.x; i < (A_BYTES + (kTmemState ? 0 : H32_BYTES)) / 16; i += blockDim.x)
         reinterpret_cast<uint4*>(a_s)[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
-    if (kFusedX && threadIdx.x < ROWS) {
-        const long long b = (long long)tile * 128 + rank * ROWS + threadIdx.x;
-        *reinterpret_cast<uint4*>(a_s + (HW / 8) * CHUNK_S + threadIdx.x * 16) =
-            pack_x(b < p.B ? p.x + (b * T + (dir ? T - 1 : 0)) * p.I : nullptr, p.I);
+    if (kXC == 1) {
+        if (kFusedX && threadIdx.x < ROWS) {
+            const long long b = (long long)tile * 128 + rank * ROWS + threadIdx.x;
+            *reinterpret_cast<uint4*>(a_s + (HW / 8) * CHUNK_S + threadIdx.x * 16) =
+                pack_x(b < p.B ? p.x + (b * T + (dir ? T - 1 : 0)) * p.I : nullptr, p.I);
+        }
+    } else {
+        for (int i = threadIdx.x; i < kXCW * ROWS; i += blockDim.x) {
+            const int rl = i % ROWS, ch = i / ROWS;
+            const long long b = (long long)tile * 128 + rank * ROWS + rl;
+            *reinterpret_cast<uint4*>(a_s + (HW / 8 + ch) * CHUNK_S + rl * 16) =
+                pack_x_chunk(b < p.B ? p.x + (b * T + (dir ? T - 1 : 0)) * p.I : nullptr, p.I, ch);
+        }
     }
     fence_proxy_async();
     tc_fence_before();
@@ -185,7 +201,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                             } else {        // layer 0: the input chunks (hi / lo split x and bias against hi / lo split W_ih)
                                 tc_mma_bf16_pair(tmem_base, da, db_r, idesc, 1u);
                                 tc_mma_bf16_pair(tmem_base + 128, da, db_z, idesc, 1u);
-                                tc_mma_bf16_pair(tmem_base + 384, da, db_n, idesc, 0u);          // W_in x + b_in -> [384, 512)
+                                tc_mma_bf16_pair(tmem_base + 384, da, db_n, idesc, kXS == 1 ? 0u : (ks != HW / 16));   // W_in x + b_in -> [384, 512)
                             }
                         }
                         tc_commit_pair(&rb->empty[st]);
@@ -248,8 +264,17 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
             if (!kFusedX) p_cur += p_step;
             if (g_cur) g_cur += g_step;
             uint4 xnext = make_uint4(0, 0, 0, 0);
-            const bool write_x = kFusedX && ub == 0 && step + 1 < T;
-            if (write_x) xnext = pack_x(live ? xrow + (long long)(dir ? t - 1 : t + 1) * p.I : nullptr, p.I);
+            const int x_ui = ub / UPT;                     // this thread's place among the 8 of its row
+            const bool write_x = kFusedX && (kXC == 1 ? ub == 0 : x_ui < kXCW) && step + 1 < T;
+            if (write_x) {
+                const float* xp = live ? xrow + (long long)(dir ? t - 1 : t + 1) * p.I : nullptr;
+                if (kXC == 1) xnext = pack_x(xp, p.I);
+                else {              // chunk x_ui (a warp-uniform switch: the column map of each case is a compile-time constant)
+#define RS_PACK_X(U) case U: if (U < kXCW) xnext = pack_x_chunk(xp, p.I, U); break
+                    switch (x_ui) { RS_PACK_X(0); RS_PACK_X(1); RS_PACK_X(2); RS_PACK_X(3); RS_PACK_X(4); RS_PACK_X(5); RS_PACK_X(6); }
+#undef RS_PACK_X
+                }
+            }
             uint4 pv[3];
             auto load_p = [&](int grp) {
 #pragma unroll
@@ -330,7 +355,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                     last_o = so; last_d = sd; last_r = sr; last_z = sz; last_n = sn; last_h = sh;
                 }
             }
-            if (write_x) *reinterpret_cast<uint4*>(a_row + (HW / 8) * CHUNK_S) = xnext;
+            if (write_x) *reinterpret_cast<uint4*>(a_row + (HW / 8 + (kXC == 1 ? 0 : x_ui)) * CHUNK_S) = xnext;
             if (kTmemState) tmem_st_wait();
             fence_proxy_async();
             tc_fence_before();
@@ -607,9 +632,10 @@ int ring_stages(const char* env, int dflt, int max) {
 
 }  // namespace
 
-/* Forward for H = 256.  Wst: [2 dirs][2 ranks][9 or 8 stages][2 K steps][2 chunks][384 rows][8] bf16, rows = r | z | n gate rows
- * of hidden units [128 rank, 128 rank + 128) (r, z scaled by 1/2), K step k = hidden units [16 k, 16 k + 16); layer 0: K step
- * 16 = the input chunk of rs_rec_fwd_bf16 (w_hi, w_hi, w_lo per input, b_hi, b_lo) + a zero chunk, K step 17 = 0. */
+/* Forward for H = 256.  Wst: [2 dirs][2 ranks][8 + (x_steps(I) + 1) / 2 or 8 stages][2 K steps][2 chunks][384 rows][8] bf16,
+ * rows = r | z | n gate rows of hidden units [128 rank, 128 rank + 128) (r, z scaled by 1/2), K step k = hidden units
+ * [16 k, 16 k + 16); layer 0: K steps 16 .. 15 + x_steps(I) = the input columns (rec_common.cuh: W_ih hi, hi, lo per input,
+ * b_hi, b_lo), zero K steps up to the whole stage. */
 extern "C" int rs_rec_fwd_bf16_wide(const float* x, int I, const void* P, const void* Wst, const float* b_hn, void* out,
                                     void* gates, float* h_n, const int* lengths, const void* drop_bits,
                                     const float* drop_scale, void* out_drop, int B, int T, void* stream_) {
@@ -617,7 +643,8 @@ extern "C" int rs_rec_fwd_bf16_wide(const float* x, int I, const void* P, const 
     if (rs::check_device_sm100()) return 3;
     if (B == 0) return 0;
     RS_REQUIRE((x != nullptr) != (P != nullptr), "rs_rec_fwd_bf16_wide: exactly one of x (layer 0) and P (deeper layers) must be given");
-    RS_REQUIRE(!x || (I >= 1 && I <= 2), "rs_rec_fwd_bf16_wide: the MMA-fused input projection takes 1 or 2 input columns");
+    RS_REQUIRE(!x || (I >= 1 && I <= rs::kMaxXInputs), "rs_rec_fwd_bf16_wide: the MMA-fused input projection takes 1 to %d input columns (got %d)",
+               rs::kMaxXInputs, I);
     RS_REQUIRE(Wst && b_hn && out && h_n && B >= 0 && T >= 0, "rs_rec_fwd_bf16_wide: bad arguments");
     RS_REQUIRE((drop_bits != nullptr) == (out_drop != nullptr) && (!drop_bits || drop_scale), "rs_rec_fwd_bf16_wide: drop_bits, drop_scale and out_drop go together");
     if (T == 0) {
@@ -635,19 +662,25 @@ extern "C" int rs_rec_fwd_bf16_wide(const float* x, int I, const void* P, const 
     // Ring depth.  More stages hide more of the L2 latency of the weight stream but every 24 KB of shared memory is taken
     // from the L1 cache that backs the epilogue's global loads (measured, tools/c4_probe.py: see DESIGN.md 4.4)
     p.nstage = ring_stages(x ? "RS_WIDE_STAGES_FWD0" : "RS_WIDE_STAGES_FWD", 4, x ? 5 : 7);
-    const int smem = p.nstage * WSTAGE + (x ? H32_BYTES : 0) + A_FWD_BYTES + HW * 4 + (int)sizeof(RingBars) + 64;
+    const int xc = x ? rs::x_chunks(I) : 1;         // layer 0: 16-byte input chunks per row (kXC of the kernel)
+    const int smem = p.nstage * WSTAGE + (x ? H32_BYTES : 0) + (HW / 8 + 2 * ((xc + 1) / 2)) * CHUNK_S + HW * 4 + (int)sizeof(RingBars) + 64;
     const dim3 grid(2 * p.n_tiles, 2);
-#define RS_LAUNCH_FWDW(FX_, VL_, DROP_)                                                                                 \
+#define RS_LAUNCH_FWDW(FX_, VL_, DROP_, XC_)                                                                            \
     do {                                                                                                                \
-        RS_CUDA_OK(cudaFuncSetAttribute(rec_fwd_wide_kernel<FX_, VL_, DROP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        rec_fwd_wide_kernel<FX_, VL_, DROP_><<<grid, NUM_THREADS, smem, stream>>>(p);                                   \
+        RS_CUDA_OK(cudaFuncSetAttribute(rec_fwd_wide_kernel<FX_, VL_, DROP_, XC_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+        rec_fwd_wide_kernel<FX_, VL_, DROP_, XC_><<<grid, NUM_THREADS, smem, stream>>>(p);                              \
     } while (0)
-#define RS_LAUNCH_FWDW_V(FX_)                                                                                           \
+#define RS_LAUNCH_FWDW_V(FX_, XC_)                                                                                      \
     do {                                                                                                                \
-        if (lengths) { if (drop_bits) RS_LAUNCH_FWDW(FX_, true, true); else RS_LAUNCH_FWDW(FX_, true, false); }         \
-        else { if (drop_bits) RS_LAUNCH_FWDW(FX_, false, true); else RS_LAUNCH_FWDW(FX_, false, false); }               \
+        if (lengths) { if (drop_bits) RS_LAUNCH_FWDW(FX_, true, true, XC_); else RS_LAUNCH_FWDW(FX_, true, false, XC_); } \
+        else { if (drop_bits) RS_LAUNCH_FWDW(FX_, false, true, XC_); else RS_LAUNCH_FWDW(FX_, false, false, XC_); }     \
     } while (0)
-    if (x) RS_LAUNCH_FWDW_V(true); else RS_LAUNCH_FWDW_V(false);
+    if (!x) RS_LAUNCH_FWDW_V(false, 1);
+    else if (xc == 1) RS_LAUNCH_FWDW_V(true, 1);
+    else if (xc == 2) RS_LAUNCH_FWDW_V(true, 2);
+    else if (xc == 4) RS_LAUNCH_FWDW_V(true, 4);
+    else if (xc == 6) RS_LAUNCH_FWDW_V(true, 6);
+    else RS_LAUNCH_FWDW_V(true, 8);
 #undef RS_LAUNCH_FWDW_V
 #undef RS_LAUNCH_FWDW
     rs::count_launch();

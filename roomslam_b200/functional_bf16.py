@@ -24,6 +24,25 @@ from .functional import _need_cuda, _p, _stream, ktime
 
 H = 128
 
+# Layer-0 input columns (csrc/rec_common.cuh): W_ih x + b rides on the recurrence MMA as x_steps(I) extra K = 16 steps.
+# Input i takes the 3 columns x_col(i, 0..2) (x hi, lo, hi against W_ih hi, hi, lo), the bias columns 6 and 7 (1, 1 against
+# b hi, lo); every other column is zero.  Inputs 0, 1 and the bias fill the first 8 columns exactly as with 2 inputs.
+MAX_X_INPUTS = 16
+
+
+def x_col(i: int, k: int) -> int:
+    return 3 * i + k if i < 2 else 8 + 3 * (i - 2) + k
+
+
+def x_steps(I: int) -> int:
+    return (3 * I + 2 + 15) // 16
+
+
+def _check_x_inputs(I: int):
+    if I > MAX_X_INPUTS:
+        raise _lib.RoomSlamError(f"bf16 mode fuses the layer-0 projection into the recurrence for input_size <= {MAX_X_INPUTS} "
+                                 f"(got {I}); use precision='fp32'")
+
 
 def _nt(A, a_cols, kchunks, W_tiled, n_tiles, C, c_cols, c_chunk0, bias, n_blocks, st, drop=None, T=0):
     """drop = (bits, scale): the result is multiplied by that dropout mask in the epilogue (data gradient of a layer whose
@@ -153,15 +172,16 @@ class GRULayerBF16Fn(torch.autograd.Function):
             # 8192 traces: 5.85 -> 5.72, 6.83 -> 6.52, 9.55 -> 8.93, 19.6 -> 18.3 ms).  RS_FUSE_PROJ=0/1 forces.
             fuse_env = os.environ.get("RS_FUSE_PROJ")
             fuse_proj = padded_in and not split and (fuse_env == "1" if fuse_env in ("0", "1") else True)
-            whh_img = torch.empty(2, (H // 8) * (1 + split) + (2 if (not padded_in or fuse_proj) else 0), 3 * H, 8, device=dev, dtype=bf)
+            if not padded_in:
+                _check_x_inputs(Il)
+            x_chunks = 2 * x_steps(Il) if not padded_in else (2 if fuse_proj else 0)   # input columns (layer 0) / bias (fused)
+            whh_img = torch.empty(2, (H // 8) * (1 + split) + x_chunks, 3 * H, 8, device=dev, dtype=bf)
             b_hn = torch.empty(2, H, device=dev)
             bias_x = torch.empty(2, 3 * H, device=dev)
             wt = torch.empty(6 * H // 128, (Il // 64) * (1 + split), 8, L.TILE, 8, device=dev, dtype=bf) if (padded_in and not fuse_proj) else None
             wih_img = torch.empty(2, Il // 8, 3 * H, 8, device=dev, dtype=bf) if fuse_proj else None
             whhT_img = torch.empty(2, (3 * H // 8) * (1 + split), H, 8, device=dev, dtype=bf)
             wt_dgrad = torch.empty(Il // 128, (6 * H // 64) * (1 + split), 8, L.TILE, 8, device=dev, dtype=bf) if need_dx else None
-            if not padded_in and Il > 2:
-                raise _lib.RoomSlamError("bf16 mode fuses the layer-0 projection for input_size <= 2")
             if padded_in and Il != 2 * H:
                 raise _lib.RoomSlamError("bf16 mode: deeper layers take the 2H-column output of the layer below")
             wp = (ctypes.c_void_p * 8)(*[t.data_ptr() for t in ws])
@@ -233,7 +253,7 @@ class GRULayerBF16Fn(torch.autograd.Function):
             sums = torch.zeros(2, 4, H, device=dev)              # per direction: r | z | n | hn column sums of dG
             roles = []
             if not padded_in:
-                # layer 0: the input has 2 columns -> it rides along as the 16-column second B source of the hh roles
+                # layer 0: the input has <= 16 columns -> it rides along as the 16-column second B source of the r, z and n roles
                 xa_tm = torch.empty(tiles, T + 2, 2, L.TILE, 8, device=dev, dtype=torch.bfloat16)
                 _lib.call("rs_pack_x_tm", _p(saved_in), B, T, Il, _p(xa_tm), st)
                 dW_ih_buf = torch.zeros(6 * H, 16, device=dev)
@@ -319,19 +339,20 @@ class GRULayerBF16WideFn(torch.autograd.Function):
             for r in (0, 1):
                 img = rows(whs, r).view(2, 384, HW // 16, 2, 8).permute(0, 2, 3, 1, 4)          # [2][16 K steps][2 chunks][384][8]
                 if not padded_in:
-                    if Il > 2:
-                        raise _lib.RoomSlamError("bf16 mode fuses the layer-0 projection for input_size <= 2")
+                    _check_x_inputs(Il)
+                    xs = x_steps(Il)
                     w_hi = w_ih_fwd.to(bf).float()
                     b_hi = bias_x.to(bf).float()
-                    xcols = torch.zeros(2, 3 * HW, 16, device=dev)
+                    xcols = torch.zeros(2, 3 * HW, 16 * xs, device=dev)           # the input columns (see x_col)
                     for c in range(Il):
-                        xcols[:, :, 3 * c] = w_hi[:, :, c]
-                        xcols[:, :, 3 * c + 1] = w_hi[:, :, c]
-                        xcols[:, :, 3 * c + 2] = w_ih_fwd[:, :, c] - w_hi[:, :, c]
+                        xcols[:, :, x_col(c, 0)] = w_hi[:, :, c]
+                        xcols[:, :, x_col(c, 1)] = w_hi[:, :, c]
+                        xcols[:, :, x_col(c, 2)] = w_ih_fwd[:, :, c] - w_hi[:, :, c]
                     xcols[:, :, 6] = b_hi
                     xcols[:, :, 7] = bias_x - b_hi
-                    xstep = rows(xcols, r).view(2, 384, 1, 2, 8).permute(0, 2, 3, 1, 4)         # the input K step
-                    img = torch.cat([img, xstep, torch.zeros_like(xstep)], 1)                   # + a zero K step: 9 full stages
+                    xstep = rows(xcols, r).view(2, 384, xs, 2, 8).permute(0, 2, 3, 1, 4)        # the input K steps
+                    pad = torch.zeros(2, xs % 2, 2, 384, 8, device=dev)                          # + a zero K step: full stages
+                    img = torch.cat([img, xstep, pad], 1)
                 per_rank.append(img)
             wst = torch.stack(per_rank, 1).to(bf).contiguous()                     # [2 dirs][2 ranks][K steps][2][384][8]
             out = L.empty_tm(B, T, 2 * HW, dev, zero_pads=False)

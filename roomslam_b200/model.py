@@ -6,7 +6,9 @@ CPU oracle (oracle/room_slam_ref.py), so `cuda_model.load_state_dict(oracle.stat
 and checkpoints interchange.  The arithmetic runs in libroomslam_b200.so; nothing falls back to torch ops.
 
 precision="fp32": CUDA-core kernels, parity 1e-4 relative to torch's CPU path.
-precision="bf16": tcgen05 tensor-core kernels (bf16 operands, fp32 accumulate), parity 2e-2.
+precision="bf16": tcgen05 tensor-core kernels (bf16 operands, fp32 accumulate), parity 2e-2; hidden_size 128 or 256 and
+                  input_size <= 16 (the layer-0 projection rides on the recurrence MMA; wider inputs: precision="fp32").
+precision="auto": bf16 from 256 traces per step when hidden_size is 128 or 256 and input_size <= 2, fp32 otherwise.
 """
 from __future__ import annotations
 
