@@ -858,7 +858,7 @@ namespace rs {
 // Forward: NT = 1 while every tile can have its own pair of SMs in both directions (<= 37 tiles), else NT = 2 (the MMA of one
 // tile runs under the epilogue of the other).  The backward kernel is built for one tile per pair only: its epilogue is bound
 // by the latency of its gate / d_out loads, which two waves of half-size CTAs hide better than two tiles on one
-// register-capped CTA.  RS_REC_MODE=2 / 3 forces NT = 1 / 2 (tests run both).
+// register-capped CTA.  RS_REC_MODE=2 / 3 forces NT = 1 / 2 (tests/test_rec_kernels_gpu.py runs both).
 int rec_fwd_nt(int B) {
     const int mode = rec_mode();
     if (mode == 2) return 1;

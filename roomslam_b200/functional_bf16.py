@@ -296,6 +296,58 @@ class GRULayerBF16Fn(torch.autograd.Function):
         return (d_xin, None, None, dW_ih[:3 * H], dW_hh[0], db_ih[0], db_hh[0], dW_ih[3 * H:], dW_hh[1], db_ih[1], db_hh[1])
 
 
+def wide_fwd_image(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, layer0: bool):
+    """The forward operands of GRULayerBF16WideFn from the fp32 master weights (torch.nn.GRU layout, both directions):
+    -> (wst, b_hn, bias_x, w_ih_fwd, w_ih_cat, w_hh_cat).  wst is the streaming W_hh image of rs_rec_fwd_bf16_wide
+    [2 dirs][2 ranks][K steps][2][384][8] bf16 (r, z rows scaled by 1/2; layer 0: then the input columns of x_col, hi / lo
+    split, and a zero K step up to whole stages); b_hn [2][H]; bias_x [2][3H] (b_ih + b_hh on r, z, b_ih on n, scaled like
+    the rows); w_ih_fwd [2][3H][I] the scaled W_ih of the projection GEMM; w_ih_cat [6H][I] and w_hh_cat [2][3H][H] unscaled."""
+    HW = w_hh.shape[1]
+    dev, bf = w_hh.device, torch.bfloat16
+    Il = w_ih.shape[1]
+    half = torch.ones(3 * HW, device=dev)
+    half[:2 * HW] = 0.5
+    w_hh_cat = torch.stack([w_hh, w_hh_r], 0).float()                      # [2, 3H, H]
+    w_ih_cat = torch.cat([w_ih, w_ih_r], 0).float()                        # [6H, Il]
+    b_hn = torch.stack([b_hh[2 * HW:], b_hh_r[2 * HW:]], 0).float().contiguous()
+    bias_x = torch.stack([b_ih, b_ih_r], 0).float().clone()
+    bias_x[0, :2 * HW] += b_hh[:2 * HW]
+    bias_x[1, :2 * HW] += b_hh_r[:2 * HW]
+    bias_x *= half[None, :]
+    whs = w_hh_cat * half[None, :, None]
+    w_ih_fwd = (w_ih_cat.view(2, 3 * HW, Il) * half[None, :, None])
+    rows = lambda t, r: torch.cat([t[:, g * HW + 128 * r: g * HW + 128 * r + 128] for g in range(3)], 1)   # noqa: E731
+    per_rank = []
+    for r in (0, 1):
+        img = rows(whs, r).view(2, 384, HW // 16, 2, 8).permute(0, 2, 3, 1, 4)          # [2][16 K steps][2 chunks][384][8]
+        if layer0:
+            xs = x_steps(Il)
+            w_hi = w_ih_fwd.to(bf).float()
+            b_hi = bias_x.to(bf).float()
+            xcols = torch.zeros(2, 3 * HW, 16 * xs, device=dev)           # the input columns (see x_col)
+            for c in range(Il):
+                xcols[:, :, x_col(c, 0)] = w_hi[:, :, c]
+                xcols[:, :, x_col(c, 1)] = w_hi[:, :, c]
+                xcols[:, :, x_col(c, 2)] = w_ih_fwd[:, :, c] - w_hi[:, :, c]
+            xcols[:, :, 6] = b_hi
+            xcols[:, :, 7] = bias_x - b_hi
+            xstep = rows(xcols, r).view(2, 384, xs, 2, 8).permute(0, 2, 3, 1, 4)        # the input K steps
+            pad = torch.zeros(2, xs % 2, 2, 384, 8, device=dev)                          # + a zero K step: full stages
+            img = torch.cat([img, xstep, pad], 1)
+        per_rank.append(img)
+    wst = torch.stack(per_rank, 1).to(bf).contiguous()                     # [2 dirs][2 ranks][K steps][2][384][8]
+    return wst, b_hn, bias_x, w_ih_fwd, w_ih_cat, w_hh_cat
+
+
+def wide_bwd_image(w_hh_cat):
+    """W_hh^T as rs_rec_bwd_bf16_wide streams it: [2 dirs][2 ranks][48 K steps][2 chunks][128 rows][8] bf16, rows = hidden
+    units [128 rank, 128 rank + 128), K = the 3H gate rows r | z | n (unscaled)."""
+    HW = w_hh_cat.shape[2]
+    whhT = w_hh_cat.transpose(1, 2)                                        # [2, H, 3H]
+    return torch.stack([whhT[:, 128 * r: 128 * r + 128].reshape(2, 128, 3 * HW // 16, 2, 8).permute(0, 2, 3, 1, 4)
+                        for r in (0, 1)], 1).to(torch.bfloat16).contiguous()   # [2][2][48 K steps][2][128][8]
+
+
 class GRULayerBF16WideFn(torch.autograd.Function):
     """GRULayerBF16Fn for hidden_size = 256 (BASELINE config 4).  Same tile-major operands and the same GEMM kernels; the
     recurrence runs on csrc/rec_wide.cu, which streams W_hh from L2 (it no longer fits in shared memory).  The GEMM calls are
@@ -323,38 +375,10 @@ class GRULayerBF16WideFn(torch.autograd.Function):
         need_grad = any(ctx.needs_input_grad)
         tiles, Il = L.n_tiles(B), w_ih.shape[1]
         with torch.no_grad():
-            half = torch.ones(3 * HW, device=dev)
-            half[:2 * HW] = 0.5
-            w_hh_cat = torch.stack([w_hh, w_hh_r], 0).float()                      # [2, 3H, H]
-            w_ih_cat = torch.cat([w_ih, w_ih_r], 0).float()                        # [6H, Il]
-            b_hn = torch.stack([b_hh[2 * HW:], b_hh_r[2 * HW:]], 0).float().contiguous()
-            bias_x = torch.stack([b_ih, b_ih_r], 0).float().clone()
-            bias_x[0, :2 * HW] += b_hh[:2 * HW]
-            bias_x[1, :2 * HW] += b_hh_r[:2 * HW]
-            bias_x *= half[None, :]
-            whs = w_hh_cat * half[None, :, None]
-            w_ih_fwd = (w_ih_cat.view(2, 3 * HW, Il) * half[None, :, None])
-            rows = lambda t, r: torch.cat([t[:, g * HW + 128 * r: g * HW + 128 * r + 128] for g in range(3)], 1)   # noqa: E731
-            per_rank = []
-            for r in (0, 1):
-                img = rows(whs, r).view(2, 384, HW // 16, 2, 8).permute(0, 2, 3, 1, 4)          # [2][16 K steps][2 chunks][384][8]
-                if not padded_in:
-                    _check_x_inputs(Il)
-                    xs = x_steps(Il)
-                    w_hi = w_ih_fwd.to(bf).float()
-                    b_hi = bias_x.to(bf).float()
-                    xcols = torch.zeros(2, 3 * HW, 16 * xs, device=dev)           # the input columns (see x_col)
-                    for c in range(Il):
-                        xcols[:, :, x_col(c, 0)] = w_hi[:, :, c]
-                        xcols[:, :, x_col(c, 1)] = w_hi[:, :, c]
-                        xcols[:, :, x_col(c, 2)] = w_ih_fwd[:, :, c] - w_hi[:, :, c]
-                    xcols[:, :, 6] = b_hi
-                    xcols[:, :, 7] = bias_x - b_hi
-                    xstep = rows(xcols, r).view(2, 384, xs, 2, 8).permute(0, 2, 3, 1, 4)        # the input K steps
-                    pad = torch.zeros(2, xs % 2, 2, 384, 8, device=dev)                          # + a zero K step: full stages
-                    img = torch.cat([img, xstep, pad], 1)
-                per_rank.append(img)
-            wst = torch.stack(per_rank, 1).to(bf).contiguous()                     # [2 dirs][2 ranks][K steps][2][384][8]
+            if not padded_in:
+                _check_x_inputs(Il)
+            wst, b_hn, bias_x, w_ih_fwd, w_ih_cat, w_hh_cat = wide_fwd_image(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r,
+                                                                             not padded_in)
             out = L.empty_tm(B, T, 2 * HW, dev, zero_pads=False)
             out_drop = L.empty_tm(B, T, 2 * HW, dev, zero_pads=False) if drop is not None else None
             d_bits, d_scale = drop if drop is not None else (None, None)
@@ -401,9 +425,7 @@ class GRULayerBF16WideFn(torch.autograd.Function):
         with torch.no_grad():
             d_out = d_out.contiguous().to(bf) if d_out is not None else None
             d_h_n = d_h_n.contiguous().float() if d_h_n is not None else None
-            whhT = w_hh_cat.transpose(1, 2)                                        # [2, H, 3H]
-            wtst = torch.stack([whhT[:, 128 * r: 128 * r + 128].reshape(2, 128, 3 * HW // 16, 2, 8).permute(0, 2, 3, 1, 4)
-                                for r in (0, 1)], 1).to(bf).contiguous()           # [2][2][48 K steps][2][128][8]
+            wtst = wide_bwd_image(w_hh_cat)
             dG = torch.empty(tiles, T + 2, 8 * HC, L.TILE, 8, device=dev, dtype=bf)
             d_bits, d_scale = ctx.drop if (ctx.drop is not None and ctx.mask_d_out) else (None, None)
             with ktime("rec_bwd_wide_kernel", 2.0 * B * T * 2 * 3 * HW * HW):
