@@ -281,3 +281,34 @@ def weight_grads(dG, x_seq, h_prev) -> dict:
     hh = dG[:, :, :, [0, 1, 3]].flatten(3)
     return {"w_ih": torch.einsum("dbtg,dbti->dgi", ih, x_seq), "w_hh": torch.einsum("dbtg,dbtk->dgk", hh, h_prev),
             "b_ih": ih.sum((1, 2)), "b_hh": hh.sum((1, 2))}
+
+
+# ---------------------------------------------------------------------------------- operands and outputs of the GEMMs
+def x_operand(x: torch.Tensor, Bp: int, T: int) -> torch.Tensor:
+    """What rs_pack_x_tm writes for the layer-0 input x (B, T, I <= 16) fp32, decoded: (Bp, T + 2, 16) float64 holding
+    bf16(x) in columns < I, and zeros in the columns >= I, the pad rows t' = 0, T + 1 and the pad traces b >= B."""
+    B, _, I = x.shape
+    xo = torch.zeros(Bp, T + 2, 16, dtype=F64, device=x.device)
+    xo[:B, 1:T + 1, :I] = bf16(x.float()).to(F64)
+    return xo
+
+
+def data_grad(dG_full: torch.Tensor, w_ih: torch.Tensor, drop: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """dX of a deeper layer over all T + 2 rows, what rs_blk_gemm_nt(_drop) computes from dG before its bf16 rounding:
+    sum over both directions and the r, z, n blocks of dG W_ih.  dG_full (2, Bp, T + 2, 4, H) (dG_full, pad rows kept);
+    w_ih (2, 3H, I): W_ih as the dgrad image holds it (unscaled; bf16, or hi + lo with split); drop (Bp, T, I) or None:
+    the multiplier (0 or scale) of the dropout on the layer input, applied at rows 1 .. T only.  -> (Bp, T + 2, I).
+    With an exact fp32 sum the kernel's result is bf16(fp32(this)): the product of the fp32 sum and the fp32 scale is exact
+    in float64, so one rounding to fp32 is the kernel's fp32 multiply."""
+    dx = sum(dG_full[d, :, :, :3].flatten(2) @ w_ih[d] for d in (0, 1))
+    if drop is not None:
+        dx[:, 1:-1] = dx[:, 1:-1] * drop
+    return dx
+
+
+def projection(X_full: torch.Tensor, w_ih: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
+    """P = X W_ih^T + b over all rows, what rs_blk_gemm_nt computes for the input projection before its bf16 rounding.
+    X_full (Bp, T + 2, I) (tm_full of the layer input, pad rows kept); w_ih (2, 3H, I): the weights as the projection
+    image holds them (r, z rows halved; bf16, or hi + lo with split); bias (2, 3H): the fp32 bias the epilogue adds
+    (bias_x).  -> (Bp, T + 2, 6H), per direction r | z | n."""
+    return torch.cat([X_full @ w_ih[d].T + bias[d] for d in (0, 1)], -1)

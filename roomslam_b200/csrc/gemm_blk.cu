@@ -164,7 +164,7 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
                     uint32_t mbits = 0xffffffffu;           // 4 chunks x 8 columns
                     if (drow) mbits = __ldg(reinterpret_cast<const uint32_t*>(drow + p.c_chunk0 + n * 16 + chalf * 8 + c0 / 8));
                     rs::tmem_ld_wait();
-                    if (p.drop_bits) {
+                    if (drow) {                             // the pad rows have no mask: left unscaled, as without dropout
 #pragma unroll
                         for (int e = 0; e < 32; ++e)
                             r[e] = ((mbits >> e) & 1u) ? __float_as_uint(__uint_as_float(r[e]) * dscale) : 0u;
@@ -812,8 +812,10 @@ extern "C" int rs_blk_wgrad(const void* dG, int64_t a_cols, const void* ones_blo
     RS_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     const int items = n_roles * p.splits;
     int grid = items < num_sms() ? items : num_sms();
-    // paired mode: roles 2 j and 2 j + 1 form a cluster; where they name the same dG columns the block is loaded once (multicast)
-    static const bool pair_off = getenv("RS_WGRAD_PAIR") && atoi(getenv("RS_WGRAD_PAIR")) == 0;
+    // paired mode: roles 2 j and 2 j + 1 form a cluster; where they name the same dG columns the block is loaded once (multicast).
+    // RS_WGRAD_PAIR=0 launches every role as a single CTA instead.  Read on every call (as RS_REC_MODE is), so one process can
+    // run both modes: tests/test_grad_gemm_gpu.py requires them to give the same values.
+    const bool pair_off = getenv("RS_WGRAD_PAIR") && atoi(getenv("RS_WGRAD_PAIR")) == 0;
     unsigned int share = 0;
     if (n_roles % 2 == 0 && !pair_off)
         for (int r = 0; r < n_roles; r += 2)

@@ -246,54 +246,64 @@ class GRULayerBF16Fn(torch.autograd.Function):
                 d_bits, d_scale = ctx.drop if (ctx.drop is not None and ctx.mask_d_out) else (None, None)
                 _lib.call("rs_rec_bwd_bf16", _p(d_out), _p(d_h_n), _p(gates), _p(out), _p(whhT_img), _p(whh_img), whh_img.shape[1],
                           _p(b_hn), _p(dG), _p(ctx.lengths), _p(d_bits), _p(d_scale), split, B, T, st)
-            # ALL weight / bias gradients of the layer in one fused pass over dG (12 roles, see csrc/gemm_blk.cu):
-            #   ih roles (dir, g in r,z,n): dG block ^T . X            -> dW_ih rows, bias sums of r, z, n
-            #   hh roles (dir, g in r,z,hn): dG block ^T . h(t' -/+ 1) -> dW_hh rows, bias sum of hn
-            dW_hh = torch.zeros(2, 3 * H, H, device=dev)
-            sums = torch.zeros(2, 4, H, device=dev)              # per direction: r | z | n | hn column sums of dG
-            roles = []
-            if not padded_in:
-                # layer 0: the input has <= 16 columns -> it rides along as the 16-column second B source of the r, z and n roles
-                xa_tm = torch.empty(tiles, T + 2, 2, L.TILE, 8, device=dev, dtype=torch.bfloat16)
-                _lib.call("rs_pack_x_tm", _p(saved_in), B, T, Il, _p(xa_tm), st)
-                dW_ih_buf = torch.zeros(6 * H, 16, device=dev)
-                for d in (0, 1):
-                    sh = -1 if d == 0 else 1
-                    for g in (0, 1):                               # r, z: hidden-side block + input-side columns + bias sum
-                        roles.append((d * 64 + g * 16, out, 2 * H, d * 16, H, sh, dW_hh[d, g * H:], H, sums[d, g],
-                                      xa_tm, dW_ih_buf[(d * 3 + g) * H:]))
-                    roles.append((d * 64 + 48, out, 2 * H, d * 16, H, sh, dW_hh[d, 2 * H:], H, sums[d, 3], None, None))   # hn
-                    roles.append((d * 64 + 32, None, 0, 0, 0, 0, None, 0, sums[d, 2], xa_tm, dW_ih_buf[(d * 3 + 2) * H:]))  # n
-                flops = 2.0 * tiles * L.TILE * T * (6 * H * 16 + 6 * H * H + 8 * H * 16)
-            else:
-                # deeper layers: 12 roles: ih (N = 2H) and hh (N = H) per gate block.  (18 equal-weight N = H roles were
-                # tried to keep the roles in lockstep for L2 sharing: slower, 6.1 ms vs 5.5 ms - more L2->SM traffic.)
-                # Roles 2 j, 2 j + 1 run as a CTA pair; where both name the same dG block (r, z) it is loaded once and
-                # multicast into both CTAs (csrc/gemm_blk.cu, paired mode).
-                dW_ih_buf = torch.zeros(6 * H, Il, device=dev)
-                for d in (0, 1):
-                    sh = -1 if d == 0 else 1
-                    ih = lambda g: (d * 64 + g * 16, saved_in, Il, 0, Il, 0, dW_ih_buf[(d * 3 + g) * H:], Il, sums[d, g], None, None)  # noqa: E731
-                    hh = lambda gi, g: (d * 64 + g * 16, out, 2 * H, d * 16, H, sh, dW_hh[d, gi * H:], H,                           # noqa: E731
-                                        sums[d, 3] if g == 3 else None, None, None)
-                    roles += [ih(0), hh(0, 0), ih(1), hh(1, 1), ih(2), hh(2, 3)]   # (r, X) (r, h) | (z, X) (z, h) | (n, X) (hn, h)
-                flops = 2.0 * tiles * L.TILE * T * (6 * H * Il + 6 * H * H + 8 * H * 16)
-            with ktime("blk_wgrad_kernel", flops):
-                _wgrad(dG, 8 * H, _ones_block(dev), roles, tiles, T, st)
-            db_ih = sums[:, :3].reshape(2, 3 * H)
-            db_hh = torch.cat([sums[:, :2].reshape(2, 2 * H), sums[:, 3]], 1)
-            dW_ih = dW_ih_buf[:, :Il].contiguous() if not padded_in else dW_ih_buf
-            d_xin = None
-            if padded_in:
-                X = saved_in
-                if ctx.needs_input_grad[0]:
-                    dX = torch.empty(tiles, T + 2, Il // 8, L.TILE, 8, device=dev, dtype=torch.bfloat16)
-                    wt = wt_dgrad                                                  # [Il/128][12][8][128][8]
-                    kch = [d * 64 + g * 16 + hf * 8 for d in (0, 1) for g in (0, 1, 2) for hf in (0, 1)]
-                    with ktime("blk_gemm_nt_kernel(dgrad)", 2.0 * tiles * L.TILE * (T + 2) * 6 * H * Il):
-                        _nt(dG, 8 * H, kch * (1 + split), wt, Il // 128, dX, Il, 0, None, tiles * (T + 2), st, ctx.in_drop, T)
-                    d_xin = dX
+            dW_ih, dW_hh, db_ih, db_hh, d_xin = grads_from_dG_128(dG, out, saved_in, padded_in, B, T, Il, split, wt_dgrad,
+                                                                  ctx.in_drop, padded_in and ctx.needs_input_grad[0])
+            dW_ih = dW_ih[:, :Il].contiguous() if not padded_in else dW_ih
         return (d_xin, None, None, dW_ih[:3 * H], dW_hh[0], db_ih[0], db_hh[0], dW_ih[3 * H:], dW_hh[1], db_ih[1], db_hh[1])
+
+
+def grads_from_dG_128(dG, out, saved_in, padded_in, B, T, Il, split, wt_dgrad, in_drop, need_dx):
+    """Everything GRULayerBF16Fn's backward computes from the BPTT's dG [tiles][T + 2][8H / 8][128][8] (per direction
+    r | z | n | hn): -> (dW_ih (6H, Il; layer 0: (6H, 16), the columns >= Il zero), dW_hh (2, 3H, H), db_ih (2, 3H), db_hh (2, 3H), dX tile-major or None), each
+    direction's rows in torch.nn.GRU's r | z | n order.  out: the layer's tile-major output; saved_in: the raw (B, T, Il)
+    fp32 input (layer 0, padded_in False) or the tile-major input X; wt_dgrad: the dgrad image of rs_gru_pack_weights_bf16
+    (used when need_dx); in_drop: (bits, scale) of the dropout on the layer input, applied to dX, or None."""
+    dev = dG.device
+    st = torch.cuda.current_stream(dev).cuda_stream
+    tiles = L.n_tiles(B)
+    # ALL weight / bias gradients of the layer in one fused pass over dG (12 roles, see csrc/gemm_blk.cu):
+    #   ih roles (dir, g in r,z,n): dG block ^T . X            -> dW_ih rows, bias sums of r, z, n
+    #   hh roles (dir, g in r,z,hn): dG block ^T . h(t' -/+ 1) -> dW_hh rows, bias sum of hn
+    dW_hh = torch.zeros(2, 3 * H, H, device=dev)
+    sums = torch.zeros(2, 4, H, device=dev)              # per direction: r | z | n | hn column sums of dG
+    roles = []
+    if not padded_in:
+        # layer 0: the input has <= 16 columns -> it rides along as the 16-column second B source of the r, z and n roles
+        xa_tm = torch.empty(tiles, T + 2, 2, L.TILE, 8, device=dev, dtype=torch.bfloat16)
+        _lib.call("rs_pack_x_tm", _p(saved_in), B, T, Il, _p(xa_tm), st)
+        dW_ih_buf = torch.zeros(6 * H, 16, device=dev)
+        for d in (0, 1):
+            sh = -1 if d == 0 else 1
+            for g in (0, 1):                               # r, z: hidden-side block + input-side columns + bias sum
+                roles.append((d * 64 + g * 16, out, 2 * H, d * 16, H, sh, dW_hh[d, g * H:], H, sums[d, g],
+                              xa_tm, dW_ih_buf[(d * 3 + g) * H:]))
+            roles.append((d * 64 + 48, out, 2 * H, d * 16, H, sh, dW_hh[d, 2 * H:], H, sums[d, 3], None, None))   # hn
+            roles.append((d * 64 + 32, None, 0, 0, 0, 0, None, 0, sums[d, 2], xa_tm, dW_ih_buf[(d * 3 + 2) * H:]))  # n
+        flops = 2.0 * tiles * L.TILE * T * (6 * H * 16 + 6 * H * H + 8 * H * 16)
+    else:
+        # deeper layers: 12 roles: ih (N = 2H) and hh (N = H) per gate block.  (18 equal-weight N = H roles were
+        # tried to keep the roles in lockstep for L2 sharing: slower, 6.1 ms vs 5.5 ms - more L2->SM traffic.)
+        # Roles 2 j, 2 j + 1 run as a CTA pair; where both name the same dG block (r, z) it is loaded once and
+        # multicast into both CTAs (csrc/gemm_blk.cu, paired mode).
+        dW_ih_buf = torch.zeros(6 * H, Il, device=dev)
+        for d in (0, 1):
+            sh = -1 if d == 0 else 1
+            ih = lambda g: (d * 64 + g * 16, saved_in, Il, 0, Il, 0, dW_ih_buf[(d * 3 + g) * H:], Il, sums[d, g], None, None)  # noqa: E731
+            hh = lambda gi, g: (d * 64 + g * 16, out, 2 * H, d * 16, H, sh, dW_hh[d, gi * H:], H,                           # noqa: E731
+                                sums[d, 3] if g == 3 else None, None, None)
+            roles += [ih(0), hh(0, 0), ih(1), hh(1, 1), ih(2), hh(2, 3)]   # (r, X) (r, h) | (z, X) (z, h) | (n, X) (hn, h)
+        flops = 2.0 * tiles * L.TILE * T * (6 * H * Il + 6 * H * H + 8 * H * 16)
+    with ktime("blk_wgrad_kernel", flops):
+        _wgrad(dG, 8 * H, _ones_block(dev), roles, tiles, T, st)
+    db_ih = sums[:, :3].reshape(2, 3 * H)
+    db_hh = torch.cat([sums[:, :2].reshape(2, 2 * H), sums[:, 3]], 1)
+    dX = None
+    if need_dx:
+        dX = torch.empty(tiles, T + 2, Il // 8, L.TILE, 8, device=dev, dtype=torch.bfloat16)
+        kch = [d * 64 + g * 16 + hf * 8 for d in (0, 1) for g in (0, 1, 2) for hf in (0, 1)]   # wt_dgrad: [Il/128][12][8][128][8]
+        with ktime("blk_gemm_nt_kernel(dgrad)", 2.0 * tiles * L.TILE * (T + 2) * 6 * H * Il):
+            _nt(dG, 8 * H, kch * (1 + split), wt_dgrad, Il // 128, dX, Il, 0, None, tiles * (T + 2), st, in_drop, T)
+    return dW_ih_buf, dW_hh, db_ih, db_hh, dX
 
 
 def wide_fwd_image(w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, layer0: bool):
@@ -394,13 +404,7 @@ class GRULayerBF16WideFn(torch.autograd.Function):
             else:
                 if Il != 2 * HW:
                     raise _lib.RoomSlamError("bf16 mode: deeper layers take the 2H-column output of the layer below")
-                P = torch.empty(tiles, T + 2, 6 * HW // 8, L.TILE, 8, device=dev, dtype=bf)
-                wt = L.tile_weight_nt(w_ih_fwd.reshape(6 * HW, Il))                # [12][Il/64][8][128][8]
-                bias_flat = bias_x.reshape(-1).contiguous()
-                with ktime("blk_gemm_nt_kernel(projection)", 2.0 * tiles * L.TILE * (T + 2) * 6 * HW * Il):
-                    for part in (0, 1):                                            # 1536 output columns: two launches of 768
-                        _nt(xin, Il, [8 * k for k in range(Il // 64)], wt[6 * part: 6 * part + 6].contiguous(), 6, P, 6 * HW,
-                            96 * part, bias_flat[768 * part: 768 * part + 768].contiguous(), tiles * (T + 2), st)
+                P = wide_projection(xin, w_ih_fwd, bias_x, B, T)
                 with ktime("rec_fwd_wide_kernel", rec_flops):
                     _lib.call("rs_rec_fwd_bf16_wide", 0, 0, _p(P), _p(wst), _p(b_hn), _p(out), _p(gates), _p(h_n), _p(lengths),
                               _p(d_bits), _p(d_scale), _p(out_drop), B, T, st)
@@ -431,52 +435,79 @@ class GRULayerBF16WideFn(torch.autograd.Function):
             with ktime("rec_bwd_wide_kernel", 2.0 * B * T * 2 * 3 * HW * HW):
                 _lib.call("rs_rec_bwd_bf16_wide", _p(d_out), _p(d_h_n), _p(gates), _p(out), _p(wtst), _p(dG), _p(ctx.lengths),
                           _p(d_bits), _p(d_scale), B, T, st)
-            dW_hh = torch.zeros(2, 3 * HW, HW, device=dev)
-            sums = torch.zeros(2, 4, HW, device=dev)             # per direction: r | z | n | hn column sums of dG
-            ones = _ones_block(dev)
-            if not padded_in:
-                xa_tm = torch.empty(tiles, T + 2, 2, L.TILE, 8, device=dev, dtype=bf)
-                _lib.call("rs_pack_x_tm", _p(saved_in), B, T, Il, _p(xa_tm), st)
-                dW_ih_buf = torch.zeros(6 * HW, 16, device=dev)
-            else:
-                dW_ih_buf = torch.zeros(6 * HW, Il, device=dev)
-            flops = 2.0 * tiles * L.TILE * T * (6 * HW * (Il if padded_in else 16) + 6 * HW * HW + 8 * HW * 16)
-            with ktime("blk_wgrad_kernel", flops):
-                for d in (0, 1):                                 # one launch per direction: <= 18 roles of one 128-row gate block
-                    sh = -1 if d == 0 else 1
-                    roles, hh_roles = [], []
-                    for mb in (0, 1):                            # the two 128-row halves of a 256-row gate block
-                        m0 = mb * 128
-                        if not padded_in:
-                            for g in (0, 1):
-                                roles.append((d * 4 * HC + g * HC + mb * 16, out, 2 * HW, d * HC, HW, sh, dW_hh[d, g * HW + m0:], HW,
-                                              sums[d, g, m0:], xa_tm, dW_ih_buf[(d * 3 + g) * HW + m0:]))
-                            roles.append((d * 4 * HC + 3 * HC + mb * 16, out, 2 * HW, d * HC, HW, sh, dW_hh[d, 2 * HW + m0:], HW,
-                                          sums[d, 3, m0:], None, None))
-                            roles.append((d * 4 * HC + 2 * HC + mb * 16, None, 0, 0, 0, 0, None, 0, sums[d, 2, m0:], xa_tm,
-                                          dW_ih_buf[(d * 3 + 2) * HW + m0:]))
-                        else:
-                            for g in (0, 1, 2):                  # r, z, n against the layer input, 256 columns at a time: the two
-                                for nb in range(Il // 256):      # halves of Il are adjacent roles = one CTA pair sharing its dG block
-                                    roles.append((d * 4 * HC + g * HC + mb * 16, saved_in, Il, nb * 32, 256, 0,
-                                                  dW_ih_buf[(d * 3 + g) * HW + m0:, nb * 256:], Il, sums[d, g, m0:] if nb == 0 else None,
-                                                  None, None))
-                            for gi, g in enumerate((0, 1, 3)):   # r, z, hn against the shifted hidden state
-                                hh_roles.append((d * 4 * HC + g * HC + mb * 16, out, 2 * HW, d * HC, HW, sh, dW_hh[d, gi * HW + m0:], HW,
-                                                 sums[d, 3, m0:] if g == 3 else None, None, None))
-                    _wgrad(dG, 8 * HW, ones, roles + hh_roles, tiles, T, st)
-            db_ih = sums[:, :3].reshape(2, 3 * HW)
-            db_hh = torch.cat([sums[:, :2].reshape(2, 2 * HW), sums[:, 3]], 1)
-            dW_ih = dW_ih_buf[:, :Il].contiguous() if not padded_in else dW_ih_buf
-            d_xin = None
-            if padded_in and ctx.needs_input_grad[0]:
-                dX = torch.empty(tiles, T + 2, Il // 8, L.TILE, 8, device=dev, dtype=bf)
-                wt = L.tile_weight_nt(w_ih_cat.t().contiguous())                   # [Il/128][6H/64][8][128][8]
-                kch = [d * 4 * HC + g * HC + hf * 8 for d in (0, 1) for g in (0, 1, 2) for hf in range(HW // 64)]
-                with ktime("blk_gemm_nt_kernel(dgrad)", 2.0 * tiles * L.TILE * (T + 2) * 6 * HW * Il):
-                    _nt(dG, 8 * HW, kch, wt, Il // 128, dX, Il, 0, None, tiles * (T + 2), st, ctx.in_drop, T)
-                d_xin = dX
+            dW_ih, dW_hh, db_ih, db_hh, d_xin = grads_from_dG_256(dG, out, saved_in, padded_in, B, T, Il, w_ih_cat, ctx.in_drop,
+                                                                  padded_in and ctx.needs_input_grad[0])
+            dW_ih = dW_ih[:, :Il].contiguous() if not padded_in else dW_ih
         return (d_xin, None, None, dW_ih[:3 * HW], dW_hh[0], db_ih[0], db_hh[0], dW_ih[3 * HW:], dW_hh[1], db_ih[1], db_hh[1])
+
+
+def wide_projection(X, w_ih_fwd, bias_x, B, T):
+    """The input projection of a deeper H = 256 layer: P = X W_ih^T + b over all T + 2 rows of the tile-major X (Il
+    columns), tile-major bf16 with 6H columns.  w_ih_fwd (2, 3H, Il) and bias_x (2, 3H) as wide_fwd_image returns them;
+    the 1536 output columns take two launches of 768 (the second writes from chunk 96 on)."""
+    HW, Il = GRULayerBF16WideFn.HW, X.shape[2] * 8
+    tiles = L.n_tiles(B)
+    P = torch.empty(tiles, T + 2, 6 * HW // 8, L.TILE, 8, device=X.device, dtype=torch.bfloat16)
+    wt = L.tile_weight_nt(w_ih_fwd.reshape(6 * HW, Il))                # [12][Il/64][8][128][8]
+    bias_flat = bias_x.reshape(-1).contiguous()
+    with ktime("blk_gemm_nt_kernel(projection)", 2.0 * tiles * L.TILE * (T + 2) * 6 * HW * Il):
+        for part in (0, 1):
+            _nt(X, Il, [8 * k for k in range(Il // 64)], wt[6 * part: 6 * part + 6].contiguous(), 6, P, 6 * HW,
+                96 * part, bias_flat[768 * part: 768 * part + 768].contiguous(), tiles * (T + 2), _stream(X))
+    return P
+
+
+def grads_from_dG_256(dG, out, saved_in, padded_in, B, T, Il, w_ih_cat, in_drop, need_dx):
+    """grads_from_dG_128 for GRULayerBF16WideFn: the same outputs at H = 256.  w_ih_cat (6H, Il): the unscaled fp32 W_ih
+    of both directions (wide_fwd_image), whose bf16 image the dgrad multiplies."""
+    HW = GRULayerBF16WideFn.HW
+    dev, bf = dG.device, torch.bfloat16
+    st = torch.cuda.current_stream(dev).cuda_stream
+    tiles, HC = L.n_tiles(B), HW // 8
+    dW_hh = torch.zeros(2, 3 * HW, HW, device=dev)
+    sums = torch.zeros(2, 4, HW, device=dev)             # per direction: r | z | n | hn column sums of dG
+    ones = _ones_block(dev)
+    if not padded_in:
+        xa_tm = torch.empty(tiles, T + 2, 2, L.TILE, 8, device=dev, dtype=bf)
+        _lib.call("rs_pack_x_tm", _p(saved_in), B, T, Il, _p(xa_tm), st)
+        dW_ih_buf = torch.zeros(6 * HW, 16, device=dev)
+    else:
+        dW_ih_buf = torch.zeros(6 * HW, Il, device=dev)
+    flops = 2.0 * tiles * L.TILE * T * (6 * HW * (Il if padded_in else 16) + 6 * HW * HW + 8 * HW * 16)
+    with ktime("blk_wgrad_kernel", flops):
+        for d in (0, 1):                                 # one launch per direction: <= 18 roles of one 128-row gate block
+            sh = -1 if d == 0 else 1
+            roles, hh_roles = [], []
+            for mb in (0, 1):                            # the two 128-row halves of a 256-row gate block
+                m0 = mb * 128
+                if not padded_in:
+                    for g in (0, 1):
+                        roles.append((d * 4 * HC + g * HC + mb * 16, out, 2 * HW, d * HC, HW, sh, dW_hh[d, g * HW + m0:], HW,
+                                      sums[d, g, m0:], xa_tm, dW_ih_buf[(d * 3 + g) * HW + m0:]))
+                    roles.append((d * 4 * HC + 3 * HC + mb * 16, out, 2 * HW, d * HC, HW, sh, dW_hh[d, 2 * HW + m0:], HW,
+                                  sums[d, 3, m0:], None, None))
+                    roles.append((d * 4 * HC + 2 * HC + mb * 16, None, 0, 0, 0, 0, None, 0, sums[d, 2, m0:], xa_tm,
+                                  dW_ih_buf[(d * 3 + 2) * HW + m0:]))
+                else:
+                    for g in (0, 1, 2):                  # r, z, n against the layer input, 256 columns at a time: the two
+                        for nb in range(Il // 256):      # halves of Il are adjacent roles = one CTA pair sharing its dG block
+                            roles.append((d * 4 * HC + g * HC + mb * 16, saved_in, Il, nb * 32, 256, 0,
+                                          dW_ih_buf[(d * 3 + g) * HW + m0:, nb * 256:], Il, sums[d, g, m0:] if nb == 0 else None,
+                                          None, None))
+                    for gi, g in enumerate((0, 1, 3)):   # r, z, hn against the shifted hidden state
+                        hh_roles.append((d * 4 * HC + g * HC + mb * 16, out, 2 * HW, d * HC, HW, sh, dW_hh[d, gi * HW + m0:], HW,
+                                         sums[d, 3, m0:] if g == 3 else None, None, None))
+            _wgrad(dG, 8 * HW, ones, roles + hh_roles, tiles, T, st)
+    db_ih = sums[:, :3].reshape(2, 3 * HW)
+    db_hh = torch.cat([sums[:, :2].reshape(2, 2 * HW), sums[:, 3]], 1)
+    dX = None
+    if need_dx:
+        dX = torch.empty(tiles, T + 2, Il // 8, L.TILE, 8, device=dev, dtype=bf)
+        wt = L.tile_weight_nt(w_ih_cat.t().contiguous())                   # [Il/128][6H/64][8][128][8]
+        kch = [d * 4 * HC + g * HC + hf * 8 for d in (0, 1) for g in (0, 1, 2) for hf in range(HW // 64)]
+        with ktime("blk_gemm_nt_kernel(dgrad)", 2.0 * tiles * L.TILE * (T + 2) * 6 * HW * Il):
+            _nt(dG, 8 * HW, kch, wt, Il // 128, dX, Il, 0, None, tiles * (T + 2), st, in_drop, T)
+    return dW_ih_buf, dW_hh, db_ih, db_hh, dX
 
 
 def _gemm_nt(A, Bw, C, bias, flags=0):

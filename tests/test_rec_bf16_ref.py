@@ -12,27 +12,30 @@ from oracle import rec_bf16_ref as R
 F64 = torch.float64
 
 
-def gru_run(H, I, B, T, lengths, seed):
+def gru_run(H, I, B, T, lengths, seed, x_mult=None):
+    """x_mult (B, T, I) or None: a dropout multiplier on the input, GRU(x * x_mult); grads["x"] is d/dx."""
     g = torch.Generator().manual_seed(seed)
     gru = torch.nn.GRU(I, H, batch_first=True, bidirectional=True).double()
     with torch.no_grad():
         for p in gru.parameters():
             p.copy_((torch.rand(p.shape, generator=g, dtype=F64) - 0.5) * (2.0 / H ** 0.5))
-    x = torch.randn(B, T, I, generator=g, dtype=F64)
+    x = torch.randn(B, T, I, generator=g, dtype=F64).requires_grad_()
     d_out = torch.randn(B, T, 2 * H, generator=g, dtype=F64)
     d_h_n = torch.randn(2, B, H, generator=g, dtype=F64)
+    xin = x * x_mult if x_mult is not None else x
     if lengths is not None:
-        packed = pack_padded_sequence(x, lengths, batch_first=True, enforce_sorted=False)
+        packed = pack_padded_sequence(xin, lengths, batch_first=True, enforce_sorted=False)
         out, h_n = gru(packed)
         out, _ = pad_packed_sequence(out, batch_first=True, total_length=T)
     else:
-        out, h_n = gru(x)
+        out, h_n = gru(xin)
     ((out * d_out).sum() + (h_n * d_h_n).sum()).backward()
     names = ("weight_ih_l0", "weight_hh_l0", "bias_ih_l0", "bias_hh_l0")
     w = [getattr(gru, n + sfx).detach() for sfx in ("", "_reverse") for n in names]
     grads = {n: torch.stack([getattr(gru, n + "_l0" + sfx).grad for sfx in ("", "_reverse")], 0)
              for n in ("weight_ih", "weight_hh", "bias_ih", "bias_hh")}
-    return x, out.detach(), h_n.detach(), d_out, d_h_n, w, grads
+    grads["x"] = x.grad
+    return x.detach(), out.detach(), h_n.detach(), d_out, d_h_n, w, grads
 
 
 CASES = [  # (H, I, B, T, lengths)
@@ -149,3 +152,64 @@ def test_quantised_weights_follow_pack_w():
     bx = (w[2] + torch.cat([w[3][:2 * H], torch.zeros(H)])) * torch.cat([torch.full((2 * H,), 0.5), torch.ones(H)])
     assert torch.equal(R.bias_x(w[2], w[3], H), bx)
     assert float((W.bias[0] - bx.double()).abs().max()) <= 2.0 ** -16 * float(bx.abs().max())
+
+
+@pytest.mark.parametrize("H,I,lengths,dropout", [(128, 256, None, False), (128, 256, [5, 1, 3, 5], True),
+                                                 (256, 512, [2, 5, 5, 4], True)])
+def test_data_grad_matches_torch_gru_input_grad(H, I, lengths, dropout):
+    """data_grad over the reference's dG, with exact weights, is autograd's gradient of the layer input -- through a
+    dropout multiplier on the input too, which data_grad applies at rows 1 .. T only (the pad rows stay unscaled)."""
+    B, T = 4, 5
+    g = torch.Generator().manual_seed(H + I)
+    mult = (torch.rand(B, T, I, generator=g) < 0.75).to(F64) / 0.75 if dropout else None
+    lt = torch.tensor(lengths, dtype=torch.int32) if lengths is not None else None
+    x, out, _, d_out, d_h_n, w, grads = gru_run(H, I, B, T, lengths, seed=7, x_mult=mult)
+    W = R.ref_weights(w, H, split=0, quant=False)
+    act = R.active_mask(lt, B, T, x.device)
+    outf = torch.zeros(2, B, T + 2, H, dtype=F64)
+    outf[0, :, 1:-1], outf[1, :, 1:-1] = out[..., :H], out[..., H:]
+    xin = x * mult if dropout else x
+    inp = torch.stack([xin @ W.wih[d].T + W.bias[d] for d in (0, 1)], 0)
+    f = R.forward_step(R.h_prev_forward(outf, lt), inp, W, act)
+    hpb = R.h_prev_backward(outf)
+    d_out_r = torch.stack([d_out[..., :H], d_out[..., H:]], 0)
+    dG = R.backward(f["r"], f["z"], f["n"], R.recompute_hn(hpb, W), hpb, W, act, d_out=d_out_r, d_h_n=d_h_n)
+    dGf = torch.zeros(2, B, T + 2, 4, H, dtype=F64)
+    dGf[:, :, 1:-1] = dG
+    dGf[:, :, 0], dGf[:, :, -1] = 1.0, -1.0                    # pad rows: they reach dX's pad rows and nothing else
+    w_ih = torch.stack([w[0], w[4]], 0).to(F64)
+    dx = R.data_grad(dGf, w_ih, mult)
+    err = float((dx[:, 1:-1] - grads["x"]).abs().max() / grads["x"].abs().max())
+    assert err < 1e-10, err
+    pads = sum(dGf[d, :, [0, -1], :3].flatten(2) @ w_ih[d] for d in (0, 1))
+    assert torch.allclose(dx[:, [0, -1]], pads, rtol=1e-12, atol=1e-12)
+
+
+def test_projection_is_the_input_pre_activation():
+    """projection with the reference's scaled weights and bias is X W_ih^T + b_ih (+ b_hh on r, z), r and z halved, at
+    every row (pad rows included), per direction r | z | n."""
+    H, I, Bp, T = 128, 256, 3, 4
+    g = torch.Generator().manual_seed(5)
+    w = [torch.randn(3 * H, I, generator=g), torch.randn(3 * H, H, generator=g), torch.randn(3 * H, generator=g),
+         torch.randn(3 * H, generator=g)] * 2
+    w[4:] = [t * 2 for t in w[4:]]
+    W = R.ref_weights(w, H, split=0, quant=False)
+    X = torch.randn(Bp, T + 2, I, generator=g, dtype=F64)
+    P = R.projection(X, W.wih, W.bias)
+    s = R.gate_scale(H, "cpu", F64)
+    for d in (0, 1):
+        w_ih, _, b_ih, b_hh = [t.to(F64) for t in w[4 * d: 4 * d + 4]]
+        want = (X @ w_ih.T + b_ih + torch.cat([b_hh[:2 * H], torch.zeros(H, dtype=F64)])) * s
+        assert float((P[..., 3 * H * d: 3 * H * (d + 1)] - want).abs().max()) < 1e-12
+
+
+def test_x_operand_layout():
+    """x_operand: bf16(x) in columns < I of rows 1 .. T of the real traces; zero columns >= I, pad rows and pad traces."""
+    B, T, I, Bp = 3, 4, 5, 128
+    x = torch.randn(B, T, I, generator=torch.Generator().manual_seed(2))
+    xo = R.x_operand(x, Bp, T)
+    assert xo.shape == (Bp, T + 2, 16) and xo.dtype == F64
+    assert torch.equal(xo[:B, 1:-1, :I], x.to(torch.bfloat16).to(F64))
+    rest = xo.clone()
+    rest[:B, 1:-1, :I] = 0
+    assert torch.equal(rest, torch.zeros_like(rest))
