@@ -60,6 +60,8 @@ __global__ void heads_merge_kernel(const float* __restrict__ raw, int B, int N, 
     }
 }
 
+// dx may alias dy (both decoders call these in place).  Each element is read and written by the same thread in one
+// iteration, and no other element is read, so __restrict__ allows no reordering that changes the result.
 __global__ void relu_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ y, float* __restrict__ dx,
                                 long long n) {
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (long long)gridDim.x * blockDim.x)

@@ -369,6 +369,84 @@ class _LazyOut:
         return layout.from_tile_major(self.tm, self.B, self.T).float()
 
 
+def heads_split(raw: torch.Tensor, N: int, C: int):
+    """raw [B, N*(C+6)] fp32 (columns class | pos | size | orient | valid) -> (cls, pos, size, orient, valid):
+    rs_heads_split_f32, sizes = softplus(raw) + 1e-4."""
+    B, dev = raw.shape[0], raw.device
+    out = (torch.empty(B, N, C, device=dev), torch.empty(B, N, 2, device=dev), torch.empty(B, N, 2, device=dev),
+           torch.empty(B, N, device=dev), torch.empty(B, N, device=dev))
+    _lib.call("rs_heads_split_f32", _p(raw), B, N, C, *[_p(t) for t in out], _stream(raw))
+    return out
+
+
+def heads_merge(raw: torch.Tensor, N: int, C: int, d_cls, d_pos, d_size, d_orient, d_valid) -> torch.Tensor:
+    """The gradients of the five prediction tensors (None: zero) -> d_raw [B, N*(C+6)]: rs_heads_merge_bwd_f32."""
+    c = lambda t: t.contiguous().float() if t is not None else None  # noqa: E731
+    d_raw = torch.empty_like(raw)
+    _lib.call("rs_heads_merge_bwd_f32", _p(raw), raw.shape[0], N, C, _p(c(d_cls)), _p(c(d_pos)), _p(c(d_size)),
+              _p(c(d_orient)), _p(c(d_valid)), _p(d_raw), _stream(raw))
+    return d_raw
+
+
+def decoder_fwd(latent, N, C, W1, b1, W2, b2, heads):
+    """Forward of DecoderFn.  Returns a dict: the saved operands latent, W1, W2, Wh, the intermediates f1, f2, raw and
+    heads = (cls, pos, size, orient, valid)."""
+    latent = latent.contiguous().float()
+    B = latent.shape[0]
+    dev = latent.device
+    Wh = torch.cat(heads[0::2], 0).contiguous()      # [N*(C+6), D]
+    bh = torch.cat(heads[1::2], 0).contiguous()
+    D1, D2, NH = W1.shape[0], W2.shape[0], Wh.shape[0]
+    f1 = torch.empty(B, D1, device=dev)
+    f2 = torch.empty(B, D2, device=dev)
+    raw = torch.empty(B, NH, device=dev)
+    with ktime("decoder_fwd(sgemm x3)", 2.0 * B * (latent.shape[1] * D1 + D1 * D2 + D2 * NH)):
+        linear_nt(latent, W1.contiguous(), b1, f1, RELU)
+        linear_nt(f1, W2.contiguous(), b2, f2, RELU)
+        linear_nt(f2, Wh, bh, raw)
+    return dict(latent=latent, W1=W1, W2=W2, Wh=Wh, f1=f1, f2=f2, raw=raw, heads=heads_split(raw, N, C))
+
+
+def decoder_bwd(latent, W1, W2, Wh, f1, f2, d_raw):
+    """Backward of DecoderFn from d_raw [B, NH].  Returns a dict of dWh, dbh, df2 (after the ReLU mask), dW2, db2, df1,
+    dW1, db1, dlat."""
+    dev = latent.device
+    st = _stream(latent)
+    kt = ktime("decoder_bwd(sgemm x6)", 4.0 * latent.shape[0] * (latent.shape[1] * W1.shape[0] + W1.shape[0] * W2.shape[0] + W2.shape[0] * Wh.shape[0]))
+    kt.__enter__()
+    dWh = torch.empty_like(Wh)
+    matmul_tn(d_raw, f2, dWh)
+    dbh = torch.empty(Wh.shape[0], device=dev)
+    colsum(d_raw, dbh)
+    df2 = torch.empty_like(f2)
+    matmul_nn(d_raw, Wh, df2)
+    _lib.call("rs_relu_bwd_f32", _p(df2), _p(f2), _p(df2), df2.numel(), st)
+    dW2 = torch.empty_like(W2)
+    matmul_tn(df2, f1, dW2)
+    db2 = torch.empty(W2.shape[0], device=dev)
+    colsum(df2, db2)
+    df1 = torch.empty_like(f1)
+    matmul_nn(df2, W2.contiguous(), df1)
+    _lib.call("rs_relu_bwd_f32", _p(df1), _p(f1), _p(df1), df1.numel(), st)
+    dW1 = torch.empty_like(W1)
+    matmul_tn(df1, latent, dW1)
+    db1 = torch.empty(W1.shape[0], device=dev)
+    colsum(df1, db1)
+    dlat = torch.empty_like(latent)
+    matmul_nn(df1, W1.contiguous(), dlat)
+    kt.__exit__(None, None, None)
+    return dict(dWh=dWh, dbh=dbh, df2=df2, dW2=dW2, db2=db2, df1=df1, dW1=dW1, db1=db1, dlat=dlat)
+
+
+def split_head_grads(dWh, dbh, head_rows):
+    """Row blocks of the stacked head gradients, one (dW, db) pair per head."""
+    out, r0 = [], 0
+    for rows in head_rows:
+        out += [dWh[r0:r0 + rows], dbh[r0:r0 + rows]]
+        r0 += rows
+    return out
+
+
 class DecoderFn(torch.autograd.Function):
     """MLP trunk (2 x Linear+ReLU) + five heads, fp32.
     apply(latent, N, C, W1, b1, W2, b2, Wc, bc, Wp, bp, Ws, bs, Wo, bo, Wv, bv) -> 5 prediction tensors."""
@@ -377,71 +455,48 @@ class DecoderFn(torch.autograd.Function):
     @_lib.on_tensor_device
     def forward(ctx, latent, N, C, W1, b1, W2, b2, *heads):
         _need_cuda(latent, W1, W2, *heads)
-        latent = latent.contiguous().float()
-        B = latent.shape[0]
-        dev = latent.device
-        Wh = torch.cat(heads[0::2], 0).contiguous()      # [N*(C+6), D]
-        bh = torch.cat(heads[1::2], 0).contiguous()
-        D1, D2, NH = W1.shape[0], W2.shape[0], Wh.shape[0]
-        f1 = torch.empty(B, D1, device=dev)
-        f2 = torch.empty(B, D2, device=dev)
-        raw = torch.empty(B, NH, device=dev)
-        with ktime("decoder_fwd(sgemm x3)", 2.0 * B * (latent.shape[1] * D1 + D1 * D2 + D2 * NH)):
-            linear_nt(latent, W1.contiguous(), b1, f1, RELU)
-            linear_nt(f1, W2.contiguous(), b2, f2, RELU)
-            linear_nt(f2, Wh, bh, raw)
-        cls = torch.empty(B, N, C, device=dev)
-        pos = torch.empty(B, N, 2, device=dev)
-        size = torch.empty(B, N, 2, device=dev)
-        orient = torch.empty(B, N, device=dev)
-        valid = torch.empty(B, N, device=dev)
-        _lib.call("rs_heads_split_f32", _p(raw), B, N, C, _p(cls), _p(pos), _p(size), _p(orient), _p(valid), _stream(raw))
-        ctx.save_for_backward(latent, W1, W2, Wh, f1, f2, raw)
-        ctx.dims = (B, N, C)
+        r = decoder_fwd(latent, N, C, W1, b1, W2, b2, heads)
+        ctx.save_for_backward(r["latent"], W1, W2, r["Wh"], r["f1"], r["f2"], r["raw"])
+        ctx.dims = (N, C)
         ctx.head_rows = [h.shape[0] for h in heads[0::2]]
-        return cls, pos, size, orient, valid
+        return r["heads"]
 
     @staticmethod
     @_lib.on_tensor_device
     def backward(ctx, d_cls, d_pos, d_size, d_orient, d_valid):
         latent, W1, W2, Wh, f1, f2, raw = ctx.saved_tensors
-        B, N, C = ctx.dims
-        dev = latent.device
-        st = torch.cuda.current_stream(dev).cuda_stream
-        c = lambda t: t.contiguous() if t is not None else None  # noqa: E731
-        d_cls, d_pos, d_size, d_orient, d_valid = c(d_cls), c(d_pos), c(d_size), c(d_orient), c(d_valid)
-        kt = ktime("decoder_bwd(sgemm x6)", 4.0 * B * (latent.shape[1] * W1.shape[0] + W1.shape[0] * W2.shape[0] + W2.shape[0] * Wh.shape[0]))
-        kt.__enter__()
-        d_raw = torch.empty_like(raw)
-        _lib.call("rs_heads_merge_bwd_f32", _p(raw), B, N, C, _p(d_cls), _p(d_pos), _p(d_size), _p(d_orient),
-                  _p(d_valid), _p(d_raw), st)
-        dWh = torch.empty_like(Wh)
-        matmul_tn(d_raw, f2, dWh)
-        dbh = torch.empty(Wh.shape[0], device=dev)
-        colsum(d_raw, dbh)
-        df2 = torch.empty_like(f2)
-        matmul_nn(d_raw, Wh, df2)
-        _lib.call("rs_relu_bwd_f32", _p(df2), _p(f2), _p(df2), df2.numel(), st)
-        dW2 = torch.empty_like(W2)
-        matmul_tn(df2, f1, dW2)
-        db2 = torch.empty(W2.shape[0], device=dev)
-        colsum(df2, db2)
-        df1 = torch.empty_like(f1)
-        matmul_nn(df2, W2.contiguous(), df1)
-        _lib.call("rs_relu_bwd_f32", _p(df1), _p(f1), _p(df1), df1.numel(), st)
-        dW1 = torch.empty_like(W1)
-        matmul_tn(df1, latent, dW1)
-        db1 = torch.empty(W1.shape[0], device=dev)
-        colsum(df1, db1)
-        dlat = torch.empty_like(latent)
-        matmul_nn(df1, W1.contiguous(), dlat)
-        kt.__exit__(None, None, None)
-        head_grads = []
-        r0 = 0
-        for rows in ctx.head_rows:
-            head_grads += [dWh[r0:r0 + rows], dbh[r0:r0 + rows]]
-            r0 += rows
-        return (dlat, None, None, dW1, db1, dW2, db2, *head_grads)
+        N, C = ctx.dims
+        d_raw = heads_merge(raw, N, C, d_cls, d_pos, d_size, d_orient, d_valid)
+        g = decoder_bwd(latent, W1, W2, Wh, f1, f2, d_raw)
+        return (g["dlat"], None, None, g["dW1"], g["db1"], g["dW2"], g["db2"], *split_head_grads(g["dWh"], g["dbh"], ctx.head_rows))
+
+
+def loss_fwd(cls, pos, size, orient, vlogit, t_cls, t_pos, t_size, t_orient, t_valid):
+    """rs_loss_fwd_f32.  Returns (losses[6] fp32, sums[6] fp64, g = [g_cls, g_pos, g_size, g_orient, g_valid]): the six
+    un-normalised sums and the per-element gradients that loss_bwd scales."""
+    B, N, C = cls.shape
+    dev = cls.device
+    f = lambda t: t.contiguous().float()  # noqa: E731
+    cls, pos, size, orient, vlogit = f(cls), f(pos), f(size), f(orient), f(vlogit)
+    t_cls = t_cls.contiguous().long()
+    t_pos, t_size, t_orient, t_valid = f(t_pos), f(t_size), f(t_orient), f(t_valid)
+    sums = torch.empty(6, dtype=torch.float64, device=dev)
+    losses = torch.empty(6, device=dev)
+    g = [torch.empty_like(t) for t in (cls, pos, size, orient, vlogit)]
+    _lib.call("rs_loss_fwd_f32", _p(cls), _p(pos), _p(size), _p(orient), _p(vlogit), _p(t_cls), _p(t_pos),
+              _p(t_size), _p(t_orient), _p(t_valid), B, N, C, ctypes.addressof(_W5), _p(sums), _p(losses),
+              *[_p(t) for t in g], _stream(cls))
+    return losses, sums, g
+
+
+def loss_bwd(sums, g, d_losses):
+    """rs_loss_bwd_f32: the gradients of the five prediction tensors for the incoming d(losses)[6]."""
+    B, N, C = g[0].shape
+    d_losses = d_losses.contiguous().float()
+    d = [torch.empty_like(t) for t in g]
+    _lib.call("rs_loss_bwd_f32", _p(sums), _p(d_losses), B, N, C, ctypes.addressof(_W5), *[_p(t) for t in g],
+              *[_p(t) for t in d], _stream(sums))
+    return d
 
 
 class MultiTaskLossFn(torch.autograd.Function):
@@ -452,29 +507,12 @@ class MultiTaskLossFn(torch.autograd.Function):
     @_lib.on_tensor_device
     def forward(ctx, cls, pos, size, orient, vlogit, t_cls, t_pos, t_size, t_orient, t_valid):
         _need_cuda(cls, pos, size, orient, vlogit, t_cls, t_pos, t_size, t_orient, t_valid)
-        B, N, C = cls.shape
-        dev = cls.device
-        f = lambda t: t.contiguous().float()  # noqa: E731
-        cls, pos, size, orient, vlogit = f(cls), f(pos), f(size), f(orient), f(vlogit)
-        t_cls = t_cls.contiguous().long()
-        t_pos, t_size, t_orient, t_valid = f(t_pos), f(t_size), f(t_orient), f(t_valid)
-        sums = torch.empty(6, dtype=torch.float64, device=dev)
-        losses = torch.empty(6, device=dev)
-        g = [torch.empty_like(t) for t in (cls, pos, size, orient, vlogit)]
-        _lib.call("rs_loss_fwd_f32", _p(cls), _p(pos), _p(size), _p(orient), _p(vlogit), _p(t_cls), _p(t_pos),
-                  _p(t_size), _p(t_orient), _p(t_valid), B, N, C, ctypes.addressof(_W5), _p(sums), _p(losses),
-                  *[_p(t) for t in g], _stream(cls))
+        losses, sums, g = loss_fwd(cls, pos, size, orient, vlogit, t_cls, t_pos, t_size, t_orient, t_valid)
         ctx.save_for_backward(sums, *g)
-        ctx.dims = (B, N, C)
         return losses
 
     @staticmethod
     @_lib.on_tensor_device
     def backward(ctx, d_losses):
         sums, *g = ctx.saved_tensors
-        B, N, C = ctx.dims
-        d_losses = d_losses.contiguous().float()
-        d = [torch.empty_like(t) for t in g]
-        _lib.call("rs_loss_bwd_f32", _p(sums), _p(d_losses), B, N, C, ctypes.addressof(_W5), *[_p(t) for t in g],
-                  *[_p(t) for t in d], _stream(sums))
-        return (*d, None, None, None, None, None)
+        return (*loss_bwd(sums, g, d_losses), None, None, None, None, None)

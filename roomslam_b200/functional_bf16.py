@@ -19,6 +19,7 @@ from typing import Optional
 import torch
 
 from . import _lib
+from . import functional as F_
 from . import layout as L
 from .functional import _need_cuda, _p, _stream, ktime
 
@@ -528,6 +529,68 @@ def _gemm_tn(A, Bm, C):
 RELU, OUT_F32 = 2, 4
 
 
+def decoder_bf16_fwd(latent, N, C, W1, b1, W2, b2, heads):
+    """Forward of DecoderBF16Fn.  The head rows are stacked into Wh [NHp, D2] (bf16) and bh [NHp] with zero rows up to
+    NHp = ceil(N (C + 6) / 128) 128.  Returns a dict: the GEMM operands lat, W1b, W2b (bf16), Wh, bh, the intermediates
+    f1, f2 (bf16), rawp [B, NHp] and raw = rawp[:, :NH] (fp32), and heads = (cls, pos, size, orient, valid)."""
+    dev = latent.device
+    bf = torch.bfloat16
+    NH = sum(h.shape[0] for h in heads[0::2])
+    NHp = (NH + 127) // 128 * 128
+    Wh = torch.zeros(NHp, W2.shape[0], device=dev, dtype=bf)
+    Wh[:NH] = torch.cat(heads[0::2], 0)
+    bh = torch.zeros(NHp, device=dev)
+    bh[:NH] = torch.cat(heads[1::2], 0)
+    lat = latent.to(bf).contiguous()
+    W1b, W2b = W1.to(bf).contiguous(), W2.to(bf).contiguous()
+    B = lat.shape[0]
+    f1 = torch.empty(B, W1.shape[0], device=dev, dtype=bf)
+    f2 = torch.empty(B, W2.shape[0], device=dev, dtype=bf)
+    rawp = torch.empty(B, NHp, device=dev)
+    flops = 2.0 * B * (lat.shape[1] * W1.shape[0] + W1.shape[0] * W2.shape[0] + W2.shape[0] * NHp)
+    with ktime("gemm_tc_kernel(decoder fwd)", flops):
+        _gemm_nt(lat, W1b, f1, b1.float().contiguous(), RELU)
+        _gemm_nt(f1, W2b, f2, b2.float().contiguous(), RELU)
+        _gemm_nt(f2, Wh, rawp, bh, OUT_F32)
+    raw = rawp[:, :NH].contiguous()
+    return dict(lat=lat, W1b=W1b, W2b=W2b, Wh=Wh, bh=bh, f1=f1, f2=f2, rawp=rawp, raw=raw, heads=F_.heads_split(raw, N, C))
+
+
+def decoder_bf16_bwd(lat, W1b, W2b, Wh, f1, f2, d_raw):
+    """Backward of DecoderBF16Fn from d_raw [B, NH] (fp32).  Returns a dict of d_rawp [B, NHp] (bf16, zero columns from NH
+    on), dWh [NHp, D2], dbh [NH], df2 (after the ReLU mask), dW2, db2, df1, dW1, db1 and dlat."""
+    B, NH = d_raw.shape
+    NHp = Wh.shape[0]
+    dev = lat.device
+    bf = torch.bfloat16
+    st = _stream(lat)
+    d_rawp = torch.zeros(B, NHp, device=dev, dtype=bf)
+    d_rawp[:, :NH] = d_raw
+    D1, D2, DL = W1b.shape[0], W2b.shape[0], lat.shape[1]
+    flops = 4.0 * B * (DL * D1 + D1 * D2 + D2 * NHp)
+    kt = ktime("gemm_tc_kernel(decoder bwd)", flops)
+    kt.__enter__()
+    dWh = torch.zeros(NHp, D2, device=dev)
+    _gemm_tn(d_rawp, f2, dWh)
+    dbh = d_raw.sum(0)
+    df2 = torch.empty(B, D2, device=dev, dtype=bf)
+    _gemm_nt(d_rawp, Wh.t().contiguous(), df2, None)
+    _lib.call("rs_relu_bwd_bf16", _p(df2), _p(f2), _p(df2), df2.numel(), st)
+    dW2 = torch.zeros(D2, D1, device=dev)
+    _gemm_tn(df2, f1, dW2)
+    db2 = df2.float().sum(0)
+    df1 = torch.empty(B, D1, device=dev, dtype=bf)
+    _gemm_nt(df2, W2b.t().contiguous(), df1, None)
+    _lib.call("rs_relu_bwd_bf16", _p(df1), _p(f1), _p(df1), df1.numel(), st)
+    dW1 = torch.zeros(D1, DL, device=dev)
+    _gemm_tn(df1, lat, dW1)
+    db1 = df1.float().sum(0)
+    dlat = torch.empty(B, DL, device=dev)
+    _gemm_nt(df1, W1b.t().contiguous(), dlat, None, OUT_F32)
+    kt.__exit__(None, None, None)
+    return dict(d_rawp=d_rawp, dWh=dWh, dbh=dbh, df2=df2, dW2=dW2, db2=db2, df1=df1, dW1=dW1, db1=db1, dlat=dlat)
+
+
 class DecoderBF16Fn(torch.autograd.Function):
     """MLP trunk + heads of the bf16 mode on the TMA-fed tcgen05 GEMM: bf16 operands, fp32 accumulate, the head
     outputs (logits, positions, ...) leave the last GEMM in fp32.  Same signature as functional.DecoderFn."""
@@ -536,78 +599,20 @@ class DecoderBF16Fn(torch.autograd.Function):
     @_lib.on_tensor_device
     def forward(ctx, latent, N, C, W1, b1, W2, b2, *heads):
         _need_cuda(latent, W1, W2, *heads)
-        B = latent.shape[0]
-        dev = latent.device
-        bf = torch.bfloat16
         with torch.no_grad():
-            NH = sum(h.shape[0] for h in heads[0::2])
-            NHp = (NH + 127) // 128 * 128
-            Wh = torch.zeros(NHp, W2.shape[0], device=dev, dtype=bf)
-            Wh[:NH] = torch.cat(heads[0::2], 0)
-            bh = torch.zeros(NHp, device=dev)
-            bh[:NH] = torch.cat(heads[1::2], 0)
-            lat = latent.to(bf).contiguous()
-            W1b, W2b = W1.to(bf).contiguous(), W2.to(bf).contiguous()
-            f1 = torch.empty(B, W1.shape[0], device=dev, dtype=bf)
-            f2 = torch.empty(B, W2.shape[0], device=dev, dtype=bf)
-            rawp = torch.empty(B, NHp, device=dev)
-            flops = 2.0 * B * (lat.shape[1] * W1.shape[0] + W1.shape[0] * W2.shape[0] + W2.shape[0] * NHp)
-            with ktime("gemm_tc_kernel(decoder fwd)", flops):
-                _gemm_nt(lat, W1b, f1, b1.float().contiguous(), RELU)
-                _gemm_nt(f1, W2b, f2, b2.float().contiguous(), RELU)
-                _gemm_nt(f2, Wh, rawp, bh, OUT_F32)
-            raw = rawp[:, :NH].contiguous()
-            cls = torch.empty(B, N, C, device=dev)
-            pos = torch.empty(B, N, 2, device=dev)
-            size = torch.empty(B, N, 2, device=dev)
-            orient = torch.empty(B, N, device=dev)
-            valid = torch.empty(B, N, device=dev)
-            _lib.call("rs_heads_split_f32", _p(raw), B, N, C, _p(cls), _p(pos), _p(size), _p(orient), _p(valid), _stream(raw))
-        ctx.save_for_backward(lat, W1b, W2b, Wh, f1, f2, raw)
-        ctx.dims = (B, N, C, NH, NHp)
+            r = decoder_bf16_fwd(latent, N, C, W1, b1, W2, b2, heads)
+        ctx.save_for_backward(r["lat"], r["W1b"], r["W2b"], r["Wh"], r["f1"], r["f2"], r["raw"])
+        ctx.dims = (N, C)
         ctx.head_rows = [h.shape[0] for h in heads[0::2]]
-        return cls, pos, size, orient, valid
+        return r["heads"]
 
     @staticmethod
     @_lib.on_tensor_device
     def backward(ctx, d_cls, d_pos, d_size, d_orient, d_valid):
         lat, W1b, W2b, Wh, f1, f2, raw = ctx.saved_tensors
-        B, N, C, NH, NHp = ctx.dims
-        dev = lat.device
-        bf = torch.bfloat16
-        st = torch.cuda.current_stream(dev).cuda_stream
-        c = lambda t: t.contiguous().float() if t is not None else None  # noqa: E731
+        N, C = ctx.dims
         with torch.no_grad():
-            d_raw = torch.empty_like(raw)
-            _lib.call("rs_heads_merge_bwd_f32", _p(raw), B, N, C, _p(c(d_cls)), _p(c(d_pos)), _p(c(d_size)), _p(c(d_orient)),
-                      _p(c(d_valid)), _p(d_raw), st)
-            d_rawp = torch.zeros(B, NHp, device=dev, dtype=bf)
-            d_rawp[:, :NH] = d_raw
-            D1, D2, DL = W1b.shape[0], W2b.shape[0], lat.shape[1]
-            flops = 4.0 * B * (DL * D1 + D1 * D2 + D2 * NHp)
-            kt = ktime("gemm_tc_kernel(decoder bwd)", flops)
-            kt.__enter__()
-            dWh = torch.zeros(NHp, D2, device=dev)
-            _gemm_tn(d_rawp, f2, dWh)
-            dbh = d_raw.sum(0)
-            df2 = torch.empty(B, D2, device=dev, dtype=bf)
-            _gemm_nt(d_rawp, Wh.t().contiguous(), df2, None)
-            _lib.call("rs_relu_bwd_bf16", _p(df2), _p(f2), _p(df2), df2.numel(), st)
-            dW2 = torch.zeros(D2, D1, device=dev)
-            _gemm_tn(df2, f1, dW2)
-            db2 = df2.float().sum(0)
-            df1 = torch.empty(B, D1, device=dev, dtype=bf)
-            _gemm_nt(df2, W2b.t().contiguous(), df1, None)
-            _lib.call("rs_relu_bwd_bf16", _p(df1), _p(f1), _p(df1), df1.numel(), st)
-            dW1 = torch.zeros(D1, DL, device=dev)
-            _gemm_tn(df1, lat, dW1)
-            db1 = df1.float().sum(0)
-            dlat = torch.empty(B, DL, device=dev)
-            _gemm_nt(df1, W1b.t().contiguous(), dlat, None, OUT_F32)
-            kt.__exit__(None, None, None)
-            head_grads = []
-            r0 = 0
-            for rows in ctx.head_rows:
-                head_grads += [dWh[r0:r0 + rows], dbh[r0:r0 + rows]]
-                r0 += rows
-        return (dlat, None, None, dW1, db1, dW2, db2, *head_grads)
+            d_raw = F_.heads_merge(raw, N, C, d_cls, d_pos, d_size, d_orient, d_valid)
+            g = decoder_bf16_bwd(lat, W1b, W2b, Wh, f1, f2, d_raw)
+        return (g["dlat"], None, None, g["dW1"], g["db1"], g["dW2"], g["db2"],
+                *F_.split_head_grads(g["dWh"], g["dbh"], ctx.head_rows))
