@@ -8,8 +8,10 @@
 //
 // One CTA owns Bt = S*R traces of ONE direction for all T steps.  blockDim = (H, S): thread (u, y) owns hidden unit u
 // of traces y*R .. y*R+R-1 and keeps their cell state in registers.  W_hh^T (H x 4H fp32) stays resident in shared
-// memory when it fits (H <= 64: 64 KB), otherwise it streams from L2.  h is double-buffered in shared memory:
-// one __syncthreads() per step.  Sequence buffers use the (rows, row0, ld) addressing of roomslam_b200.h.
+// memory when it fits (H <= 64: 64 KB), otherwise it streams from L2; since H <= 64 always takes the register-resident
+// kernels further down, these run with W streamed (S = 2 at H <= 128, S = 1 above; R = 1, or 4 when B > 296).  h is
+// double-buffered in shared memory: one __syncthreads() per step.  Sequence buffers use the (rows, row0, ld) addressing
+// of roomslam_b200.h.
 #include "common.cuh"
 #include "../../include/roomslam_b200.h"
 
@@ -374,7 +376,11 @@ lstm_reg_bwd_kernel(SeqF d_out, const float* __restrict__ saved, const float* __
 }
 
 // traces per CTA: the smallest R whose grid is co-resident in one wave (several small CTAs per SM overlap each other's
-// barrier and latency stalls; resident CTAs per SM follow the register footprint of each variant)
+// barrier and latency stalls; resident CTAs per SM follow the register footprint of each variant).  What it returns:
+// R = 1 for B <= 148, 2 for B <= 296, 4 for B <= 592, 16 above.  R = 8 is never returned: R = 4 already covers every
+// B <= 592, and R = 8's own condition (2 ceil(B / 8) <= 148) also ends at 592.  The <HH, 8> launches below are kept
+// so that a change of the occupancy table needs no new instantiation; tests/test_bilstm_kernels_gpu.py reaches every
+// other one.
 int pick_r(int B) {
     const int rs[5] = {1, 2, 4, 8, 16}, occ[5] = {2, 2, 2, 1, 1};
     for (int i = 0; i < 5; ++i)
@@ -419,6 +425,8 @@ SeqF mkf(const float* p, int64_t ld, int64_t trace_rows, int64_t row0) {
     return s;
 }
 
+// The general kernels run at H = 96 .. 256 only (H = 32 and 64 take the register kernels above), so wsmem, which needs
+// H <= 64, is always false here: the <R, true> instantiations cannot be reached.
 struct Shape { int S, R; bool wsmem; };
 Shape pick(int B, int H) {
     Shape s;

@@ -89,6 +89,100 @@ def linear(x: torch.Tensor, w: torch.Tensor, b: Optional[torch.Tensor], allow_tc
     return LinearFn.apply(x.reshape(-1, x.shape[-1]), w, b, allow_tc).view(*lead, w.shape[0])
 
 
+def lstm_layer_fwd(xin, mask, weights, need_grad=True):
+    """Forward of ONE bidirectional LSTM layer (the body of LSTMLayerFn.forward).
+
+    xin (B, T+2, I) padded; mask (B, T, I) inter-layer dropout multiplier or None; weights = (w_ih, w_hh, b_ih, b_hh,
+    w_ih_r, w_hh_r, b_ih_r, b_hh_r).  Returns (out (B, T+2, 2H) padded with zero pad rows, saved [2][B][T][5][H] (i, f,
+    g, o, c; None unless need_grad), xin_saved, w_ih_cat [8H, I], w_hh_cat [2][4H][H], tc): xin_saved is the masked input
+    the projection read, as its bf16x6 split when tc (the tensor-core path) is taken."""
+    w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r = weights
+    xin = xin.contiguous().float()
+    B, Tp, I = xin.shape
+    T, H = Tp - 2, w_hh.shape[1]
+    dev, st = xin.device, _stream(xin)
+    if mask is not None:
+        xm = padded(B, T, I, dev)
+        m = mask.contiguous().float()
+        _lib.call("rs_seq_mul_f32", _p(xin), I, Tp, 1, _p(m), I, T, 0, _p(xm), I, Tp, 1, B, T, I, st)
+        xin = xm
+    w_ih_cat = torch.cat([w_ih, w_ih_r], 0).contiguous().float()              # [8H, I]
+    w_hh_cat = torch.stack([w_hh, w_hh_r], 0).contiguous().float()            # [2, 4H, H]
+    w_hh_t = w_hh_cat.transpose(1, 2).contiguous()                            # [2, H, 4H]
+    bias = (torch.cat([b_ih, b_ih_r], 0) + torch.cat([b_hh, b_hh_r], 0)).contiguous().float()
+    P = torch.empty(B, Tp, 8 * H, device=dev)
+    tc = _tc_ok(B * Tp, I, 2 * H)
+    if tc:
+        xin3, kpi = split3(xin.view(B * Tp, I))
+        with ktime("gemm_tc_kernel(lstm projection bf16x6)", 12.0 * B * Tp * 8 * H * kpi):
+            nt_tc(xin3, split3(w_ih_cat, role_b=True)[0], bias, P.view(B * Tp, 8 * H))
+    else:
+        with ktime("sgemm_kernel(lstm projection)", 2.0 * B * Tp * 8 * H * I):
+            linear_nt(xin.view(B * Tp, I), w_ih_cat, bias, P.view(B * Tp, 8 * H))
+    out = padded(B, T, 2 * H, dev)
+    saved = torch.empty(2, B, T, 5, H, device=dev) if need_grad else None
+    with ktime("lstm_fwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
+        _lib.call("rs_lstm_fwd_f32", _p(P), 8 * H, Tp, 1, _p(w_hh_cat), _p(w_hh_t), _p(out), 2 * H, Tp, 1, _p(saved), B, T, H, st)
+    del P
+    return out, saved, (xin3 if tc else xin), w_ih_cat, w_hh_cat, tc
+
+
+def lstm_bptt(d_out, saved, w_hh_cat):
+    """Backward through time of one layer: d_out (B, T+2, 2H) padded -> dG (B, T+2, 8H) padded (pad rows zero), the
+    gradient w.r.t. the gate pre-activations, columns [forward i | f | g | o, reverse i | f | g | o]."""
+    _, B, T, _, H = saved.shape
+    Tp = T + 2
+    d_out = d_out.contiguous().float()
+    dG = padded(B, T, 8 * H, d_out.device)
+    with ktime("lstm_bwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
+        _lib.call("rs_lstm_bwd_f32", _p(d_out), 2 * H, Tp, 1, _p(saved), _p(w_hh_cat), _p(dG), 8 * H, Tp, 1, B, T, H, _stream(d_out))
+    return dG
+
+
+def lstm_grads_from_dG(dG, out, xin_saved, w_ih_cat, mask, tc, need_dx=True):
+    """Everything LSTMLayerFn.backward does after the BPTT: (dW_ih [8H, I], dW_hh [2][4H][H], db [8H], d_xin (B, T+2, I)
+    or None).  db is the gradient of b_ih and of b_hh alike; d_xin is multiplied by the dropout mask at rows 1..T."""
+    B, Tp, H8 = dG.shape
+    T, H, I, M = Tp - 2, H8 // 8, w_ih_cat.shape[1], B * Tp
+    dev, st = dG.device, _stream(dG)
+    dG2, out2 = dG.view(M, 8 * H), out.view(M, 2 * H)
+    # h_{t-1} of a step is the row before (forward) / after (reverse); the zero pad rows close the boundary
+    if tc:
+        dG3, kpg = split3(dG2)
+        out3, kpo = split3(out2)
+        kpi = xin_saved.shape[1] // 6
+        dW_ih = torch.zeros(8 * H, I, device=dev)
+        hh = torch.zeros(2, 4 * H, 2 * H, device=dev)
+        with ktime("gemm_tc_kernel(lstm wgrad bf16x6)", 12.0 * M * 8 * H * (I + 2 * H)):
+            tn_tc(dG3, kpg, 0, 8 * H, xin_saved, kpi, I, dW_ih)
+            tn_tc(dG3, kpg, 0, 4 * H, out3, kpo, 2 * H, hh[0], a_shift=1, b_shift=0)
+            tn_tc(dG3, kpg, 4 * H, 4 * H, out3, kpo, 2 * H, hh[1], a_shift=0, b_shift=1)
+        dW_hh = torch.stack([hh[0, :, 0:H], hh[1, :, H:2 * H]], 0)
+        del out3
+    else:
+        dW_ih = torch.empty(8 * H, I, device=dev)
+        with ktime("sgemm_kernel(lstm wgrad)", 2.0 * M * 8 * H * (I + H)):
+            matmul_tn(dG2, xin_saved.view(M, I), dW_ih)
+            dW_hh = torch.empty(2, 4 * H, H, device=dev)
+            matmul_tn(dG2[1:, 0:4 * H], out2[:M - 1, 0:H], dW_hh[0])
+            matmul_tn(dG2[:M - 1, 4 * H:8 * H], out2[1:, H:2 * H], dW_hh[1])
+    db = torch.empty(8 * H, device=dev)
+    colsum(dG2, db)
+    d_xin = None
+    if need_dx:
+        d_xin = torch.empty(B, Tp, I, device=dev)
+        if tc:
+            with ktime("gemm_tc_kernel(lstm dgrad bf16x6)", 12.0 * M * I * kpg):
+                nt_tc(dG3, split3(w_ih_cat.t(), role_b=True)[0], None, d_xin.view(M, I))
+        else:
+            with ktime("sgemm_kernel(lstm dgrad)", 2.0 * M * 8 * H * I):
+                matmul_nn(dG2, w_ih_cat, d_xin.view(M, I))
+        if mask is not None:
+            m = mask.contiguous().float()
+            _lib.call("rs_seq_mul_f32", _p(d_xin), I, Tp, 1, _p(m), I, T, 0, _p(d_xin), I, Tp, 1, B, T, I, st)
+    return dW_ih, dW_hh, db, d_xin
+
+
 class LSTMLayerFn(torch.autograd.Function):
     """ONE bidirectional LSTM layer over the padded activation layout.
 
@@ -99,88 +193,22 @@ class LSTMLayerFn(torch.autograd.Function):
     @_lib.on_tensor_device
     def forward(ctx, xin, mask, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r):
         _need_cuda(xin, mask, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r)
-        xin = xin.contiguous().float()
-        B, Tp, I = xin.shape
-        T, H = Tp - 2, w_hh.shape[1]
-        dev, st = xin.device, _stream(xin)
-        need_grad = any(ctx.needs_input_grad)
-        if mask is not None:
-            xm = padded(B, T, I, dev)
-            m = mask.contiguous().float()
-            _lib.call("rs_seq_mul_f32", _p(xin), I, Tp, 1, _p(m), I, T, 0, _p(xm), I, Tp, 1, B, T, I, st)
-            xin = xm
-        w_ih_cat = torch.cat([w_ih, w_ih_r], 0).contiguous().float()              # [8H, I]
-        w_hh_cat = torch.stack([w_hh, w_hh_r], 0).contiguous().float()            # [2, 4H, H]
-        w_hh_t = w_hh_cat.transpose(1, 2).contiguous()                            # [2, H, 4H]
-        bias = (torch.cat([b_ih, b_ih_r], 0) + torch.cat([b_hh, b_hh_r], 0)).contiguous().float()
-        P = torch.empty(B, Tp, 8 * H, device=dev)
-        tc = _tc_ok(B * Tp, I, 2 * H)
-        if tc:
-            xin3, kpi = split3(xin.view(B * Tp, I))
-            with ktime("gemm_tc_kernel(lstm projection bf16x6)", 12.0 * B * Tp * 8 * H * kpi):
-                nt_tc(xin3, split3(w_ih_cat, role_b=True)[0], bias, P.view(B * Tp, 8 * H))
-        else:
-            with ktime("sgemm_kernel(lstm projection)", 2.0 * B * Tp * 8 * H * I):
-                linear_nt(xin.view(B * Tp, I), w_ih_cat, bias, P.view(B * Tp, 8 * H))
-        out = padded(B, T, 2 * H, dev)
-        saved = torch.empty(2, B, T, 5, H, device=dev) if need_grad else None
-        with ktime("lstm_fwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
-            _lib.call("rs_lstm_fwd_f32", _p(P), 8 * H, Tp, 1, _p(w_hh_cat), _p(w_hh_t), _p(out), 2 * H, Tp, 1, _p(saved), B, T, H, st)
-        del P
-        ctx.dims = (B, T, I, H)
+        out, saved, xin_saved, w_ih_cat, w_hh_cat, tc = lstm_layer_fwd(
+            xin, mask, (w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r), need_grad=any(ctx.needs_input_grad))
         ctx.mask = mask
         ctx.tc = tc
-        ctx.save_for_backward(out, saved, xin3 if tc else xin, w_ih_cat, w_hh_cat)
+        ctx.save_for_backward(out, saved, xin_saved, w_ih_cat, w_hh_cat)
         return out
 
     @staticmethod
     @_lib.on_tensor_device
     def backward(ctx, d_out):
-        B, T, I, H = ctx.dims
-        out, saved, xin, w_ih_cat, w_hh_cat = ctx.saved_tensors
+        out, saved, xin_saved, w_ih_cat, w_hh_cat = ctx.saved_tensors
         if saved is None:
             raise RuntimeError("LSTMLayerFn: forward ran without saving activations (nothing required grad)")
-        dev, st = out.device, _stream(out)
-        Tp, M = T + 2, B * (T + 2)
-        d_out = d_out.contiguous().float()
-        dG = padded(B, T, 8 * H, dev)
-        with ktime("lstm_bwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
-            _lib.call("rs_lstm_bwd_f32", _p(d_out), 2 * H, Tp, 1, _p(saved), _p(w_hh_cat), _p(dG), 8 * H, Tp, 1, B, T, H, st)
-        dG2, out2 = dG.view(M, 8 * H), out.view(M, 2 * H)
-        # h_{t-1} of a step is the row before (forward) / after (reverse); the zero pad rows close the boundary
-        if ctx.tc:
-            dG3, kpg = split3(dG2)
-            out3, kpo = split3(out2)
-            kpi = xin.shape[1] // 6
-            dW_ih = torch.zeros(8 * H, I, device=dev)
-            hh = torch.zeros(2, 4 * H, 2 * H, device=dev)
-            with ktime("gemm_tc_kernel(lstm wgrad bf16x6)", 12.0 * M * 8 * H * (I + 2 * H)):
-                tn_tc(dG3, kpg, 0, 8 * H, xin, kpi, I, dW_ih)
-                tn_tc(dG3, kpg, 0, 4 * H, out3, kpo, 2 * H, hh[0], a_shift=1, b_shift=0)
-                tn_tc(dG3, kpg, 4 * H, 4 * H, out3, kpo, 2 * H, hh[1], a_shift=0, b_shift=1)
-            dW_hh = torch.stack([hh[0, :, 0:H], hh[1, :, H:2 * H]], 0)
-            del out3
-        else:
-            dW_ih = torch.empty(8 * H, I, device=dev)
-            with ktime("sgemm_kernel(lstm wgrad)", 2.0 * M * 8 * H * (I + H)):
-                matmul_tn(dG2, xin.view(M, I), dW_ih)
-                dW_hh = torch.empty(2, 4 * H, H, device=dev)
-                matmul_tn(dG2[1:, 0:4 * H], out2[:M - 1, 0:H], dW_hh[0])
-                matmul_tn(dG2[:M - 1, 4 * H:8 * H], out2[1:, H:2 * H], dW_hh[1])
-        db = torch.empty(8 * H, device=dev)
-        colsum(dG2, db)
-        d_xin = None
-        if ctx.needs_input_grad[0]:
-            d_xin = torch.empty(B, Tp, I, device=dev)
-            if ctx.tc:
-                with ktime("gemm_tc_kernel(lstm dgrad bf16x6)", 12.0 * M * I * kpg):
-                    nt_tc(dG3, split3(w_ih_cat.t(), role_b=True)[0], None, d_xin.view(M, I))
-            else:
-                with ktime("sgemm_kernel(lstm dgrad)", 2.0 * M * 8 * H * I):
-                    matmul_nn(dG2, w_ih_cat, d_xin.view(M, I))
-            if ctx.mask is not None:
-                m = ctx.mask.contiguous().float()
-                _lib.call("rs_seq_mul_f32", _p(d_xin), I, Tp, 1, _p(m), I, T, 0, _p(d_xin), I, Tp, 1, B, T, I, st)
+        dG = lstm_bptt(d_out, saved, w_hh_cat)
+        dW_ih, dW_hh, db, d_xin = lstm_grads_from_dG(dG, out, xin_saved, w_ih_cat, ctx.mask, ctx.tc, ctx.needs_input_grad[0])
+        H = w_hh_cat.shape[2]
         return (d_xin, None, dW_ih[:4 * H], dW_hh[0], db[:4 * H], db[:4 * H], dW_ih[4 * H:], dW_hh[1], db[4 * H:], db[4 * H:])
 
 
@@ -189,6 +217,48 @@ def _splits(B: int, N: int, Q: int) -> int:
     qtiles = (Q + 31) // 32
     want = -(-2 * 148 // max(1, B * qtiles))
     return max(1, min(want, (N + 31) // 32))
+
+
+def query_attn_fwd(memory, qk, qb, traces, mask_u8, mean, rms, splits=None):
+    """Forward of the query attention (the body of QueryAttnFn.forward): memory padded (B, N+2, D), qk (Q, D), qb (Q,),
+    traces (B, N, F), mask_u8 (B, N) or None, mean (B, 3), rms (B,) -> (ctx (B, Q, D), anchor (B, Q, 3), summary (B, D),
+    stats (B, Q, 2) = per-query softmax (max, sum), splits).  splits defaults to what _splits picks for the shape."""
+    memory, qk, qb = memory.contiguous().float(), qk.contiguous().float(), qb.contiguous().float()
+    B, Np, D = memory.shape
+    N, Q, Fdim = Np - 2, qk.shape[0], traces.shape[2]
+    dev, st = memory.device, _stream(memory)
+    splits = _splits(B, N, Q) if splits is None else splits
+    ws = torch.empty(_lib.load().rs_query_attn_workspace(B, Q, D, splits), device=dev)
+    ctx = torch.empty(B, Q, D, device=dev)
+    anchor = torch.empty(B, Q, 3, device=dev)
+    summary = torch.empty(B, D, device=dev)
+    stats = torch.empty(B, Q, 2, device=dev)
+    with ktime("query_attn_fwd_kernel", 4.0 * B * N * Q * D):
+        _lib.call("rs_query_attn_fwd_f32", _p(memory), D, Np, 1, _p(traces), Fdim, _p(mask_u8), _p(mean), _p(rms), _p(qk),
+                  _p(qb), B, N, Q, D, splits, _p(ws), _p(ctx), _p(anchor), _p(summary), _p(stats), st)
+    return ctx, anchor, summary, stats, splits
+
+
+def query_attn_bwd(memory, qk, qb, traces, mask_u8, mean, rms, count, ctx, anchor, stats, d_ctx, d_anchor, d_summary, splits):
+    """Backward of the query attention (the body of QueryAttnFn.backward) -> (d_memory (B, N+2, D) padded with zero pad
+    rows, dqk (Q, D), dqb (Q,)).  The kernel leaves per-(trace, split) partials of [dqk | dqb]; their column sum is the
+    gradient.  d_ctx / d_anchor None stand for zeros, d_summary None for no summary gradient."""
+    B, Np, D = memory.shape
+    N, Q, Fdim = Np - 2, qk.shape[0], traces.shape[2]
+    dev, st = memory.device, _stream(memory)
+    d_ctx = d_ctx.contiguous().float() if d_ctx is not None else torch.zeros_like(ctx)
+    d_anchor = d_anchor.contiguous().float() if d_anchor is not None else torch.zeros_like(anchor)
+    d_summary = d_summary.contiguous().float() if d_summary is not None else None
+    d_mem = torch.zeros(B, Np, D, device=dev) if Q > 32 else padded(B, N, D, dev)
+    dq_part = torch.empty(B * splits, Q * (D + 1), device=dev)
+    with ktime("query_attn_bwd_kernel", 10.0 * B * N * Q * D):
+        _lib.call("rs_query_attn_bwd_f32", _p(memory), D, Np, 1, _p(traces), Fdim, _p(mask_u8), _p(mean), _p(rms), _p(count),
+                  _p(qk), _p(qb), _p(ctx), _p(anchor), _p(stats), _p(d_ctx), _p(d_anchor), _p(d_summary), B, N, Q, D,
+                  splits, _p(d_mem), D, Np, 1, _p(dq_part), st)
+    dq = torch.empty(Q * (D + 1), device=dev)
+    colsum(dq_part, dq)
+    dq = dq.view(Q, D + 1)
+    return d_mem, dq[:, :D].contiguous(), dq[:, D].contiguous()
 
 
 class QueryAttnFn(torch.autograd.Function):
@@ -200,18 +270,7 @@ class QueryAttnFn(torch.autograd.Function):
     def forward(ctx_, memory, qk, qb, traces, mask_u8, mean, rms, count):
         _need_cuda(memory, qk, qb, traces, mask_u8, mean, rms, count)
         memory, qk, qb = memory.contiguous().float(), qk.contiguous().float(), qb.contiguous().float()
-        B, Np, D = memory.shape
-        N, Q, Fdim = Np - 2, qk.shape[0], traces.shape[2]
-        dev, st = memory.device, _stream(memory)
-        splits = _splits(B, N, Q)
-        ws = torch.empty(_lib.load().rs_query_attn_workspace(B, Q, D, splits), device=dev)
-        ctx = torch.empty(B, Q, D, device=dev)
-        anchor = torch.empty(B, Q, 3, device=dev)
-        summary = torch.empty(B, D, device=dev)
-        stats = torch.empty(B, Q, 2, device=dev)
-        with ktime("query_attn_fwd_kernel", 4.0 * B * N * Q * D):
-            _lib.call("rs_query_attn_fwd_f32", _p(memory), D, Np, 1, _p(traces), Fdim, _p(mask_u8), _p(mean), _p(rms), _p(qk),
-                      _p(qb), B, N, Q, D, splits, _p(ws), _p(ctx), _p(anchor), _p(summary), _p(stats), st)
+        ctx, anchor, summary, stats, splits = query_attn_fwd(memory, qk, qb, traces, mask_u8, mean, rms)
         ctx_.save_for_backward(memory, qk, qb, traces, mask_u8, mean, rms, count, ctx, anchor, stats)
         ctx_.splits = splits
         return ctx, anchor, summary
@@ -219,23 +278,8 @@ class QueryAttnFn(torch.autograd.Function):
     @staticmethod
     @_lib.on_tensor_device
     def backward(ctx_, d_ctx, d_anchor, d_summary):
-        memory, qk, qb, traces, mask_u8, mean, rms, count, ctx, anchor, stats = ctx_.saved_tensors
-        B, Np, D = memory.shape
-        N, Q, Fdim = Np - 2, qk.shape[0], traces.shape[2]
-        dev, st, splits = memory.device, _stream(memory), ctx_.splits
-        d_ctx = d_ctx.contiguous().float() if d_ctx is not None else torch.zeros_like(ctx)
-        d_anchor = d_anchor.contiguous().float() if d_anchor is not None else torch.zeros_like(anchor)
-        d_summary = d_summary.contiguous().float() if d_summary is not None else None
-        d_mem = torch.zeros(B, Np, D, device=dev) if Q > 32 else padded(B, N, D, dev)
-        dq_part = torch.empty(B * splits, Q * (D + 1), device=dev)
-        with ktime("query_attn_bwd_kernel", 10.0 * B * N * Q * D):
-            _lib.call("rs_query_attn_bwd_f32", _p(memory), D, Np, 1, _p(traces), Fdim, _p(mask_u8), _p(mean), _p(rms), _p(count),
-                      _p(qk), _p(qb), _p(ctx), _p(anchor), _p(stats), _p(d_ctx), _p(d_anchor), _p(d_summary), B, N, Q, D,
-                      splits, _p(d_mem), D, Np, 1, _p(dq_part), st)
-        dq = torch.empty(Q * (D + 1), device=dev)
-        colsum(dq_part, dq)
-        dq = dq.view(Q, D + 1)
-        return d_mem, dq[:, :D].contiguous(), dq[:, D].contiguous(), None, None, None, None, None
+        d_mem, dqk, dqb = query_attn_bwd(*ctx_.saved_tensors, d_ctx, d_anchor, d_summary, ctx_.splits)
+        return d_mem, dqk, dqb, None, None, None, None, None
 
 
 @_lib.on_tensor_device
