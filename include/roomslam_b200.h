@@ -152,12 +152,6 @@ int rs_blk_gemm_nt(const void* A, int64_t a_cols, const int* a_kchunk, int k_blo
 int rs_blk_gemm_nt_drop(const void* A, int64_t a_cols, const int* a_kchunk, int k_blocks, const void* W, int n_tiles, void* C,
                         int64_t c_cols, int c_chunk0, int64_t n_blocks, const void* drop_bits, const float* drop_scale, int T,
                         void* stream);
-/* C[c_row0[mt] + i, j] (fp32, ldc) += sum over blocks (tile, t' = 1..T) of A_blk[:, (a_mchunk[mt])*8 + i] *
- * B_blk'[:, b_chunk0*8 + j] with B_blk' = the block b_shift time rows away (b_broadcast != 0: B is ONE block used
- * for every (tile, t'), e.g. a column of ones for bias gradients); n_cols % 16 == 0.  HOST arrays. */
-int rs_blk_gemm_tn_acc(const void* A, int64_t a_cols, const int* a_mchunk, const int* c_row0, int m_tiles, const void* B,
-                       int64_t b_cols, int b_chunk0, int n_cols, int b_shift, int b_broadcast, float* C, int64_t ldc,
-                       int tiles, int T, void* stream);
 /* Fused weight-gradient pass of one layer: every role r < n_roles (<= 18) accumulates C[r][128, n_cols[r]] += sum over
  * blocks dG_blk[:, a_mchunk[r]*8 .. +128]^T . B[r]_blk'[:, b_chunk0[r]*8 .. + n_cols[r]] (time shift b_shift[r]; n_cols
  * may be 0), when bias[r] != NULL bias[r][128] += column sums of the same dG columns, and when B2[r] != NULL

@@ -83,7 +83,7 @@ int make_tmap_2d(CUtensorMap* out, const void* base, CUtensorMapDataType dtype, 
 }  // namespace rs
 
 extern "C" const char* rs_last_error(void) { return rs::g_error; }
-extern "C" int rs_abi_version(void) { return 1; }
+extern "C" int rs_abi_version(void) { return 2; }
 extern "C" int64_t rs_launch_count(void) { return (int64_t)__atomic_load_n(&rs::g_launches, __ATOMIC_RELAXED); }
 extern "C" int rs_device_ok(void) { return rs::check_device_sm100() == 0 ? 1 : 0; }
 extern "C" int rs_set_deterministic(int on) {

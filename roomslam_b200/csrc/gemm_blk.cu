@@ -10,9 +10,9 @@
 //
 //   blk_gemm_nt : per block m:  C_blk[:, n] = A_blk[:, kchunks] . W[n, :]^T + bias      (bf16 out, direct stores)
 //                 -> input projection P = X W_ih^T + b  and  dX = dG W_ih
-//   blk_gemm_tn : C[M, N] += sum over blocks  A_blk[:, mchunks]^T . B_blk'[:, nchunks]   (fp32 out, split over blocks)
+//   blk_wgrad   : C[M, N] += sum over blocks  A_blk[:, mchunks]^T . B_blk'[:, nchunks]   (fp32 out, split over blocks)
 //                 (the split reductions end in fp32 atomics; deterministic mode stores per-split partials into a workspace
-//                 and rs::slot_sum adds them in split order, here and in blk_wgrad)
+//                 and rs::slot_sum adds them in split order)
 //                 -> dW_ih, dW_hh (block of dG at t' paired with the block of h at t' -/+ 1), bias gradients (ones column)
 //
 // Warp roles: warp 0 = bulk-copy producer, warp 1 = tcgen05.mma issuer (one lane), warps 2..5 = TMEM epilogue.
@@ -25,7 +25,7 @@ namespace {
 
 constexpr int CHUNK_BYTES = 2048;          // one 16-byte column chunk of a 128-trace block
 constexpr int PIECE_BYTES = 8 * CHUNK_BYTES;   // 64 columns x 128 traces = 16 KB
-constexpr int NT_STAGES_MAX = 6;           // ring depth (5 resident / 6 streaming): look-ahead that covers the L2 latency of the W pieces
+constexpr int NT_STAGES = 6;               // ring depth: look-ahead that covers the L2 latency of the W pieces
 constexpr int NT_MAX_KB = 24;             // 12 K blocks of the data gradient, twice with split (hi + lo) weights
 constexpr int NUM_THREADS = 192;
 
@@ -43,23 +43,19 @@ struct NtParams {
 constexpr int NT_THREADS = 320;            // warp 0 producer, warp 1 MMA issuer, warps 2..9 epilogue (2 per TMEM lane quadrant)
 constexpr int NT_MAX_N = 1024;             // bias staged in shared memory
 
-template <bool kResident>
 __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
-    // resident: two A blocks (2 x 64 KB, double-buffered across blocks) + ring of W pieces (16 KB each)
-    // streaming: ring of (A piece | W piece) stages (32 KB each)
-    constexpr int kStageBytes = kResident ? PIECE_BYTES : 2 * PIECE_BYTES;
-    constexpr int NT_STAGES = kResident ? 5 : 6;
-    uint8_t* a_res = smem;
-    uint8_t* stages = smem + (kResident ? 2 * 4 * PIECE_BYTES : 0);
+    // ring of (A piece | W piece) stages (32 KB each)
+    constexpr int kStageBytes = 2 * PIECE_BYTES;
+    uint8_t* stages = smem;
     float* bias_s = reinterpret_cast<float*>(stages + NT_STAGES * kStageBytes);
     uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + NT_MAX_N);
     uint64_t* full_bar = bars;                       // [NT_STAGES]
     uint64_t* empty_bar = bars + NT_STAGES;          // [NT_STAGES]
     uint64_t* acc_full = bars + 2 * NT_STAGES;       // [2]
     uint64_t* acc_empty = bars + 2 * NT_STAGES + 2;  // [2]
-    uint64_t* a_full = bars + 2 * NT_STAGES + 4;     // [2] resident A block landed
-    uint64_t* a_empty = bars + 2 * NT_STAGES + 6;    // [2] MMAs of that block retired
+    // [4] unused barriers, still initialised: removing them changes this kernel's machine code, a change to measure on its own
+    uint64_t* spare = bars + 2 * NT_STAGES + 4;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * NT_STAGES + 8);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
@@ -67,7 +63,7 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
         for (int s = 0; s < NT_STAGES; ++s) { rs::mbar_init(&full_bar[s], 1); rs::mbar_init(&empty_bar[s], 1); }
         for (int s = 0; s < 2; ++s) {
             rs::mbar_init(&acc_full[s], 1); rs::mbar_init(&acc_empty[s], 8);
-            rs::mbar_init(&a_full[s], 1);   rs::mbar_init(&a_empty[s], 1);
+            rs::mbar_init(&spare[s], 1);    rs::mbar_init(&spare[2 + s], 1);
         }
         rs::fence_mbar_init();
     }
@@ -80,26 +76,17 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
 
     if (warp == 0) {
         if (rs::elect_one()) {
-            int stage = 0; uint32_t phase = 0; int ab = 0; uint32_t a_phase = 0;
+            int stage = 0; uint32_t phase = 0;
             for (int m = blockIdx.x; m < p.n_blocks; m += gridDim.x) {
                 const uint8_t* ablk = p.A + (long long)m * p.a_block_bytes;
-                if (kResident) {
-                    rs::mbar_wait(&a_empty[ab], a_phase ^ 1);
-                    rs::mbar_expect_tx(&a_full[ab], p.k_blocks * PIECE_BYTES);
-                    for (int kb = 0; kb < p.k_blocks; ++kb)
-                        rs::bulk_load(a_res + (ab * 4 + kb) * PIECE_BYTES, ablk + (long long)p.a_kchunk[kb] * CHUNK_BYTES, PIECE_BYTES,
-                                      &a_full[ab]);
-                    if (++ab == 2) { ab = 0; a_phase ^= 1; }
-                }
                 for (int n = 0; n < p.n_tiles; ++n) {
                     for (int kb = 0; kb < p.k_blocks; ++kb) {
                         rs::mbar_wait(&empty_bar[stage], phase ^ 1);
                         uint8_t* ss = stages + stage * kStageBytes;
                         rs::mbar_expect_tx(&full_bar[stage], kStageBytes);
-                        if (!kResident)
-                            rs::bulk_load(ss, ablk + (long long)p.a_kchunk[kb] * CHUNK_BYTES, PIECE_BYTES, &full_bar[stage]);
-                        rs::bulk_load(ss + (kResident ? 0 : PIECE_BYTES), p.W + ((long long)n * p.k_blocks + kb) * PIECE_BYTES,
-                                      PIECE_BYTES, &full_bar[stage]);
+                        rs::bulk_load(ss, ablk + (long long)p.a_kchunk[kb] * CHUNK_BYTES, PIECE_BYTES, &full_bar[stage]);
+                        rs::bulk_load(ss + PIECE_BYTES, p.W + ((long long)n * p.k_blocks + kb) * PIECE_BYTES, PIECE_BYTES,
+                                      &full_bar[stage]);
                         if (++stage == NT_STAGES) { stage = 0; phase ^= 1; }
                     }
                 }
@@ -107,9 +94,8 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
         }
     } else if (warp == 1) {
         constexpr uint32_t idesc = rs::umma_idesc_bf16(128, 128, 0, 0);
-        int stage = 0; uint32_t phase = 0; int ab = 0; uint32_t a_phase = 0; int acc = 0; uint32_t acc_phase = 0;
+        int stage = 0; uint32_t phase = 0; int acc = 0; uint32_t acc_phase = 0;
         for (int m = blockIdx.x; m < p.n_blocks; m += gridDim.x) {
-            if (kResident) { rs::mbar_wait(&a_full[ab], a_phase); rs::tc_fence_after(); }
             for (int n = 0; n < p.n_tiles; ++n) {
                 rs::mbar_wait(&acc_empty[acc], acc_phase ^ 1);
                 rs::tc_fence_after();
@@ -118,9 +104,8 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
                     rs::mbar_wait(&full_bar[stage], phase);
                     rs::tc_fence_after();
                     if (rs::elect_one()) {
-                        const uint32_t ss = rs::smem_u32(stages + stage * kStageBytes);
-                        const uint32_t sa = kResident ? rs::smem_u32(a_res + (ab * 4 + kb) * PIECE_BYTES) : ss;
-                        const uint32_t sb = kResident ? ss : ss + PIECE_BYTES;
+                        const uint32_t sa = rs::smem_u32(stages + stage * kStageBytes);
+                        const uint32_t sb = sa + PIECE_BYTES;
 #pragma unroll
                         for (int k = 0; k < 4; ++k) {
                             const uint64_t da = rs::umma_desc_noswz(sa + k * 2 * CHUNK_BYTES, CHUNK_BYTES, 128);
@@ -128,17 +113,13 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
                             rs::tc_mma_bf16(tmem_d, da, db, idesc, (kb | k) != 0);
                         }
                         rs::tc_commit(&empty_bar[stage]);
-                        if (kb == p.k_blocks - 1) {
-                            rs::tc_commit(&acc_full[acc]);
-                            if (kResident && n == p.n_tiles - 1) rs::tc_commit(&a_empty[ab]);
-                        }
+                        if (kb == p.k_blocks - 1) rs::tc_commit(&acc_full[acc]);
                     }
                     __syncwarp();
                     if (++stage == NT_STAGES) { stage = 0; phase ^= 1; }
                 }
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
-            if (kResident && ++ab == 2) { ab = 0; a_phase ^= 1; }
         }
     } else {
         const int q = warp & 3, row = q * 32 + lane;
@@ -193,243 +174,6 @@ __global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_kernel(const NtPara
                 if (++acc == 2) { acc = 0; acc_phase ^= 1; }
             }
         }
-    }
-    rs::tc_fence_before();
-    __syncthreads();
-    if (warp == 1) rs::tmem_dealloc<256>(tmem_base);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// Weight-resident variant for the input projection (K <= 256, N a multiple of 256).  The kernel above re-streams the
-// whole W (N x K: 384 KB for the layer-1 projection) through shared memory for EVERY 128-trace block: 448 KB of L2->SM
-// traffic and ~1.2 MB of shared-memory traffic per block against 786 KB the SM can move while the tensor core does the
-// block's 50 MFLOP -- shared-memory bandwidth, not HBM, bounds it.  Here a CTA owns ONE 256-column slice of W (128 KB,
-// loaded once, resident for the whole launch) and streams only the A blocks (64 KB each, 16 KB pieces through a ring);
-// the CTAs of a group (one per W slice) walk the same blocks at the same time, so A comes from HBM once and from L2 for
-// the other slices.  MMA shape 128 x 256 x 16; two 256-column accumulators (all 512 TMEM columns) overlap the
-// epilogue of one block with the MMAs of the next.
-constexpr int WRES_STAGES = 5;
-__global__ void __launch_bounds__(NT_THREADS, 1) blk_gemm_nt_wres_kernel(const NtParams p, int n_parts) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint8_t* w_s = smem;                                           // [k_blocks][8 chunks][256 rows][16 B]
-    uint8_t* stages = smem + p.k_blocks * 2 * PIECE_BYTES;         // ring of A pieces
-    float* bias_s = reinterpret_cast<float*>(stages + WRES_STAGES * PIECE_BYTES);   // [256]
-    uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + 256);
-    uint64_t* full_bar = bars;                        // [WRES_STAGES]
-    uint64_t* empty_bar = bars + WRES_STAGES;         // [WRES_STAGES]
-    uint64_t* acc_full = bars + 2 * WRES_STAGES;      // [2]
-    uint64_t* acc_empty = bars + 2 * WRES_STAGES + 2; // [2]
-    uint64_t* w_full = bars + 2 * WRES_STAGES + 4;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * WRES_STAGES + 5);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int part = blockIdx.x % n_parts, group = blockIdx.x / n_parts, groups = gridDim.x / n_parts;
-
-    if (warp == 0 && lane == 0) {
-        for (int s = 0; s < WRES_STAGES; ++s) { rs::mbar_init(&full_bar[s], 1); rs::mbar_init(&empty_bar[s], 1); }
-        for (int s = 0; s < 2; ++s) { rs::mbar_init(&acc_full[s], 1); rs::mbar_init(&acc_empty[s], 8); }
-        rs::mbar_init(w_full, 1);
-        rs::fence_mbar_init();
-    }
-    if (warp == 1) rs::tmem_alloc<512>(tmem_slot);
-    for (int i = threadIdx.x; i < 256; i += NT_THREADS) bias_s[i] = p.bias ? p.bias[part * 256 + i] : 0.0f;
-    rs::tc_fence_before();
-    __syncthreads();
-    rs::tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    if (warp == 0) {
-        if (rs::elect_one()) {
-            // W slice: the two 128-row pieces of every K block are interleaved chunk by chunk into 256-row chunk columns
-            rs::mbar_expect_tx(w_full, p.k_blocks * 2 * PIECE_BYTES);
-            for (int kb = 0; kb < p.k_blocks; ++kb)
-                for (int half = 0; half < 2; ++half) {
-                    const uint8_t* src = p.W + ((long long)(part * 2 + half) * p.k_blocks + kb) * PIECE_BYTES;
-                    for (int c = 0; c < 8; ++c)
-                        rs::bulk_load(w_s + kb * 2 * PIECE_BYTES + c * 2 * CHUNK_BYTES + half * CHUNK_BYTES, src + c * CHUNK_BYTES,
-                                      CHUNK_BYTES, w_full);
-                }
-            int stage = 0; uint32_t phase = 0;
-            for (int m = group; m < p.n_blocks; m += groups) {
-                const uint8_t* ablk = p.A + (long long)m * p.a_block_bytes;
-                for (int kb = 0; kb < p.k_blocks; ++kb) {
-                    rs::mbar_wait(&empty_bar[stage], phase ^ 1);
-                    rs::mbar_expect_tx(&full_bar[stage], PIECE_BYTES);
-                    rs::bulk_load(stages + stage * PIECE_BYTES, ablk + (long long)p.a_kchunk[kb] * CHUNK_BYTES, PIECE_BYTES, &full_bar[stage]);
-                    if (++stage == WRES_STAGES) { stage = 0; phase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        constexpr uint32_t idesc = rs::umma_idesc_bf16(128, 256, 0, 0);
-        rs::mbar_wait(w_full, 0);
-        rs::tc_fence_after();
-        int stage = 0; uint32_t phase = 0; int acc = 0; uint32_t acc_phase = 0;
-        const uint32_t w_addr = rs::smem_u32(w_s);
-        for (int m = group; m < p.n_blocks; m += groups) {
-            rs::mbar_wait(&acc_empty[acc], acc_phase ^ 1);
-            rs::tc_fence_after();
-            const uint32_t tmem_d = tmem_base + acc * 256;
-            for (int kb = 0; kb < p.k_blocks; ++kb) {
-                rs::mbar_wait(&full_bar[stage], phase);
-                rs::tc_fence_after();
-                if (rs::elect_one()) {
-                    const uint32_t sa = rs::smem_u32(stages + stage * PIECE_BYTES);
-                    const uint32_t sb = w_addr + kb * 2 * PIECE_BYTES;
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        const uint64_t da = rs::umma_desc_noswz(sa + k * 2 * CHUNK_BYTES, CHUNK_BYTES, 128);
-                        const uint64_t db = rs::umma_desc_noswz(sb + k * 2 * (2 * CHUNK_BYTES), 2 * CHUNK_BYTES, 128);
-                        rs::tc_mma_bf16(tmem_d, da, db, idesc, (kb | k) != 0);
-                    }
-                    rs::tc_commit(&empty_bar[stage]);
-                    if (kb == p.k_blocks - 1) rs::tc_commit(&acc_full[acc]);
-                }
-                __syncwarp();
-                if (++stage == WRES_STAGES) { stage = 0; phase ^= 1; }
-            }
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    } else {
-        const int q = warp & 3, row = q * 32 + lane;
-        const int chalf = (warp - 2) >> 2;              // which 128 of the slice's 256 columns this warp converts
-        int acc = 0; uint32_t acc_phase = 0;
-        for (int m = group; m < p.n_blocks; m += groups) {
-            uint8_t* cblk = p.C + (long long)m * p.c_block_bytes + row * 16;
-            rs::mbar_wait(&acc_full[acc], acc_phase);
-            rs::tc_fence_after();
-            const uint32_t taddr = tmem_base + acc * 256 + chalf * 128 + (static_cast<uint32_t>(q * 32) << 16);
-#pragma unroll
-            for (int c0 = 0; c0 < 128; c0 += 32) {
-                uint32_t r[32];
-                rs::tmem_ld_32x32b_x32(taddr + c0, r);
-                rs::tmem_ld_wait();
-                const float* bs = bias_s + chalf * 128 + c0;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    uint32_t pk[4];
-                    const float4 b0 = *reinterpret_cast<const float4*>(bs + 8 * j);
-                    const float4 b1 = *reinterpret_cast<const float4*>(bs + 8 * j + 4);
-                    const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const float v0 = __uint_as_float(r[8 * j + 2 * e]) + bb[2 * e];
-                        const float v1 = __uint_as_float(r[8 * j + 2 * e + 1]) + bb[2 * e + 1];
-                        __nv_bfloat162 h2 = __floats2bfloat162_rn(v0, v1);
-                        pk[e] = *reinterpret_cast<uint32_t*>(&h2);
-                    }
-                    const int chunk = p.c_chunk0 + part * 32 + chalf * 16 + c0 / 8 + j;
-                    *reinterpret_cast<uint4*>(cblk + (long long)chunk * CHUNK_BYTES) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-                }
-            }
-            rs::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) rs::mbar_arrive(&acc_empty[acc]);
-            if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-        }
-    }
-    rs::tc_fence_before();
-    __syncthreads();
-    if (warp == 1) rs::tmem_dealloc<512>(tmem_base);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-constexpr int TN_MAX_MT = 8;
-struct TnParams {
-    const uint8_t* A;  long long a_block_bytes;  int a_mchunk[TN_MAX_MT];  int c_row0[TN_MAX_MT];
-    const uint8_t* B;  long long b_block_bytes;  int b_chunk0;  int n_cols;  int b_shift;   // B block = A block + b_shift
-    float* C;  long long ldc;
-    int m_tiles, tiles, T, Tp;          // logical blocks: (tile, t' = 1..T)
-    int splits, blocks_per_split;
-};
-
-// kDet: item (split, mt) stores its tile to p.C + ((split * m_tiles + mt) * 128 + row) * ldc (workspace, ldc = n_cols)
-template <bool kDet>
-__global__ void __launch_bounds__(NUM_THREADS, 1) blk_gemm_tn_kernel(const TnParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const int b_bytes = p.n_cols * 256;
-    const int stage_bytes = 2 * PIECE_BYTES + b_bytes;            // A: 16 chunks (32 KB) | B: n_cols/8 chunks
-    uint8_t* stages = smem;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 2 * stage_bytes);
-    uint64_t* full_bar = bars;        // [2]
-    uint64_t* empty_bar = bars + 2;   // [2]
-    uint64_t* acc_full = bars + 4;
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5);
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        for (int s = 0; s < 2; ++s) { rs::mbar_init(&full_bar[s], 1); rs::mbar_init(&empty_bar[s], 1); }
-        rs::mbar_init(acc_full, 1);
-        rs::fence_mbar_init();
-    }
-    if (warp == 1) rs::tmem_alloc<256>(tmem_slot);
-    rs::tc_fence_before();
-    __syncthreads();
-    rs::tc_fence_after();
-    const uint32_t tmem_base = *tmem_slot;
-
-    const int total_blocks = p.tiles * p.T;
-    const int items = p.m_tiles * p.splits;
-    int stage = 0; uint32_t phase = 0, acc_phase = 0;
-    for (int item = blockIdx.x; item < items; item += gridDim.x) {
-        const int mt = item % p.m_tiles, split = item / p.m_tiles;
-        const int i0 = split * p.blocks_per_split;
-        const int i1 = min(total_blocks, i0 + p.blocks_per_split);
-        if (warp == 0) {
-            if (rs::elect_one()) {
-                for (int i = i0; i < i1; ++i) {
-                    const long long blk = (long long)(i / p.T) * p.Tp + 1 + (i % p.T);
-                    rs::mbar_wait(&empty_bar[stage], phase ^ 1);
-                    uint8_t* sa = stages + stage * stage_bytes;
-                    rs::mbar_expect_tx(&full_bar[stage], 2 * PIECE_BYTES + b_bytes);
-                    rs::bulk_load(sa, p.A + blk * p.a_block_bytes + (long long)p.a_mchunk[mt] * CHUNK_BYTES, 2 * PIECE_BYTES,
-                                  &full_bar[stage]);
-                    rs::bulk_load(sa + 2 * PIECE_BYTES, p.B + (blk + p.b_shift) * p.b_block_bytes + (long long)p.b_chunk0 * CHUNK_BYTES,
-                                  b_bytes, &full_bar[stage]);
-                    if (++stage == 2) { stage = 0; phase ^= 1; }
-                }
-            }
-        } else if (warp == 1) {
-            const uint32_t idesc = rs::umma_idesc_bf16(128, p.n_cols, 1, 1);
-            for (int i = i0; i < i1; ++i) {
-                rs::mbar_wait(&full_bar[stage], phase);
-                rs::tc_fence_after();
-                if (rs::elect_one()) {
-                    const uint32_t sa = rs::smem_u32(stages + stage * stage_bytes);
-                    const uint32_t sb = sa + 2 * PIECE_BYTES;
-#pragma unroll
-                    for (int k = 0; k < 8; ++k) {       // 128 traces = 8 K-steps of 16
-                        const uint64_t da = rs::umma_desc_noswz(sa + k * 256, 128, CHUNK_BYTES);
-                        const uint64_t db = rs::umma_desc_noswz(sb + k * 256, 128, CHUNK_BYTES);
-                        rs::tc_mma_bf16(tmem_base, da, db, idesc, (i != i0) || (k != 0));
-                    }
-                    rs::tc_commit(&empty_bar[stage]);
-                    if (i == i1 - 1) rs::tc_commit(acc_full);
-                }
-                __syncwarp();
-                if (++stage == 2) { stage = 0; phase ^= 1; }
-            }
-        } else if (i1 > i0) {
-            const int q = warp & 3, row = q * 32 + lane;
-            rs::mbar_wait(acc_full, acc_phase);
-            rs::tc_fence_after();
-            const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
-            float* crow = p.C + (long long)((kDet ? (split * p.m_tiles + mt) * 128 : p.c_row0[mt]) + row) * p.ldc;
-            for (int c0 = 0; c0 < p.n_cols; c0 += 16) {
-                uint32_t r[16];
-                rs::tmem_ld_32x32b_x16(taddr + c0, r);
-                rs::tmem_ld_wait();
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    if (kDet) crow[c0 + j] = __uint_as_float(r[j]);
-                    else atomicAdd(crow + c0 + j, __uint_as_float(r[j]));
-                }
-            }
-            rs::tc_fence_before();
-        }
-        if (i1 > i0) acc_phase ^= 1;
-        // the single accumulator is reused by the next item: everyone meets here (rarely more than one item per CTA)
-        __syncthreads();
-        rs::tc_fence_after();
     }
     rs::tc_fence_before();
     __syncthreads();
@@ -655,26 +399,10 @@ static int blk_gemm_nt_impl(const void* A, int64_t a_cols, const int* a_kchunk, 
         p.drop_row_bytes = (int)(c_cols / 8);
     }
     const int grid = (int)(n_blocks < num_sms() ? n_blocks : num_sms());
-    static const bool wres_off = getenv("RS_NT_WRES") && atoi(getenv("RS_NT_WRES")) == 0;
-    if (k_blocks <= 4 && n_tiles % 2 == 0 && n_tiles / 2 <= 8 && n_blocks >= 2 * num_sms() && !wres_off && !drop_bits) {
-        // weight-resident: one CTA per (group, 256-column W slice); groups walk the blocks together
-        const int n_parts = n_tiles / 2;
-        const int groups = num_sms() / n_parts;
-        const int smem = k_blocks * 2 * PIECE_BYTES + WRES_STAGES * PIECE_BYTES + 256 * 4 + 256;
-        RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_nt_wres_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        blk_gemm_nt_wres_kernel<<<groups * n_parts, NT_THREADS, smem, stream>>>(p, n_parts);
-        rs::count_launch();
-    } else if (k_blocks <= 4) {
-        const int smem = 2 * 4 * PIECE_BYTES + 5 * PIECE_BYTES + NT_MAX_N * 4 + 256;
-        RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_nt_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        blk_gemm_nt_kernel<true><<<grid, NT_THREADS, smem, stream>>>(p);
-        rs::count_launch();
-    } else {
-        const int smem = 6 * 2 * PIECE_BYTES + NT_MAX_N * 4 + 256;
-        RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_nt_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        blk_gemm_nt_kernel<false><<<grid, NT_THREADS, smem, stream>>>(p);
-        rs::count_launch();
-    }
+    const int smem = NT_STAGES * 2 * PIECE_BYTES + NT_MAX_N * 4 + 256;
+    RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_nt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    blk_gemm_nt_kernel<<<grid, NT_THREADS, smem, stream>>>(p);
+    rs::count_launch();
     RS_CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -693,56 +421,6 @@ extern "C" int rs_blk_gemm_nt_drop(const void* A, int64_t a_cols, const int* a_k
                                    const float* drop_scale, int T, void* stream_) {
     RS_REQUIRE(drop_bits != nullptr, "rs_blk_gemm_nt_drop: drop_bits is required");
     return blk_gemm_nt_impl(A, a_cols, a_kchunk, k_blocks, W, n_tiles, C, c_cols, c_chunk0, nullptr, n_blocks, drop_bits, drop_scale, T, stream_);
-}
-
-extern "C" int rs_blk_gemm_tn_acc(const void* A, int64_t a_cols, const int* a_mchunk, const int* c_row0, int m_tiles,
-                                  const void* B, int64_t b_cols, int b_chunk0, int n_cols, int b_shift, int b_broadcast,
-                                  float* C, int64_t ldc, int tiles, int T, void* stream_) {
-    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-    if (rs::check_device_sm100()) return 3;
-    RS_REQUIRE(A && B && C && a_mchunk && c_row0, "rs_blk_gemm_tn_acc: null pointer");
-    RS_REQUIRE(m_tiles >= 1 && m_tiles <= TN_MAX_MT, "rs_blk_gemm_tn_acc: 1 <= m_tiles <= %d", TN_MAX_MT);
-    RS_REQUIRE(n_cols >= 16 && n_cols <= 256 && n_cols % 16 == 0, "rs_blk_gemm_tn_acc: n_cols must be a multiple of 16 in [16,256]");
-    RS_REQUIRE(b_shift >= -1 && b_shift <= 1 && tiles >= 0 && T >= 0, "rs_blk_gemm_tn_acc: bad arguments");
-    RS_REQUIRE((b_chunk0 * 8 + n_cols) <= b_cols && a_cols % 8 == 0 && b_cols % 8 == 0, "rs_blk_gemm_tn_acc: B columns outside the block");
-    const long long total = (long long)tiles * T;
-    if (total == 0) return 0;
-    RS_REQUIRE(total < (1ll << 31), "rs_blk_gemm_tn_acc: too many blocks");
-    TnParams p = {};
-    p.A = static_cast<const uint8_t*>(A); p.a_block_bytes = a_cols * 256;
-    for (int i = 0; i < m_tiles; ++i) {
-        RS_REQUIRE(a_mchunk[i] >= 0 && (a_mchunk[i] + 16) * 8 <= a_cols, "rs_blk_gemm_tn_acc: M tile %d outside the A block", i);
-        p.a_mchunk[i] = a_mchunk[i]; p.c_row0[i] = c_row0[i];
-    }
-    p.B = static_cast<const uint8_t*>(B); p.b_block_bytes = b_broadcast ? 0 : b_cols * 256; p.b_chunk0 = b_chunk0; p.n_cols = n_cols; p.b_shift = b_shift;
-    p.C = C; p.ldc = ldc; p.m_tiles = m_tiles; p.tiles = tiles; p.T = T; p.Tp = T + 2;
-    const bool det = rs::deterministic();
-    int splits = (det ? rs::kDetSplitSms : num_sms()) / m_tiles;
-    if (splits < 1) splits = 1;
-    if (splits > total) splits = (int)total;
-    p.blocks_per_split = (int)((total + splits - 1) / splits);
-    p.splits = (int)((total + p.blocks_per_split - 1) / p.blocks_per_split);
-    const int smem = 2 * (2 * PIECE_BYTES + n_cols * 256) + 256;
-    const int items = p.m_tiles * p.splits;
-    const int grid = items < num_sms() ? items : num_sms();
-    if (det) {
-        rs::StreamScratch ws(stream);
-        const long long slot = (long long)m_tiles * 128 * n_cols;
-        RS_CUDA_OK(ws.alloc(sizeof(float) * p.splits * slot));
-        p.C = ws.as<float>(); p.ldc = n_cols;
-        RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_tn_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        blk_gemm_tn_kernel<true><<<grid, NUM_THREADS, smem, stream>>>(p);
-        rs::count_launch();
-        RS_CUDA_OK(cudaGetLastError());
-        rs::SlotSum<float> jobs[TN_MAX_MT];
-        for (int i = 0; i < m_tiles; ++i) jobs[i] = {ws.as<float>() + (long long)i * 128 * n_cols, C + (long long)c_row0[i] * ldc, ldc, 128, n_cols};
-        return rs::slot_sum(jobs, m_tiles, p.splits, slot, true, stream);
-    }
-    RS_CUDA_OK(cudaFuncSetAttribute(blk_gemm_tn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    blk_gemm_tn_kernel<false><<<grid, NUM_THREADS, smem, stream>>>(p);
-    rs::count_launch();
-    RS_CUDA_OK(cudaGetLastError());
-    return 0;
 }
 
 // One launch for all weight / bias gradients of a layer.  Per role r < n_roles (HOST arrays of length n_roles):

@@ -3,7 +3,6 @@
 // cta_group::2); round 1's one-CTA-per-tile kernels lived here and were retired once the pair kernels beat them at every
 // batch size (DESIGN.md 4.2 has the A/B numbers).
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "rec_common.cuh"
@@ -38,13 +37,12 @@ __global__ void pack_x_tm_kernel(const float* __restrict__ x, int B, int T, int 
     }
 }
 
-int pf_dist_env(const char* name, int dflt) {
-    const char* e = getenv(name);
-    int v = e ? atoi(e) : dflt;
-    if (v < 0) v = 0;
-    if (v > 64) v = 64;
-    return v;
-}
+// L2 prefetch distance in steps (0 = off): forward, of the projection blocks P; backward, of the gate / d_out blocks, issued
+// by the thread that also issues the h_{t-1} tile copies.  The backward one was measured once single-thread issue had become
+// cheap (elect.sync): BPTT at 8192 traces 3.14 / 3.30 ms per layer without, 2.94 / 3.21 with distance 1, 3.11 / 3.53 with
+// 2, 3.43 / 3.94 with 4 (evicted before use); at 1024 traces 1.16 / 1.18 -> 1.13 / 1.14 ms.
+constexpr int PF_DIST_FWD = 1;
+constexpr int PF_DIST_BWD = 1;
 
 }  // namespace
 
@@ -69,7 +67,7 @@ extern "C" int rs_rec_fwd_bf16(const float* x, int I, const void* P, int64_t p_c
     RS_REQUIRE((drop_bits != nullptr) == (out_drop != nullptr) && (!drop_bits || drop_scale),
                "rs_rec_fwd_bf16: drop_bits, drop_scale and out_drop go together");
     return rs::rec_fwd_pair(x, I, P, X, Wih, Whh, b_hn, out, gates, h_n, lengths, drop_bits, drop_scale, out_drop, split, B, T,
-                            rs::rec_fwd_nt(B), pf_dist_env("RS_PF_DIST_FWD", 1), stream);
+                            rs::rec_fwd_nt(B), PF_DIST_FWD, stream);
 }
 
 extern "C" int rs_rec_bwd_bf16(const void* d_out, const float* d_h_n, const void* gates, const void* out, const void* WhhT,
@@ -81,12 +79,8 @@ extern "C" int rs_rec_bwd_bf16(const void* d_out, const float* d_h_n, const void
     RS_REQUIRE(gates && out && WhhT && Whh && b_hn && dG && B >= 0 && T >= 0, "rs_rec_bwd_bf16: bad arguments");
     RS_REQUIRE(whh_chunks >= 16 * (split ? 2 : 1), "rs_rec_bwd_bf16: Whh is the forward image (16 hidden chunks, twice with split)");
     RS_REQUIRE(!drop_bits || drop_scale, "rs_rec_bwd_bf16: drop_bits needs drop_scale");
-    // L2 prefetch of the gate / d_out blocks RS_PF_DIST_BWD steps ahead (default 1; issued by the thread that also issues the
-    // h_{t-1} tile copies).  Measured once single-thread issue had become cheap (elect.sync): BPTT at 8192 traces 3.14 / 3.30 ms
-    // per layer without, 2.94 / 3.21 with distance 1, 3.11 / 3.53 with 2, 3.43 / 3.94 with 4 (evicted before use); at 1024
-    // traces 1.16 / 1.18 -> 1.13 / 1.14 ms.
     return rs::rec_bwd_pair(d_out, d_h_n, gates, out, WhhT, Whh, whh_chunks, b_hn, dG, lengths, drop_bits, drop_scale, split, B, T,
-                            pf_dist_env("RS_PF_DIST_BWD", 1), stream);
+                            PF_DIST_BWD, stream);
 }
 
 extern "C" int rs_pack_x_tm(const float* x, int B, int T, int I, void* out, void* stream_) {

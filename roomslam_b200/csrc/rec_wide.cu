@@ -3,14 +3,13 @@
 // = half of the hidden units), same tile-major operands -- but W_hh (3H x H bf16 = 384 KB) no longer fits: half of it per
 // CTA would be 192 KB next to the h tile and the fp32 master state.  So W is NOT resident: each CTA streams its half
 // (the gate rows of its 128 hidden units) from L2 through a ring of 24 KB bulk copies (cp.async.bulk, mbarrier full /
-// empty pairs; 5 to 7 stages), once per time step, while the tensor core consumes it K = 16 step by K = 16 step.  The ring
+// empty pairs; RING_STAGES = 4 stages), once per time step, while the tensor core consumes it K = 16 step by K = 16 step.  The ring
 // runs ahead of the recurrence: most of step t+1's weights land during the epilogue of step t, the rest under the MMA
 // itself.  The whole of W_hh for both directions is 768 KB and stays L2-resident; 32 CTAs at batch 1024 pull ~2 TB/s from
 // L2, nothing from HBM.  (An odd CTA's stage arrival is relayed to the issuing CTA by its otherwise idle warp 0.)
 //   forward : G[64 x 768 per CTA] = h_{t-1}[64 x 256] . W_hh^T, 3 MMAs (N = 256: r, z, hn) per K step, 16 (+1) K steps
 //   backward: dh[64 x 256] = z (.) dh + dGh[64 x 768] . W_hh,   1 MMA (N = 256) per K step, 48 K steps
 // The epilogues are those of rec_pair.cu with 32 hidden units per thread (16 warps per CTA).
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "rec_common.cuh"
@@ -624,11 +623,10 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
     if (warp == 0) tmem_dealloc_pair<128>(tmem_base);
 }
 
-int ring_stages(const char* env, int dflt, int max) {
-    const char* e = getenv(env);
-    int v = e ? atoi(e) : dflt;
-    return v < 2 ? 2 : (v > max ? max : v);
-}
+// Ring depth of the weight stream, the same in all three launches (layer 0 forward, deeper forward, backward).  More stages
+// hide more of the L2 latency of the weight stream but every 24 KB of shared memory is taken from the L1 cache that backs
+// the epilogue's global loads (measured, tools/c4_probe.py: see DESIGN.md 4.4).
+constexpr int RING_STAGES = 4;
 
 }  // namespace
 
@@ -659,9 +657,7 @@ extern "C" int rs_rec_fwd_bf16_wide(const float* x, int I, const void* P, const 
     p.gates = static_cast<uint8_t*>(gates); p.h_n = h_n; p.lengths = lengths;
     p.drop_bits = static_cast<const uint8_t*>(drop_bits); p.drop_scale = drop_scale; p.out_drop = static_cast<uint8_t*>(out_drop);
     p.B = B; p.T = T; p.n_tiles = (B + 127) / 128;
-    // Ring depth.  More stages hide more of the L2 latency of the weight stream but every 24 KB of shared memory is taken
-    // from the L1 cache that backs the epilogue's global loads (measured, tools/c4_probe.py: see DESIGN.md 4.4)
-    p.nstage = ring_stages(x ? "RS_WIDE_STAGES_FWD0" : "RS_WIDE_STAGES_FWD", 4, x ? 5 : 7);
+    p.nstage = RING_STAGES;
     const int xc = x ? rs::x_chunks(I) : 1;         // layer 0: 16-byte input chunks per row (kXC of the kernel)
     const int smem = p.nstage * WSTAGE + (x ? H32_BYTES : 0) + (HW / 8 + 2 * ((xc + 1) / 2)) * CHUNK_S + HW * 4 + (int)sizeof(RingBars) + 64;
     const dim3 grid(2 * p.n_tiles, 2);
@@ -707,7 +703,7 @@ extern "C" int rs_rec_bwd_bf16_wide(const void* d_out, const float* d_h_n, const
     p.lengths = lengths;
     p.drop_bits = static_cast<const uint8_t*>(drop_bits); p.drop_scale = drop_scale;
     p.B = B; p.T = T; p.n_tiles = (B + 127) / 128;
-    p.nstage = ring_stages("RS_WIDE_STAGES_BWD", 4, 5);
+    p.nstage = RING_STAGES;
     const int smem = p.nstage * WSTAGE + A_BWD_BYTES + (int)sizeof(RingBars) + 64;
 #define RS_LAUNCH_BWDW(VL_, DROP_)                                                                                      \
     do {                                                                                                                \

@@ -12,7 +12,6 @@ ONE time-parallel GEMM with a one-row pointer shift.
 from __future__ import annotations
 
 import ctypes
-import os
 from typing import List, Optional, Tuple
 
 import torch
@@ -116,7 +115,7 @@ def colsum(a2d: torch.Tensor, out: torch.Tensor, accumulate=False):
 # accumulator, so the result is fp32-grade -- at tensor-core instead of CUDA-core speed.  Used when the row count is
 # large enough to matter.
 TC_MIN_ROWS = 4096
-TC_ENABLED = os.environ.get("RS_TC_GEMM", "1") != "0"
+TC_ENABLED = True                   # tests set it False to reach the CUDA-core SGEMM path
 OUT_F32 = 4
 _HI, _MID, _LO = 5, 2, 0            # column sixths of an A-role buffer that hold hi, mid, lo
 

@@ -13,7 +13,6 @@ weight gradients are fp32.  Tolerance against the fp32 CPU oracle: 2e-2 relative
 from __future__ import annotations
 
 import ctypes
-import os
 from typing import Optional
 
 import torch
@@ -55,12 +54,6 @@ def _nt(A, a_cols, kchunks, W_tiled, n_tiles, C, c_cols, c_chunk0, bias, n_block
         return
     _lib.call("rs_blk_gemm_nt", _p(A), a_cols, ctypes.addressof(kch), len(kchunks), _p(W_tiled), n_tiles, _p(C), c_cols,
               c_chunk0, _p(bias), n_blocks, st)
-
-
-def _tn(A, a_cols, mchunks, rows, Bm, b_cols, b_chunk0, n_cols, shift, bcast, C, ldc, tiles, T, st):
-    mch, r0 = L.int_array(mchunks), L.int_array(rows)
-    _lib.call("rs_blk_gemm_tn_acc", _p(A), a_cols, ctypes.addressof(mch), ctypes.addressof(r0), len(mchunks), _p(Bm), b_cols,
-              b_chunk0, n_cols, shift, int(bcast), _p(C), ldc, tiles, T, st)
 
 
 def _wgrad(dG, a_cols, ones, roles, tiles, T, st):
@@ -170,9 +163,8 @@ class GRULayerBF16Fn(torch.autograd.Function):
             # no projection GEMM) whenever the weights are not split into hi + lo pairs (W_ih hi + lo would not fit).  Since the
             # X tile copies are issued by one elected thread the fused kernel is within 6 % of the plain one per time step, and
             # the projection launch it replaces costs more than that at every batch size (training step at 1024 / 2048 / 4096 /
-            # 8192 traces: 5.85 -> 5.72, 6.83 -> 6.52, 9.55 -> 8.93, 19.6 -> 18.3 ms).  RS_FUSE_PROJ=0/1 forces.
-            fuse_env = os.environ.get("RS_FUSE_PROJ")
-            fuse_proj = padded_in and not split and (fuse_env == "1" if fuse_env in ("0", "1") else True)
+            # 8192 traces: 5.85 -> 5.72, 6.83 -> 6.52, 9.55 -> 8.93, 19.6 -> 18.3 ms).
+            fuse_proj = padded_in and not split
             if not padded_in:
                 _check_x_inputs(Il)
             x_chunks = 2 * x_steps(Il) if not padded_in else (2 if fuse_proj else 0)   # input columns (layer 0) / bias (fused)

@@ -233,35 +233,32 @@ def test_device_drawn_dropout_bits_match_the_oracle_with_the_same_mask():
 
 
 @pytest.mark.parametrize("B,T,use_mask,varlen", [(130, 40, False, False), (300, 64, True, False), (260, 50, False, True), (1100, 30, False, False)])
-def test_fused_projection_matches_the_projection_gemm_path(B, T, use_mask, varlen, monkeypatch):
+def test_fused_projection_meets_the_oracle(B, T, use_mask, varlen):
     """Deeper layers with unsplit weights run the K = 256 input projection INSIDE the recurrence kernel (W_ih resident,
-    no P tensor, no projection GEMM).  Same operands as the projection-GEMM path, which rounds P to bf16 on the way: the two
-    must agree far inside the bf16 tolerance, and the fused path must meet the oracle like the other one does."""
+    no P tensor, no projection GEMM): h_n, the losses and the encoder gradients against the fp32 oracle within 2e-2."""
     torch.manual_seed(B)
     ref = RefRoomSLAM(dropout=0.1 if use_mask else 0.0)
     ref.train(use_mask)
     x, tgt = synth.make_sample(B, T, 10, seed=B)
     mask = ref.make_dropout_mask(B, T, torch.Generator().manual_seed(1)) if use_mask else None
     lengths = torch.randint(1, T + 1, (B,), generator=torch.Generator().manual_seed(2)) if varlen else None
-    res = {}
-    for fuse in ("1", "0"):
-        monkeypatch.setenv("RS_FUSE_PROJ", fuse)
-        dev = RoomSLAM(dropout=ref.dropout, precision="bf16", bf16_split_weights=False).cuda()
-        dev.load_state_dict(ref.state_dict())
-        dev.train(use_mask)
-        xm = mask.cuda() if mask is not None else None
-        _, h_n = dev.encode(x.cuda(), xm, lengths)
-        loss = dev.compute_loss(dev(x.cuda(), xm, lengths), to_cuda(tgt))
-        loss["total"].backward()
-        res[fuse] = (h_n.detach().cpu(), {k: v.item() for k, v in loss.items()}, {k: p.grad.detach().cpu() for k, p in dev.named_parameters()})
-    assert rel_err(res["1"][0], res["0"][0]) < 5e-3
+    dev = RoomSLAM(dropout=ref.dropout, precision="bf16", bf16_split_weights=False).cuda()
+    dev.load_state_dict(ref.state_dict())
+    dev.train(use_mask)
+    xm = mask.cuda() if mask is not None else None
+    _, hn_dev = dev.encode(x.cuda(), xm, lengths)
+    loss_dev = dev.compute_loss(dev(x.cuda(), xm, lengths), to_cuda(tgt))
+    loss_dev["total"].backward()
+    _, hn_ref = ref.encode(x, mask, lengths)
+    loss_ref = ref.compute_loss(ref(x, mask, lengths), tgt)
+    loss_ref["total"].backward()
+    assert rel_err(hn_dev, hn_ref) < RTOL
     for k in LOSS_KEYS:
-        assert abs(res["1"][1][k] - res["0"][1][k]) <= 5e-3 * max(abs(res["0"][1][k]), 1e-6), k
-    bad = {k: l2_err(res["1"][2][k], res["0"][2][k]) for k in res["0"][2] if k.startswith("encoder.")}
+        assert abs(loss_dev[k].item() - loss_ref[k].item()) <= RTOL * max(abs(loss_ref[k].item()), 1e-6), k
+    ref_grads = dict(ref.named_parameters())
+    bad = {pn: l2_err(p.grad, ref_grads[pn].grad) for pn, p in dev.named_parameters() if pn.startswith("encoder.")}
     bad = {k: v for k, v in bad.items() if not v < RTOL}
     assert not bad, bad
-    _, hn_ref = ref.encode(x, mask, lengths) if not varlen else ref.encode(x, None, lengths)
-    assert rel_err(res["1"][0], hn_ref) < RTOL
 
 
 @pytest.mark.parametrize("H,B,T", [(128, 300, 40), (128, 1100, 24), (256, 200, 24)])

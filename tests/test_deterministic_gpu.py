@@ -172,29 +172,6 @@ def test_gemm_bf16_tn_seg_acc(det):
 
 
 @pytest.mark.gpu
-def test_blk_gemm_tn_acc(det):
-    torch.manual_seed(3)
-    B, T, Ca, Cb, n_cols, shift = 300, 30, 1024, 256, 128, -1
-    mcols = [0, 128, 384]
-    a, b = torch.randn(B, T, Ca, device="cuda"), torch.randn(B, T, Cb, device="cuda")
-    at, bt = L.to_tile_major(a), L.to_tile_major(b)
-    mch, rows = L.int_array([c // 8 for c in mcols]), L.int_array([i * 128 for i in range(len(mcols))])
-
-    def run():
-        C = torch.ones(len(mcols) * 128, n_cols, device="cuda")
-        _lib.call("rs_blk_gemm_tn_acc", at.data_ptr(), Ca, ctypes.addressof(mch), ctypes.addressof(rows), len(mcols), bt.data_ptr(),
-                  Cb, 128 // 8, n_cols, shift, 0, C.data_ptr(), n_cols, at.shape[0], T, st())
-        return C
-    got = twice(run)
-    aa = torch.cat([a[..., c:c + 128] for c in mcols], -1).bfloat16().double()
-    src = b[..., 128:128 + n_cols].bfloat16().double()
-    bb = torch.zeros_like(src)
-    bb[:, 1:] = src[:, :-1]
-    ref = 1.0 + torch.einsum("btm,btn->mn", aa, bb)
-    assert rel_max(got, ref) < 1e-5
-
-
-@pytest.mark.gpu
 @pytest.mark.parametrize("paired", [True, False])
 def test_blk_wgrad(det, paired):
     from roomslam_b200.functional_bf16 import _ones_block, _wgrad

@@ -40,7 +40,6 @@ def test_gemm_bf16_tn_row_major(rows, M, N, sa, sb, ca, cb):
 @pytest.mark.parametrize("B,T,Ca,kcols,N,Cc,c0", [(128, 1, 64, [0], 128, 128, 0), (200, 5, 256, [0, 64, 128, 192], 768, 768, 0),
                                                     (300, 7, 1024, [0, 64, 128, 192, 256, 320, 512, 576, 640, 704, 768, 832], 256, 256, 0),
                                                     (128, 3, 128, [64], 128, 512, 256),
-                                                    # >= 2 x 148 blocks and an even number of N tiles: the weight-resident variant
                                                     (700, 60, 256, [0, 64, 128, 192], 768, 768, 0), (256, 149, 128, [0, 64], 256, 512, 128),
                                                     (1300, 40, 256, [64, 128, 192], 512, 1024, 256)])
 def test_blk_gemm_nt_tile_major(B, T, Ca, kcols, N, Cc, c0):
@@ -63,16 +62,18 @@ def test_blk_gemm_nt_tile_major(B, T, Ca, kcols, N, Cc, c0):
 
 
 @pytest.mark.parametrize("shift", [0, -1, 1])
-def test_blk_gemm_tn_tile_major_with_time_shift(shift):
+def test_blk_wgrad_tile_major_with_time_shift(shift):
+    """rs_blk_wgrad with three roles on dG columns 0, 128 and 384 against the time-shifted B columns 128..255, no bias, no
+    B2: C += sum over blocks dG_blk^T . B_blk'."""
+    from roomslam_b200.functional_bf16 import _ones_block, _wgrad
     torch.manual_seed(3)
     B, T, Ca, Cb, n_cols = 300, 9, 1024, 256, 128
     mcols = [0, 128, 384]
     a = torch.randn(B, T, Ca, device="cuda"); b = torch.randn(B, T, Cb, device="cuda")
     at, bt = L.to_tile_major(a), L.to_tile_major(b)
     C = torch.ones(len(mcols) * 128, n_cols, device="cuda")
-    mch = L.int_array([c // 8 for c in mcols]); rows = L.int_array([i * 128 for i in range(len(mcols))])
-    _lib.call("rs_blk_gemm_tn_acc", at.data_ptr(), Ca, ctypes.addressof(mch), ctypes.addressof(rows), len(mcols), bt.data_ptr(), Cb,
-              128 // 8, n_cols, shift, 0, C.data_ptr(), n_cols, at.shape[0], T, st())
+    roles = [(c // 8, bt, Cb, 128 // 8, n_cols, shift, C[i * 128:(i + 1) * 128], n_cols, None, None, None) for i, c in enumerate(mcols)]
+    _wgrad(at, Ca, _ones_block(torch.device("cuda")), roles, at.shape[0], T, st())
     aa = torch.cat([a[..., c:c + 128] for c in mcols], -1).bfloat16().float()
     src = b[..., 128:128 + n_cols].bfloat16().float()
     bb = torch.zeros_like(src)

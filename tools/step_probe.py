@@ -16,7 +16,7 @@ e0.record()
 for _ in range(3): step()
 e1.record(); torch.cuda.synchronize()
 F_.enable_kernel_timing(True); step(); k = F_.collect_kernel_timing(); F_.enable_kernel_timing(False)
-print(os.environ.get("RS_PF_DIST", "-"), "ms/step %.2f" % (e0.elapsed_time(e1) / 3), {n: round(v[0], 2) for n, v in k.items()})
+print("ms/step %.2f" % (e0.elapsed_time(e1) / 3), {n: round(v[0], 2) for n, v in k.items()})
 # per-launch detail (layer order: forward L0, L1; backward L1, L0)
 F_.enable_kernel_timing(True); step(); torch.cuda.synchronize()
 for name, a, b, fl in F_._KT["events"]:
