@@ -249,6 +249,23 @@ int rs_lstm_fwd_f32(const float* P, int64_t p_ld, int64_t p_rows, int64_t p_row0
 int rs_lstm_bwd_f32(const float* d_out, int64_t do_ld, int64_t do_rows, int64_t do_row0, const float* saved,
                     const float* w_hh, float* dG, int64_t g_ld, int64_t g_rows, int64_t g_row0, int B, int T, int H,
                     void* stream);
+/* bf16 tensor-core recurrence of the same layer, H = 128 only (d_model 256): any other H returns 1 and rs_last_error names the
+ * limit.  Same P / out / saved / d_out / dG operands as the fp32 pair above; W_hh h_{t-1} and dG_t W_hh run with bf16 operands
+ * and fp32 accumulation, everything else (gates, cell state, carries, stores) in fp32.  Pad rows of out and dG are not written;
+ * no atomics (reruns are bit-identical).
+ * rs_lstm_pack_weights_bf16 builds both weight images of a layer in one launch from W_hh of the forward (w_hh) and reverse
+ * (w_hh_r) direction, [4H][H] fp32 each.  split = 0: one bf16 part per weight; split = 1: hi = bf16(w) then lo = bf16(w - hi),
+ * which doubles K (the hi chunks come first, the lo chunks after them):
+ *   fwd_img [2][16 (x2)][4H][8] bf16: element (d, part * 16 + c, n, e) = part of W_d[n][8 c + e]   (2 * 128 KB unsplit)
+ *   bwd_img [2][64 (x2)][H][8]  bf16: element (d, part * 64 + c, u, e) = part of W_d[8 c + e][u]   (2 * 128 KB unsplit)
+ * rs_lstm_fwd_bf16 reads fwd_img and rs_lstm_bwd_bf16 bwd_img, with the split flag they were packed with.  P, out, saved,
+ * d_out and dG must be 16-byte aligned with row strides a multiple of 4 floats. */
+int rs_lstm_pack_weights_bf16(const float* w_hh, const float* w_hh_r, int H, int split, void* fwd_img, void* bwd_img, void* stream);
+int rs_lstm_fwd_bf16(const float* P, int64_t p_ld, int64_t p_rows, int64_t p_row0, const void* fwd_img, float* out,
+                     int64_t o_ld, int64_t o_rows, int64_t o_row0, float* saved, int B, int T, int H, int split, void* stream);
+int rs_lstm_bwd_bf16(const float* d_out, int64_t do_ld, int64_t do_rows, int64_t do_row0, const float* saved,
+                     const void* bwd_img, float* dG, int64_t g_ld, int64_t g_rows, int64_t g_row0, int B, int T, int H, int split,
+                     void* stream);
 /* Per-trace normaliser (model.py:38-46): mean [B,3] of the valid (x, y, z), rms [B] of the centred (x, z) (floor 1e-3),
  * count [B] = max(valid tokens, 1).  traces: [B, N, F]; mask: [B, N] uint8 or NULL. */
 int rs_trace_stats_f32(const float* traces, int F, const unsigned char* mask, int B, int N, float* mean, float* rms,

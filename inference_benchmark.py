@@ -15,12 +15,13 @@ from roomslam_b200.evaluation import post_process_predictions
 from roomslam_b200.lstm_model import build_model
 
 
-def load_model(checkpoint_path: str, device="cuda"):
-    """inference.py:8-21: the checkpoint's own config picks the architecture (defaults: 50 queries, d_model 256)."""
+def load_model(checkpoint_path: str, device="cuda", precision: str = "fp32"):
+    """inference.py:8-21: the checkpoint's own config picks the architecture (defaults: 50 queries, d_model 256).
+    precision "bf16" runs the LSTM recurrence on tensor cores (d_model 256); checkpoints load into either precision."""
     ck = torch.load(checkpoint_path, map_location="cpu", weights_only=False)
     config = ck.get("config", {})
     model = build_model(num_queries=config.get("num_queries", 50), d_model=config.get("d_model", 256),
-                        model_type=config.get("model_type", "lstm"))
+                        model_type=config.get("model_type", "lstm"), precision=precision)
     model.load_state_dict(ck["model_state_dict"], strict=True)
     return model.to(device).eval(), config
 
@@ -47,9 +48,11 @@ def main():
     ap.add_argument("--output", default=None, help="Output file for predictions")
     ap.add_argument("--threshold", type=float, default=0.7, help="Confidence threshold (default: 0.7)")
     ap.add_argument("--nms", type=float, default=0.3, help="NMS IoU threshold (default: 0.3)")
+    ap.add_argument("--precision", choices=("fp32", "bf16"), default="fp32",
+                    help="LSTM recurrence: fp32, or bf16 on tensor cores (d_model 256 checkpoints only)")
     args = ap.parse_args()
     print(f"Loading model from {args.checkpoint}")
-    model, _ = load_model(args.checkpoint)
+    model, _ = load_model(args.checkpoint, precision=args.precision)
     print(f"Processing {args.input}")
     preds = predict(model, args.input, args.threshold, args.nms)
     print(f"\nFound {len(preds)} colliders:")

@@ -89,14 +89,45 @@ def linear(x: torch.Tensor, w: torch.Tensor, b: Optional[torch.Tensor], allow_tc
     return LinearFn.apply(x.reshape(-1, x.shape[-1]), w, b, allow_tc).view(*lead, w.shape[0])
 
 
-def lstm_layer_fwd(xin, mask, weights, need_grad=True):
+PRECISIONS = ("fp32", "bf16")
+# Weight form of the bf16 recurrence: False = W_hh rounded to bf16 once, True = hi + lo bf16 parts (K doubles).  The
+# cheapest form that keeps the model within 2e-2 of fp32 at 20 x 3000 (DESIGN.md section 7.2).
+LSTM_BF16_SPLIT = False
+
+
+def check_precision(precision: str, H: int) -> None:
+    """ValueError for an unknown precision; RoomSlamError for "bf16" at a hidden size without a tensor-core kernel."""
+    if precision not in PRECISIONS:
+        raise ValueError(f"precision must be one of {PRECISIONS}, got {precision!r}")
+    if precision == "bf16" and H != 128:
+        raise _lib.RoomSlamError(f"precision='bf16': the tensor-core LSTM recurrence exists for d_model 256 (hidden size 128) "
+                                 f"only, not d_model {2 * H}; use precision='fp32'")
+
+
+def lstm_pack_bf16(w_hh, w_hh_r, split=None):
+    """(fwd_img, bwd_img): the bf16 weight images rs_lstm_fwd_bf16 / rs_lstm_bwd_bf16 read (layouts in roomslam_b200.h),
+    built from W_hh of both directions in one launch.  split None: LSTM_BF16_SPLIT."""
+    split = LSTM_BF16_SPLIT if split is None else split
+    w_hh, w_hh_r = w_hh.contiguous().float(), w_hh_r.contiguous().float()
+    H = w_hh.shape[1]
+    n = 2 * (1 + int(split)) * 4 * H * H
+    fwd = torch.empty(n, dtype=torch.bfloat16, device=w_hh.device)
+    bwd = torch.empty(n, dtype=torch.bfloat16, device=w_hh.device)
+    _lib.call("rs_lstm_pack_weights_bf16", _p(w_hh), _p(w_hh_r), H, int(split), _p(fwd), _p(bwd), _stream(w_hh))
+    return fwd, bwd
+
+
+def lstm_layer_fwd(xin, mask, weights, need_grad=True, precision="fp32", images=None, split=None):
     """Forward of ONE bidirectional LSTM layer (the body of LSTMLayerFn.forward).
 
     xin (B, T+2, I) padded; mask (B, T, I) inter-layer dropout multiplier or None; weights = (w_ih, w_hh, b_ih, b_hh,
     w_ih_r, w_hh_r, b_ih_r, b_hh_r).  Returns (out (B, T+2, 2H) padded with zero pad rows, saved [2][B][T][5][H] (i, f,
     g, o, c; None unless need_grad), xin_saved, w_ih_cat [8H, I], w_hh_cat [2][4H][H], tc): xin_saved is the masked input
-    the projection read, as its bf16x6 split when tc (the tensor-core path) is taken."""
+    the projection read, as its bf16x6 split when tc (the tensor-core path) is taken.
+    precision "bf16" (H = 128 only) runs the recurrence on rs_lstm_fwd_bf16 with the weight images `images` (packed here
+    with `split` when None; split None: LSTM_BF16_SPLIT); everything else is the same."""
     w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r = weights
+    check_precision(precision, w_hh.shape[1])
     xin = xin.contiguous().float()
     B, Tp, I = xin.shape
     T, H = Tp - 2, w_hh.shape[1]
@@ -108,7 +139,7 @@ def lstm_layer_fwd(xin, mask, weights, need_grad=True):
         xin = xm
     w_ih_cat = torch.cat([w_ih, w_ih_r], 0).contiguous().float()              # [8H, I]
     w_hh_cat = torch.stack([w_hh, w_hh_r], 0).contiguous().float()            # [2, 4H, H]
-    w_hh_t = w_hh_cat.transpose(1, 2).contiguous()                            # [2, H, 4H]
+    w_hh_t = w_hh_cat.transpose(1, 2).contiguous() if precision == "fp32" else None   # [2, H, 4H]
     bias = (torch.cat([b_ih, b_ih_r], 0) + torch.cat([b_hh, b_hh_r], 0)).contiguous().float()
     P = torch.empty(B, Tp, 8 * H, device=dev)
     tc = _tc_ok(B * Tp, I, 2 * H)
@@ -121,19 +152,37 @@ def lstm_layer_fwd(xin, mask, weights, need_grad=True):
             linear_nt(xin.view(B * Tp, I), w_ih_cat, bias, P.view(B * Tp, 8 * H))
     out = padded(B, T, 2 * H, dev)
     saved = torch.empty(2, B, T, 5, H, device=dev) if need_grad else None
-    with ktime("lstm_fwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
-        _lib.call("rs_lstm_fwd_f32", _p(P), 8 * H, Tp, 1, _p(w_hh_cat), _p(w_hh_t), _p(out), 2 * H, Tp, 1, _p(saved), B, T, H, st)
+    if precision == "bf16":
+        split = LSTM_BF16_SPLIT if split is None else split
+        if images is None:
+            images = lstm_pack_bf16(w_hh_cat[0], w_hh_cat[1], split)
+        with ktime("lstm_fwd_bf16_kernel", 2.0 * B * T * 2 * 4 * H * H):
+            _lib.call("rs_lstm_fwd_bf16", _p(P), 8 * H, Tp, 1, _p(images[0]), _p(out), 2 * H, Tp, 1, _p(saved), B, T, H, int(split), st)
+    else:
+        with ktime("lstm_fwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
+            _lib.call("rs_lstm_fwd_f32", _p(P), 8 * H, Tp, 1, _p(w_hh_cat), _p(w_hh_t), _p(out), 2 * H, Tp, 1, _p(saved), B, T, H, st)
     del P
     return out, saved, (xin3 if tc else xin), w_ih_cat, w_hh_cat, tc
 
 
-def lstm_bptt(d_out, saved, w_hh_cat):
+def lstm_bptt(d_out, saved, w_hh_cat, precision="fp32", w_img=None, split=None):
     """Backward through time of one layer: d_out (B, T+2, 2H) padded -> dG (B, T+2, 8H) padded (pad rows zero), the
-    gradient w.r.t. the gate pre-activations, columns [forward i | f | g | o, reverse i | f | g | o]."""
+    gradient w.r.t. the gate pre-activations, columns [forward i | f | g | o, reverse i | f | g | o].  precision "bf16":
+    rs_lstm_bwd_bf16 with the backward weight image w_img (packed from w_hh_cat with `split` when None; split None:
+    LSTM_BF16_SPLIT)."""
     _, B, T, _, H = saved.shape
+    check_precision(precision, H)
     Tp = T + 2
     d_out = d_out.contiguous().float()
     dG = padded(B, T, 8 * H, d_out.device)
+    if precision == "bf16":
+        split = LSTM_BF16_SPLIT if split is None else split
+        if w_img is None:
+            w_img = lstm_pack_bf16(w_hh_cat[0], w_hh_cat[1], split)[1]
+        with ktime("lstm_bwd_bf16_kernel", 2.0 * B * T * 2 * 4 * H * H):
+            _lib.call("rs_lstm_bwd_bf16", _p(d_out), 2 * H, Tp, 1, _p(saved), _p(w_img), _p(dG), 8 * H, Tp, 1, B, T, H, int(split),
+                      _stream(d_out))
+        return dG
     with ktime("lstm_bwd_f32_kernel", 2.0 * B * T * 2 * 4 * H * H):
         _lib.call("rs_lstm_bwd_f32", _p(d_out), 2 * H, Tp, 1, _p(saved), _p(w_hh_cat), _p(dG), 8 * H, Tp, 1, B, T, H, _stream(d_out))
     return dG
@@ -186,17 +235,25 @@ def lstm_grads_from_dG(dG, out, xin_saved, w_ih_cat, mask, tc, need_dx=True):
 class LSTMLayerFn(torch.autograd.Function):
     """ONE bidirectional LSTM layer over the padded activation layout.
 
-    apply(xin (B, T+2, I) padded, mask (B, T, I) or None, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r)
-        -> out (B, T+2, 2H) padded (pad rows zero).  Replaces one layer of torch.nn.LSTM (model.py:16-23)."""
+    apply(xin (B, T+2, I) padded, mask (B, T, I) or None, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r
+          [, precision "fp32" | "bf16"])
+        -> out (B, T+2, 2H) padded (pad rows zero).  Replaces one layer of torch.nn.LSTM (model.py:16-23).  With "bf16" the
+    weight images are packed once per forward and kept for the backward pass."""
 
     @staticmethod
     @_lib.on_tensor_device
-    def forward(ctx, xin, mask, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r):
+    def forward(ctx, xin, mask, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r, precision="fp32"):
         _need_cuda(xin, mask, w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r)
+        check_precision(precision, w_hh.shape[1])
+        split = LSTM_BF16_SPLIT
+        images = lstm_pack_bf16(w_hh, w_hh_r, split) if precision == "bf16" else None
         out, saved, xin_saved, w_ih_cat, w_hh_cat, tc = lstm_layer_fwd(
-            xin, mask, (w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r), need_grad=any(ctx.needs_input_grad))
+            xin, mask, (w_ih, w_hh, b_ih, b_hh, w_ih_r, w_hh_r, b_ih_r, b_hh_r), need_grad=any(ctx.needs_input_grad),
+            precision=precision, images=images, split=split)
+        ctx.split = split
         ctx.mask = mask
         ctx.tc = tc
+        ctx.precision, ctx.w_img = precision, (images[1] if images is not None else None)
         ctx.save_for_backward(out, saved, xin_saved, w_ih_cat, w_hh_cat)
         return out
 
@@ -206,10 +263,10 @@ class LSTMLayerFn(torch.autograd.Function):
         out, saved, xin_saved, w_ih_cat, w_hh_cat = ctx.saved_tensors
         if saved is None:
             raise RuntimeError("LSTMLayerFn: forward ran without saving activations (nothing required grad)")
-        dG = lstm_bptt(d_out, saved, w_hh_cat)
+        dG = lstm_bptt(d_out, saved, w_hh_cat, ctx.precision, ctx.w_img, ctx.split)
         dW_ih, dW_hh, db, d_xin = lstm_grads_from_dG(dG, out, xin_saved, w_ih_cat, ctx.mask, ctx.tc, ctx.needs_input_grad[0])
         H = w_hh_cat.shape[2]
-        return (d_xin, None, dW_ih[:4 * H], dW_hh[0], db[:4 * H], db[:4 * H], dW_ih[4 * H:], dW_hh[1], db[4 * H:], db[4 * H:])
+        return (d_xin, None, dW_ih[:4 * H], dW_hh[0], db[:4 * H], db[:4 * H], dW_ih[4 * H:], dW_hh[1], db[4 * H:], db[4 * H:], None)
 
 
 def _splits(B: int, N: int, Q: int) -> int:
@@ -309,12 +366,15 @@ def _seq2(seq: nn.Sequential, x):
 
 
 class LSTMTraceEncoder(nn.Module):
-    """src/benchmark/model.py:6-57.  forward -> (memory padded (B, N+2, D), mean (B,3), rms (B,), count (B,))."""
+    """src/benchmark/model.py:6-57.  forward -> (memory padded (B, N+2, D), mean (B,3), rms (B,), count (B,)).
+    precision "bf16" runs the LSTM recurrence on the tensor core (d_model 256 only); the parameters are the same."""
 
-    def __init__(self, input_dim: int = 11, d_model: int = 128, num_layers: int = 2, dropout: float = 0.1):
+    def __init__(self, input_dim: int = 11, d_model: int = 128, num_layers: int = 2, dropout: float = 0.1, precision: str = "fp32"):
         super().__init__()
         if (d_model // 2) % 32 != 0 or d_model > 256:
             raise ValueError("d_model must be a multiple of 64, at most 256 (LSTM hidden size = d_model / 2 is a multiple of 32)")
+        check_precision(precision, d_model // 2)
+        self.precision = precision
         self.input_proj = nn.Linear(input_dim, d_model)
         self.lstm = nn.LSTM(input_size=d_model, hidden_size=d_model // 2, num_layers=num_layers,
                             dropout=dropout if num_layers > 1 else 0.0, batch_first=True, bidirectional=True)
@@ -336,7 +396,7 @@ class LSTMTraceEncoder(nn.Module):
                     keep = 1.0 - self.dropout
                     m = torch.bernoulli(torch.full((B, N, self.d_model), keep, device=traces.device)) / keep
             w = [getattr(self.lstm, f"{n}_l{l}{sfx}") for sfx in ("", "_reverse") for n in ("weight_ih", "weight_hh", "bias_ih", "bias_hh")]
-            cur = LSTMLayerFn.apply(cur, m, *w)
+            cur = LSTMLayerFn.apply(cur, m, *w, self.precision)
         memory = linear(cur, self.out_proj.weight, self.out_proj.bias, allow_tc=True)          # pad rows hold the bias; never read as tokens
         return memory, mean, rms, count
 
@@ -375,11 +435,12 @@ class SimpleQueryDecoder(nn.Module):
 
 
 class TraceToColliderLSTM(nn.Module):
-    """src/benchmark/model.py:140-153.  ``forward(traces [B,N,11], mask [B,N] bool or None)``."""
+    """src/benchmark/model.py:140-153.  ``forward(traces [B,N,11], mask [B,N] bool or None)``.  precision: "fp32" (default)
+    or "bf16" (tensor-core LSTM recurrence, d_model 256 only); state_dicts interchange between the two."""
 
-    def __init__(self, d_model: int = 128, num_queries: int = 30, lstm_layers: int = 2, dropout: float = 0.1):
+    def __init__(self, d_model: int = 128, num_queries: int = 30, lstm_layers: int = 2, dropout: float = 0.1, precision: str = "fp32"):
         super().__init__()
-        self.encoder = LSTMTraceEncoder(11, d_model, lstm_layers, dropout)
+        self.encoder = LSTMTraceEncoder(11, d_model, lstm_layers, dropout, precision)
         self.decoder = SimpleQueryDecoder(d_model, num_queries)
 
     def forward(self, traces: torch.Tensor, mask: Optional[torch.Tensor] = None, dropout_mask=None) -> Dict[str, torch.Tensor]:
@@ -395,8 +456,9 @@ class TraceToColliderLSTM(nn.Module):
 
 
 def build_model(num_queries: int = 80, d_model: int = 256, model_type: str = "lstm", lstm_layers: int = 2,
-                dropout: float = 0.1, **unused):
-    """Signature of src/benchmark/model.py:406-443; only the 'lstm' variant is on this library's path."""
+                dropout: float = 0.1, precision: str = "fp32", **unused):
+    """Signature of src/benchmark/model.py:406-443; only the 'lstm' variant is on this library's path.  precision "bf16"
+    (d_model 256) runs the LSTM recurrence on the tensor core."""
     if model_type.lower() != "lstm":
         raise ValueError("roomslam_b200.build_model implements model_type='lstm' only (the transformer variant is out of scope)")
-    return TraceToColliderLSTM(d_model=d_model, num_queries=num_queries, lstm_layers=lstm_layers, dropout=dropout)
+    return TraceToColliderLSTM(d_model=d_model, num_queries=num_queries, lstm_layers=lstm_layers, dropout=dropout, precision=precision)

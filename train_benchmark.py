@@ -4,6 +4,11 @@ collider files in, BiLSTM + query decoder trained with the Hungarian set loss, e
 upstream layout (model_state_dict / optimizer_state_dict / val_loss / metrics / config).
 
     python train_benchmark.py --data_dir dataset/train --val_dir dataset/val --epochs 200
+    python train_benchmark.py --d_model 256 --num_queries 80 --precision bf16     # build_model's defaults, tensor cores
+
+--precision bf16 runs the LSTM recurrence on tensor cores (bf16 operands, fp32 accumulation and cell state); it exists for
+--d_model 256 only and is about 6x faster per training step there (DESIGN.md section 7.2).  fp32 is the default and the
+exact path.  The precision is recorded in config.json; checkpoints load into either precision.
 
 Everything between the JSON files and the optimizer runs on the GPU: features (rs_trace_features), model, matching,
 loss, metrics.  The JSON parsing and the upstream augmentation pipeline (dataloader.py:340-392) are host-side and out of
@@ -52,6 +57,8 @@ def main():
     ap.add_argument("--lr", type=float, default=2e-4)
     ap.add_argument("--weight_decay", type=float, default=1e-4)
     ap.add_argument("--d_model", type=int, default=128)
+    ap.add_argument("--precision", choices=("fp32", "bf16"), default="fp32",
+                    help="LSTM recurrence: fp32, or bf16 on tensor cores (d_model 256 only)")
     ap.add_argument("--num_queries", type=int, default=30)
     ap.add_argument("--max_trace_len", type=int, default=3000)
     ap.add_argument("--iou_thresh", type=float, default=0.5)
@@ -68,7 +75,7 @@ def main():
     gen = torch.Generator().manual_seed(args.seed)
     train_pts, train_tgt = load_split(args.data_dir)
     val_pts, val_tgt = load_split(args.val_dir)
-    model = build_model(num_queries=args.num_queries, d_model=args.d_model, model_type="lstm").cuda()
+    model = build_model(num_queries=args.num_queries, d_model=args.d_model, model_type="lstm", precision=args.precision).cuda()
     criterion = SetCriterion(WEIGHTS)
     optimizer = torch.optim.AdamW(model.parameters(), lr=args.lr, weight_decay=args.weight_decay)
     scheduler = torch.optim.lr_scheduler.ReduceLROnPlateau(optimizer, mode="min", factor=0.5, patience=5, threshold=1e-3,
