@@ -187,8 +187,9 @@ int rs_gru_pack_weights_bf16(const float* const* w, int H, int I, int split, voi
  * [2][32][384][8] and Whh [2][18][384][8] whose chunk 16 holds only the bias (rs_gru_pack_weights_bf16 with wih_img) --
  * P and the projection GEMM are then not needed at all.  The r and z rows of all
  * weights / biases carry the factor 1/2 of sigma(a) = tanh(a/2)/2 + 1/2.  b_hn [2][H], out tile-major (2H columns,
- * zero pad rows), gates [tiles][T][2][48][128][8] fp16 = r | z | n (NULL for inference; W_hn h + b_hn is NOT saved, the
- * backward kernel recomputes it), h_n [2][B][H] fp32. */
+ * zero pad rows), gates [tiles][T][2][48][128][8] fp16 = r | z | n (NULL for inference, and for a layer 0 whose backward
+ * recomputes them: rs_rec_bwd_bf16_recompute; W_hn h + b_hn is NOT saved, the backward kernel recomputes it), h_n [2][B][H]
+ * fp32. */
 int rs_rec_fwd_bf16(const float* x, int I, const void* P, int64_t p_cols, const void* X, const void* Wih, const void* Whh,
                     const float* b_hn, void* out,
                     void* gates, float* h_n, const int* lengths, const void* drop_bits, const float* drop_scale,
@@ -201,6 +202,14 @@ int rs_pack_x_tm(const float* x, int B, int T, int I, void* out, void* stream);
 int rs_rec_bwd_bf16(const void* d_out, const float* d_h_n, const void* gates, const void* out, const void* WhhT,
                     const void* Whh, int whh_chunks, const float* b_hn, void* dG, const int* lengths, const void* drop_bits,
                     const float* drop_scale, int split, int B, int T, void* stream);
+/* rs_rec_bwd_bf16 for layer 0 with unsplit weights and 1 <= I <= 2 inputs, WITHOUT saved gates: the forward ran with
+ * gates = NULL, and the kernel recomputes r, z and n by replaying the forward's MMA on the tensor core (same operands, shapes
+ * and K order) and its gate math; dG is bit-identical to rs_rec_bwd_bf16's from the saved gates.  x (B, T, I) fp32 is the
+ * layer input the forward took, xpack a [tiles][T][128][8] bf16 workspace (its packed input chunks, written here), Whh the
+ * forward image with its 18 chunks per direction; the other arguments as for rs_rec_bwd_bf16. */
+int rs_rec_bwd_bf16_recompute(const void* d_out, const float* d_h_n, const float* x, int I, void* xpack, const void* out,
+                              const void* WhhT, const void* Whh, int whh_chunks, const float* b_hn, void* dG, const int* lengths,
+                              const void* drop_bits, const float* drop_scale, int B, int T, void* stream);
 /* The same two kernels for hidden_size = 256 (BASELINE config 4: H 256, T 4000), where W_hh no longer fits in shared memory:
  * each CTA of the pair streams its half of the weights from L2 through a ring of bulk copies once per time step
  * (csrc/rec_wide.cu).  Tile-major operands as above with H = 256 (P 6H, out 2H, dG 8H columns; gates

@@ -79,8 +79,23 @@ extern "C" int rs_rec_bwd_bf16(const void* d_out, const float* d_h_n, const void
     RS_REQUIRE(gates && out && WhhT && Whh && b_hn && dG && B >= 0 && T >= 0, "rs_rec_bwd_bf16: bad arguments");
     RS_REQUIRE(whh_chunks >= 16 * (split ? 2 : 1), "rs_rec_bwd_bf16: Whh is the forward image (16 hidden chunks, twice with split)");
     RS_REQUIRE(!drop_bits || drop_scale, "rs_rec_bwd_bf16: drop_bits needs drop_scale");
-    return rs::rec_bwd_pair(d_out, d_h_n, gates, out, WhhT, Whh, whh_chunks, b_hn, dG, lengths, drop_bits, drop_scale, split, B, T,
-                            PF_DIST_BWD, stream);
+    return rs::rec_bwd_pair(d_out, d_h_n, gates, nullptr, 0, nullptr, out, WhhT, Whh, whh_chunks, b_hn, dG, lengths, drop_bits,
+                            drop_scale, split, B, T, PF_DIST_BWD, stream);
+}
+
+extern "C" int rs_rec_bwd_bf16_recompute(const void* d_out, const float* d_h_n, const float* x, int I, void* xpack, const void* out,
+                                         const void* WhhT, const void* Whh, int whh_chunks, const float* b_hn, void* dG,
+                                         const int* lengths, const void* drop_bits, const float* drop_scale, int B, int T,
+                                         void* stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    if (rs::check_device_sm100()) return 3;
+    if (B == 0 || T == 0) return 0;        // nothing to do: empty tensors carry null pointers
+    RS_REQUIRE(x && xpack && out && WhhT && Whh && b_hn && dG && B >= 0 && T >= 0, "rs_rec_bwd_bf16_recompute: bad arguments");
+    RS_REQUIRE(I >= 1 && I <= 2, "rs_rec_bwd_bf16_recompute: layer 0 with 1 or 2 input columns only (got %d)", I);
+    RS_REQUIRE(whh_chunks == 16 + 2, "rs_rec_bwd_bf16_recompute: Whh is the unsplit layer-0 forward image (18 chunks, got %d)", whh_chunks);
+    RS_REQUIRE(!drop_bits || drop_scale, "rs_rec_bwd_bf16_recompute: drop_bits needs drop_scale");
+    return rs::rec_bwd_pair(d_out, d_h_n, nullptr, x, I, xpack, out, WhhT, Whh, whh_chunks, b_hn, dG, lengths, drop_bits, drop_scale,
+                            0, B, T, PF_DIST_BWD, stream);
 }
 
 extern "C" int rs_pack_x_tm(const float* x, int B, int T, int I, void* out, void* stream_) {

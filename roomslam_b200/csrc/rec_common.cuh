@@ -32,6 +32,7 @@ __device__ __forceinline__ uint32_t f2_to_h2(float a, float b) {
     __half2 h = __floats2half2_rn(a, b);
     return *reinterpret_cast<uint32_t*>(&h);
 }
+__device__ __forceinline__ float round_h(float a) { return __half2float(__float2half_rn(a)); }   // a saved gate's value
 __device__ __forceinline__ uint4 pack8h(const float* f) {
     return make_uint4(f2_to_h2(f[0], f[1]), f2_to_h2(f[2], f[3]), f2_to_h2(f[4], f[5]), f2_to_h2(f[6], f[7]));
 }
@@ -117,9 +118,10 @@ int rec_fwd_nt(int B);                      // tiles in flight per pair of the f
 int rec_fwd_pair(const float* x, int I, const void* P, const void* X, const void* Wih, const void* Whh, const float* b_hn, void* out,
                  void* gates, float* h_n, const int* lengths, const void* drop_bits, const float* drop_scale, void* out_drop, int split,
                  int B, int T, int nt, int pf_dist, cudaStream_t stream);
-int rec_bwd_pair(const void* d_out, const float* d_h_n, const void* gates, const void* out, const void* WhhT, const void* Whh,
-                 int whh_chunks, const float* b_hn, void* dG, const int* lengths, const void* drop_bits, const float* drop_scale,
-                 int split, int B, int T, int pf_dist, cudaStream_t stream);
+// x != NULL: layer 0 (I <= 2, unsplit, gates NULL) recomputes r, z, n; xpack is its [tiles][T][128][8] bf16 workspace
+int rec_bwd_pair(const void* d_out, const float* d_h_n, const void* gates, const float* x, int I, void* xpack, const void* out,
+                 const void* WhhT, const void* Whh, int whh_chunks, const float* b_hn, void* dG, const int* lengths,
+                 const void* drop_bits, const float* drop_scale, int split, int B, int T, int pf_dist, cudaStream_t stream);
 #endif
 
 }  // namespace rs

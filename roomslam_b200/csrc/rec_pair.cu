@@ -506,10 +506,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
 // hn = h_{t-1} . W_hn^T (N = 128, K = 128) into one of two 64-column TMEM buffers as soon as both CTAs' tiles landed, and
 // the epilogue reads hn from TMEM and h_{t-1} from shared memory.  Same bf16 operands and K order as the forward MMA: the
 // recomputed value is the forward's fp32 accumulator, not its fp16 rounding.
+//
+// kRecompute (layer 0, unsplit weights, I <= 2): r, z and n are not saved by the forward pass either (6.3 GB written and
+// 6.3 GB read per step at the benchmark shape).  The even CTA's warp 1 replays the forward's whole layer-0 MMA -- the same
+// A bytes (the h_{t-1} tile, which is what the forward's A tile held, plus the packed input chunk of step t, bulk-copied
+// next to it), the same B image (the r | z | n rows of whh_img with its input chunk), the same instruction shapes and the
+// same K order -- into one of two 256-column TMEM buffers (r | z | hn | the input part of n), and the epilogue forms r, z
+// and n exactly as the forward epilogue does: the gate gradients are bit-identical to those from saved gates.  TMEM holds
+// two such buffers and nothing else (512 columns), so the z (.) dh carry lives in the r columns of the buffer of the step
+// that wrote it: the epilogue of step s reads r there, writes the carry over it, the dh MMA of step s + 1 accumulates onto
+// it, the epilogue of step s + 1 reads dh from it first and then hands the buffer to the recompute of step s + 2, which runs
+// under the rest of that epilogue.
 struct BwdPairParams {
     const uint8_t* d_out; long long dout_block_bytes;
     const float* d_h_n;
-    const uint8_t* gates;                                // [tiles][T][2][48 chunks: r | z | n][128][8] fp16
+    const uint8_t* gates;                                // [tiles][T][2][48 chunks: r | z | n][128][8] fp16 (NULL: kRecompute)
+    const uint8_t* xpack;                                // kRecompute: [tiles][T][128][8] bf16, pack_x of each trace row and step
     const uint8_t* out; long long out_block_bytes;
     const uint8_t* WhhT;                                 // [2][48 (x2 split)][128][8] bf16
     const uint8_t* Whh;                                  // forward image [2][16 (x2 split) (+2)][384][8]: its n rows are W_hn
@@ -525,24 +537,29 @@ struct BwdPairParams {
 };
 
 constexpr int HP_BYTES = 16 * CHUNK_S;                   // 16 KB: the h_{t-1} tile of this CTA's 64 rows (K-major A operand)
-template <bool kVarLen, bool kDrop>
+constexpr int WF_BYTES = 18 * W_CHUNK;                   // kRecompute: 54 KB, r | z | n rows of whh_img (16 hidden + 2 input chunks)
+template <bool kVarLen, bool kDrop, bool kRecompute>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_bwd_pair_kernel(const BwdPairParams p) {
     extern __shared__ __align__(1024) uint8_t smem[];
+    constexpr int STAGE = kRecompute ? HP_BYTES + 2 * CHUNK_S : HP_BYTES;   // + the input chunk of step t and a zero chunk
+    constexpr uint32_t TMEM_COLS = kRecompute ? 512 : 256;
     const int w_chunks = 48 * (1 + p.split), n_hid = 16 * (1 + p.split);
     uint8_t* w_s = smem;                                   // [48 chunks][64 rows = hidden units of this CTA][16 B]   W_hh^T
     uint8_t* a_s = w_s + w_chunks * CHUNK_S;               // [48 chunks][64 rows][16 B]  dGh_t
     uint8_t* wn_s = a_s + A_BWD_BYTES;                     // [16 chunks][64 rows = hidden units of this CTA][16 B]   W_hn
-    uint8_t* hp_s = wn_s + n_hid * CHUNK_S;                // [2 stages][16 chunks][64 rows][16 B]  h_{t-1}
-    float* bhn_s = reinterpret_cast<float*>(hp_s + 2 * HP_BYTES);
+                                                           // kRecompute: [18 chunks][192 rows][16 B] as the forward's w_s
+    uint8_t* hp_s = wn_s + (kRecompute ? WF_BYTES : n_hid * CHUNK_S);   // [2 stages][16 (+2) chunks][64 rows][16 B]  h_{t-1} (| x_t)
+    float* bhn_s = reinterpret_cast<float*>(hp_s + 2 * STAGE);
     uint64_t* bars = reinterpret_cast<uint64_t*>(bhn_s + H);
     uint64_t* w_full = bars;
     uint64_t* a_ready = bars + 1;               // even CTA: dGh_t of both CTAs written (32 warps)
     uint64_t* acc_full = bars + 2;              // both: the dh MMA chain retired (multicast commit)
     uint64_t* hp_full = bars + 3;               // [2] this CTA's h_{t-1} tile landed (bulk-copy bytes)
     uint64_t* hp_rdy = bars + 5;                // [2] even CTA: both CTAs' tiles landed (2 arrivals)
-    uint64_t* hn_full = bars + 7;               // [2] both: the hn MMA retired (multicast commit)
+    uint64_t* hn_full = bars + 7;               // [2] both: the hn MMA (kRecompute: the gate MMAs) retired (multicast commit)
     uint64_t* hp_free = bars + 9;               // [2] this CTA's 16 epilogue warps are done with the stage (tile and TMEM buffer)
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 11);
+    uint64_t* tm_free = bars + 11;              // [2] kRecompute, even CTA: both CTAs' epilogues have read dh out of the buffer
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 13);
 
     constexpr int UPT = 16, NGRP = 2;
     const uint32_t rank = cluster_ctarank();
@@ -555,21 +572,37 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
         mbar_init(w_full, 1);
         mbar_init(a_ready, 2 * 16);
         mbar_init(acc_full, 1);
-        for (int i = 0; i < 2; ++i) { mbar_init(&hp_full[i], 1); mbar_init(&hp_rdy[i], 2); mbar_init(&hn_full[i], 1); mbar_init(&hp_free[i], 16); }
+        for (int i = 0; i < 2; ++i) {
+            mbar_init(&hp_full[i], 1); mbar_init(&hp_rdy[i], 2); mbar_init(&hn_full[i], 1); mbar_init(&hp_free[i], 16);
+            mbar_init(&tm_free[i], 2 * 16);
+        }
         fence_mbar_init();
     }
     if (warp == 0) {
-        tmem_alloc_pair<256>(tmem_slot);        // dh accumulator [0, 64), hn buffers [64, 128) and [128, 192)
+        // dh accumulator [0, 64), hn buffers [64, 128) and [128, 192); kRecompute: two gate buffers [0, 256), [256, 512)
+        tmem_alloc_pair<TMEM_COLS>(tmem_slot);
         if (lane == 0) {
-            mbar_expect_tx(w_full, (w_chunks + n_hid) * CHUNK_S);
+            mbar_expect_tx(w_full, w_chunks * CHUNK_S + (kRecompute ? WF_BYTES : n_hid * CHUNK_S));
             const uint8_t* src = p.WhhT + (long long)dir * w_chunks * CHUNK_G + rank * 1024;
             for (int c = 0; c < w_chunks; ++c) bulk_load(w_s + c * CHUNK_S, src + (long long)c * CHUNK_G, 1024, w_full);
-            const uint8_t* srcn = p.Whh + (long long)dir * p.whh_chunks * (384 * 16) + (256 + rank * 64) * 16;
-            for (int c = 0; c < n_hid; ++c) bulk_load(wn_s + c * CHUNK_S, srcn + (long long)c * (384 * 16), 1024, w_full);
+            if (kRecompute) {           // the forward kernel's copy of its W half (rec_fwd_pair_kernel, layer 0, kXC = 1)
+                const uint8_t* srcf = p.Whh + (long long)dir * p.whh_chunks * (384 * 16);
+                for (int c = 0; c < 18; ++c)
+                    for (int g = 0; g < 3; ++g)
+                        bulk_load(wn_s + c * W_CHUNK + g * 1024, srcf + (long long)c * (384 * 16) + (g * 128 + rank * 64) * 16, 1024, w_full);
+            } else {
+                const uint8_t* srcn = p.Whh + (long long)dir * p.whh_chunks * (384 * 16) + (256 + rank * 64) * 16;
+                for (int c = 0; c < n_hid; ++c) bulk_load(wn_s + c * CHUNK_S, srcn + (long long)c * (384 * 16), 1024, w_full);
+            }
         }
         mbar_wait(w_full, 0);
     }
     for (int i = threadIdx.x; i < H; i += blockDim.x) bhn_s[i] = p.b_hn[dir * H + i];
+    if (kRecompute) {                   // the second input chunk of the one input K step stays zero, as in the forward's A tile
+        for (int i = threadIdx.x; i < 2 * CHUNK_S / 16; i += blockDim.x)
+            reinterpret_cast<uint4*>(hp_s + (i / (CHUNK_S / 16)) * STAGE + 17 * CHUNK_S)[i % (CHUNK_S / 16)] = make_uint4(0, 0, 0, 0);
+        fence_proxy_async();
+    }
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();
@@ -592,13 +625,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
             for (int sidx = 0; sidx < T - 1; ++sidx) {     // the result of the last reverse step is unused
                 mbar_wait_cluster(a_ready, sidx & 1);
                 tc_fence_after();
+                const uint32_t d = tmem_base + (kRecompute ? (sidx & 1) * 256 : 0);    // kRecompute: the carry of step sidx
                 if (elect_one()) {
                     for (int part = 0; part <= p.split; ++part) {
 #pragma unroll
                         for (int k = 0; k < 24; ++k) {
                             const uint64_t da = umma_desc_noswz(a_addr + k * 2 * CHUNK_S, CHUNK_S, 128);
                             const uint64_t db = umma_desc_noswz(w_addr + (part * 48 + k * 2) * CHUNK_S, CHUNK_S, 128);
-                            tc_mma_bf16_pair(tmem_base, da, db, idesc, 1u);   // accumulates onto the z (.) dh carry in TMEM
+                            tc_mma_bf16_pair(d, da, db, idesc, 1u);           // accumulates onto the z (.) dh carry in TMEM
                         }
                     }
                     tc_commit_pair(acc_full);
@@ -619,28 +653,49 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                 const int t_prev = dir ? t + 1 : t - 1;
                 if (elect_one()) {
                     if (sidx >= 2) mbar_wait(&hp_free[st], ph ^ 1);    // the epilogue of step sidx - 2 is done with this stage
-                    mbar_expect_tx(&hp_full[st], HP_BYTES);
+                    mbar_expect_tx(&hp_full[st], HP_BYTES + (kRecompute ? CHUNK_S : 0));
                     const uint8_t* src = p.out + ((long long)tile * (T + 2) + t_prev + 1) * p.out_block_bytes + (long long)(dir * 16) * CHUNK_G + rank * 1024;
 #pragma unroll
                     for (int c = 0; c < 16; ++c)                       // 16 pieces of 1 KB, back to back (see the X tile producer)
-                        bulk_load(hp_s + st * HP_BYTES + c * CHUNK_S, src + (long long)c * CHUNK_G, 1024, &hp_full[st]);
+                        bulk_load(hp_s + st * STAGE + c * CHUNK_S, src + (long long)c * CHUNK_G, 1024, &hp_full[st]);
+                    if (kRecompute)                                    // the input chunk of step t: the A tile's chunk 16 in the forward
+                        bulk_load(hp_s + st * STAGE + 16 * CHUNK_S, p.xpack + ((long long)tile * T + t) * CHUNK_G + rank * 1024, 1024, &hp_full[st]);
                     if (p.pf_dist > 0 && sidx + p.pf_dist < T) {       // optional L2 prefetch of a later step's gate / d_out blocks
                         const int t2 = dir ? sidx + p.pf_dist : (T - 1 - sidx - p.pf_dist);
-                        l2_prefetch(p.gates + (((long long)tile * T + t2) * 2 + dir) * (48LL * CHUNK_G) + (long long)(rank * 24) * CHUNK_G, 24 * CHUNK_G);
+                        if (!kRecompute)
+                            l2_prefetch(p.gates + (((long long)tile * T + t2) * 2 + dir) * (48LL * CHUNK_G) + (long long)(rank * 24) * CHUNK_G, 24 * CHUNK_G);
                         if (p.d_out) l2_prefetch(p.d_out + ((long long)tile * (T + 2) + t2 + 1) * p.dout_block_bytes + (long long)(dir * 16 + rank * 8) * CHUNK_G, 8 * CHUNK_G);
                     }
                     mbar_wait(&hp_full[st], ph);
                     mbar_arrive_cluster(rdy_remote[st]);
                     if (rank == 0) {
                         mbar_wait(&hp_rdy[st], ph);
+                        // kRecompute: buffer st last held the carry of step sidx - 2, read as dh by the epilogue of step sidx - 1
+                        if (kRecompute && sidx >= 1) mbar_wait(&tm_free[st], ((sidx - 1) >> 1) & 1);
                         tc_fence_after();
-                        const uint32_t hp_addr = smem_u32(hp_s + st * HP_BYTES);
-                        for (int part = 0; part <= p.split; ++part) {
+                        const uint32_t hp_addr = smem_u32(hp_s + st * STAGE);
+                        if (kRecompute) {       // rec_fwd_pair_kernel's layer-0 MMAs (split = 0, kXC = 1), operand for operand
+                            constexpr uint32_t idesc256 = umma_idesc_bf16(128, 256, 0, 0);
+                            const uint32_t d = tmem_base + st * 256;
 #pragma unroll
                             for (int k = 0; k < 8; ++k) {
                                 const uint64_t da = umma_desc_noswz(hp_addr + k * 2 * CHUNK_S, CHUNK_S, 128);
-                                const uint64_t db = umma_desc_noswz(wn_addr + (part * 16 + k * 2) * CHUNK_S, CHUNK_S, 128);
-                                tc_mma_bf16_pair(tmem_base + 64 + st * 64, da, db, idesc, (k | part) != 0);
+                                const uint32_t wk = wn_addr + k * 2 * W_CHUNK;
+                                tc_mma_bf16_pair(d, da, umma_desc_noswz(wk, W_CHUNK, 128), idesc256, k != 0);             // r | z
+                                tc_mma_bf16_pair(d + 128, da, umma_desc_noswz(wk + 128 * 16, W_CHUNK, 128), idesc, k != 0);   // W_hn h
+                            }
+                            const uint64_t da = umma_desc_noswz(hp_addr + 16 * CHUNK_S, CHUNK_S, 128);
+                            const uint32_t wx = wn_addr + 16 * W_CHUNK;
+                            tc_mma_bf16_pair(d, da, umma_desc_noswz(wx, W_CHUNK, 128), idesc256, 1u);
+                            tc_mma_bf16_pair(d + 192, da, umma_desc_noswz(wx + 128 * 16, W_CHUNK, 128), idesc, 0u);     // W_in x + b_in
+                        } else {
+                            for (int part = 0; part <= p.split; ++part) {
+#pragma unroll
+                                for (int k = 0; k < 8; ++k) {
+                                    const uint64_t da = umma_desc_noswz(hp_addr + k * 2 * CHUNK_S, CHUNK_S, 128);
+                                    const uint64_t db = umma_desc_noswz(wn_addr + (part * 16 + k * 2) * CHUNK_S, CHUNK_S, 128);
+                                    tc_mma_bf16_pair(tmem_base + 64 + st * 64, da, db, idesc, (k | part) != 0);
+                                }
                             }
                         }
                         tc_commit_pair(&hn_full[st]);
@@ -665,7 +720,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
         const uint32_t ar_remote = mapa_cluster(smem_u32(a_ready), 0);
         const int len = (kVarLen && live) ? p.lengths[b] : T;
         const float dscale = kDrop ? __ldg(p.drop_scale) : 1.0f;
-        // the carry z (.) dh lives in the TMEM accumulator; it starts as d_h_n
+        // the carry z (.) dh lives in the TMEM accumulator (kRecompute: the r columns of buffer 1); it starts as d_h_n
 #pragma unroll
         for (int sc = 0; sc < NGRP; ++sc) {
             uint32_t init[8];
@@ -678,12 +733,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                 init[0] = __float_as_uint(v0.x); init[1] = __float_as_uint(v0.y); init[2] = __float_as_uint(v0.z); init[3] = __float_as_uint(v0.w);
                 init[4] = __float_as_uint(v1.x); init[5] = __float_as_uint(v1.y); init[6] = __float_as_uint(v1.z); init[7] = __float_as_uint(v1.w);
             }
-            tmem_st_32x32b_x8(taddr + sc * 8, init);
+            tmem_st_32x32b_x8(taddr + (kRecompute ? 256 : 0) + sc * 8, init);
         }
         tmem_st_wait();
 
-        // r, z, n (fp16) and d_out (bf16) of the thread's two chunks (8 units each): per-thread global loads, requested one chunk
-        // ahead of their use
+        // r, z, n (fp16; not with kRecompute) and d_out (bf16) of the thread's two chunks (8 units each): per-thread global
+        // loads, requested one chunk ahead of their use
         uint4 raw[4];
         uint32_t dbits_next = 0;
         // running pointers of this thread's pieces (one signed stride per time step instead of 64-bit index arithmetic)
@@ -691,7 +746,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
         const long long g_step = (dir ? 2 : -2) * (48LL * CHUNK_G);
         const long long do_step = dir ? p.dout_block_bytes : -p.dout_block_bytes;
         const long long dg_step = dir ? p.dg_block_bytes : -p.dg_block_bytes;
-        const uint8_t* g_ptr = p.gates + (((long long)tile * T + t_first) * 2 + dir) * (48LL * CHUNK_G) + (long long)cb * CHUNK_G + row * 16;
+        const uint8_t* g_ptr = kRecompute ? nullptr : p.gates + (((long long)tile * T + t_first) * 2 + dir) * (48LL * CHUNK_G) + (long long)cb * CHUNK_G + row * 16;
         const uint8_t* do_ptr = p.d_out ? p.d_out + ((long long)tile * (T + 2) + t_first + 1) * p.dout_block_bytes
                                                                    + (long long)(dir * 16 + cb) * CHUNK_G + row * 16 : nullptr;
         const uint8_t* db_next = kDrop ? p.drop_bits + (((long long)tile * T + t_first) * 128 + row) * 32 + dir * 16 + (cb & ~3) : nullptr;
@@ -699,7 +754,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
         uint8_t* dg_cur = p.dG + ((long long)tile * (T + 2) + t_first + 1) * p.dg_block_bytes + (long long)(dir * 64 + cb) * CHUNK_G + row * 16;
         auto load_raw = [&](int sc) {                      // chunk sc of the step g_ptr / do_ptr stand at
 #pragma unroll
-            for (int g = 0; g < 3; ++g) raw[g] = ldg16(g_ptr + (long long)(g * 16 + sc) * CHUNK_G);
+            for (int g = 0; g < 3; ++g) raw[g] = kRecompute ? make_uint4(0, 0, 0, 0) : ldg16(g_ptr + (long long)(g * 16 + sc) * CHUNK_G);
             raw[3] = do_ptr ? ldg16(do_ptr + (long long)sc * CHUNK_G) : make_uint4(0, 0, 0, 0);
         };
         load_raw(0);
@@ -710,7 +765,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
             const bool active = !kVarLen || t < len;
             uint8_t* dgblk = dg_cur;
             dg_cur += dg_step;
-            const uint8_t* hp_row = hp_s + st * HP_BYTES + rl * 16;
+            const uint8_t* hp_row = hp_s + st * STAGE + rl * 16;
             const uint32_t dbits = dbits_next;
             if (kDrop && sidx + 1 < T) {                   // next step's mask word: requested a whole step ahead
                 db_next += db_step;
@@ -719,25 +774,56 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
             mbar_wait(&hn_full[st], (sidx >> 1) & 1);      // W_hn h_{t-1} of this step is in TMEM, the h_{t-1} tile in shared memory
             if (sidx > 0) mbar_wait(acc_full, (sidx - 1) & 1);
             tc_fence_after();
+            uint32_t dh16[16];
+            if (kRecompute) {                              // dh out of the other buffer first, then that buffer is free
+                tmem_ld_32x32b_x16(taddr + (st ^ 1) * 256, dh16);
+                tmem_ld_wait();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_cluster(mapa_cluster(smem_u32(&tm_free[st ^ 1]), 0));
+            }
 #pragma unroll
             for (int sc = 0; sc < NGRP; ++sc) {
-                uint32_t acc[8], ahn[8];
-                tmem_ld_32x32b_x8(taddr + sc * 8, acc);
-                tmem_ld_32x32b_x8(taddr + 64 + st * 64 + sc * 8, ahn);
+                uint32_t acc[8], ahn[8], ar[8], az[8], ax[8];
+                if (kRecompute) {
+                    const uint32_t tb = taddr + st * 256 + sc * 8;
+                    tmem_ld_32x32b_x8(tb, ar);
+                    tmem_ld_32x32b_x8(tb + 128, ahn);
+                    tmem_ld_32x32b_x8(tb + 192, ax);
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) acc[j] = dh16[sc * 8 + j];
+                } else {
+                    tmem_ld_32x32b_x8(taddr + sc * 8, acc);
+                    tmem_ld_32x32b_x8(taddr + 64 + st * 64 + sc * 8, ahn);
+                }
                 uint4 cur[4];
 #pragma unroll
                 for (int i = 0; i < 4; ++i) cur[i] = raw[i];
                 if (sc < NGRP - 1) load_raw(sc + 1);
                 float r[8], z[8], n[8], hp[8], dout[8], bh[8];
-                unpack8h(cur[0], r); unpack8h(cur[1], z); unpack8h(cur[2], n);
+                if (!kRecompute) { unpack8h(cur[0], r); unpack8h(cur[1], z); unpack8h(cur[2], n); }
                 unpack8(cur[3], dout);
-                unpack8(*reinterpret_cast<const uint4*>(hp_row + (cb + sc) * CHUNK_S), hp);
-                {
+                auto load_hp_bh = [&]() {
+                    unpack8(*reinterpret_cast<const uint4*>(hp_row + (cb + sc) * CHUNK_S), hp);
                     const float4 b0 = *reinterpret_cast<const float4*>(bhn_s + ub + sc * 8);
                     const float4 b1 = *reinterpret_cast<const float4*>(bhn_s + ub + sc * 8 + 4);
                     bh[0] = b0.x; bh[1] = b0.y; bh[2] = b0.z; bh[3] = b0.w; bh[4] = b1.x; bh[5] = b1.y; bh[6] = b1.z; bh[7] = b1.w;
-                }
+                };
+                if (!kRecompute) load_hp_bh();
                 tmem_ld_wait();
+                if (kRecompute) {               // rec_fwd_pair_kernel's gate math, then the fp16 rounding of the saved gates
+                    tmem_ld_32x32b_x8(taddr + st * 256 + sc * 8 + 64, az);     // (z after r and n: 8 registers fewer at the peak)
+                    load_hp_bh();
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {
+                        const float rf = fmaf(0.5f, tanh_fast(__uint_as_float(ar[j])), 0.5f);
+                        const float nf = tanh_fast(fmaf(rf, __uint_as_float(ahn[j]) + bh[j], __uint_as_float(ax[j])));
+                        r[j] = round_h(rf); n[j] = round_h(nf);
+                    }
+                    tmem_ld_wait();
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) z[j] = round_h(active ? fmaf(0.5f, tanh_fast(__uint_as_float(az[j])), 0.5f) : 1.0f);
+                }
                 float gr[8], gz[8], gn[8], ghn[8];
                 uint32_t carry[8];
 #pragma unroll
@@ -752,6 +838,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                     ghn[j] = gn[j] * r[j];
                     gr[j] = ghn[j] * (hn * (1.0f - r[j]));
                     carry[j] = __float_as_uint(dh * z[j]);
+                    // past a trace's end (z = 1) every gate gradient is zero; written as +0: the r and n a forward step past
+                    // the end saw are not those of the recorded h_{t-1}, and only the sign of that zero could tell them apart
+                    if (kVarLen && !active) gr[j] = gz[j] = gn[j] = ghn[j] = 0.0f;
                 }
                 const uint4 vr = pack8(gr), vz = pack8(gz), vn = pack8(gn), vh = pack8(ghn);
                 // A operand of the dh matvec: K order r | z | hn
@@ -762,7 +851,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
                 stg16(dgblk + (long long)(1 * 16 + sc) * CHUNK_G, vz);
                 stg16(dgblk + (long long)(2 * 16 + sc) * CHUNK_G, vn);
                 stg16(dgblk + (long long)(3 * 16 + sc) * CHUNK_G, vh);
-                tmem_st_32x32b_x8(taddr + sc * 8, carry);
+                tmem_st_32x32b_x8(taddr + (kRecompute ? st * 256 : 0) + sc * 8, carry);   // kRecompute: over r, read above
             }
             tmem_st_wait();
             fence_proxy_async();
@@ -776,7 +865,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
             // step), so the next step's first chunk is requested only AFTER the arrival: it flies under the wait for the dh MMA.
             // (Deferring the last chunk's four stores the same way, which pays in the forward kernel, costs 17 % here.)
             if (sidx + 1 < T) {
-                g_ptr += g_step;
+                if (!kRecompute) g_ptr += g_step;
                 if (do_ptr) do_ptr += do_step;
                 load_raw(0);
             }
@@ -785,7 +874,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1) rec_
     tc_fence_before();
     __syncthreads();
     cluster_sync_all();
-    if (warp == 0) tmem_dealloc_pair<256>(tmem_base);
+    if (warp == 0) tmem_dealloc_pair<TMEM_COLS>(tmem_base);
 }
 
 // (B, T, C) fp32 mask (0 or 1/keep) -> one bit per element in the order the recurrence kernels read them,
@@ -839,6 +928,16 @@ __global__ void gen_drop_bits_kernel(uint8_t* __restrict__ bits, long long n_byt
             for (int q = 0; q < 4; ++q) word |= (((h >> (16 * q)) & 0xffffu) < keep_thr16 ? 1u : 0u) << (4 * k + q);
         }
         reinterpret_cast<uint32_t*>(bits)[e] = word;
+    }
+}
+
+// x (B, T, I <= 2) fp32 -> [tiles][T][128 rows][8] bf16: the input chunk the layer-0 forward kernel packs into its A tile, for
+// every trace row and step (pad traces: the bias columns only, as there).  The A operand of the backward's gate recompute.
+__global__ void pack_x_steps_kernel(const float* __restrict__ x, int B, int T, int I, uint4* __restrict__ out, long long n_rows) {
+    for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < n_rows; e += (long long)gridDim.x * blockDim.x) {
+        const long long bt = e >> 7;                   // e = (tile * T + t) * 128 + row
+        const long long b = (bt / T) * 128 + (e & 127);
+        out[e] = pack_x(b < B ? x + (b * T + bt % T) * I : nullptr, I);
     }
 }
 
@@ -923,12 +1022,21 @@ int rec_fwd_pair(const float* x, int I, const void* P, const void* X, const void
     return 0;
 }
 
-int rec_bwd_pair(const void* d_out, const float* d_h_n, const void* gates, const void* out, const void* WhhT, const void* Whh,
-                 int whh_chunks, const float* b_hn, void* dG, const int* lengths, const void* drop_bits, const float* drop_scale,
-                 int split, int B, int T, int pf_dist, cudaStream_t stream) {
+int rec_bwd_pair(const void* d_out, const float* d_h_n, const void* gates, const float* x, int I, void* xpack, const void* out,
+                 const void* WhhT, const void* Whh, int whh_chunks, const float* b_hn, void* dG, const int* lengths,
+                 const void* drop_bits, const float* drop_scale, int split, int B, int T, int pf_dist, cudaStream_t stream) {
+    const bool recompute = x != nullptr;
+    if (recompute) {
+        const long long n_rows = (long long)((B + 127) / 128) * T * 128;
+        long long blocks = (n_rows + 255) / 256;
+        if (blocks > 148 * 16) blocks = 148 * 16;
+        pack_x_steps_kernel<<<(int)blocks, 256, 0, stream>>>(x, B, T, I, static_cast<uint4*>(xpack), n_rows);
+        count_launch();
+        RS_CUDA_OK(cudaGetLastError());
+    }
     BwdPairParams p = {};
     p.d_out = static_cast<const uint8_t*>(d_out); p.dout_block_bytes = 2LL * H * 256;
-    p.d_h_n = d_h_n; p.gates = static_cast<const uint8_t*>(gates);
+    p.d_h_n = d_h_n; p.gates = static_cast<const uint8_t*>(gates); p.xpack = static_cast<const uint8_t*>(xpack);
     p.out = static_cast<const uint8_t*>(out); p.out_block_bytes = 2LL * H * 256;
     p.WhhT = static_cast<const uint8_t*>(WhhT);
     p.Whh = static_cast<const uint8_t*>(Whh); p.whh_chunks = whh_chunks; p.b_hn = b_hn;
@@ -936,16 +1044,22 @@ int rec_bwd_pair(const void* d_out, const float* d_h_n, const void* gates, const
     p.lengths = lengths;
     p.drop_bits = static_cast<const uint8_t*>(drop_bits); p.drop_scale = drop_scale;
     p.B = B; p.T = T; p.n_tiles = (B + 127) / 128; p.split = split ? 1 : 0; p.pf_dist = pf_dist;
-    const int smem = (1 + p.split) * (W_BWD_BYTES + 16 * CHUNK_S) + A_BWD_BYTES + 2 * HP_BYTES + H * 4 + 256;
+    const int smem = recompute ? W_BWD_BYTES + A_BWD_BYTES + WF_BYTES + 2 * (HP_BYTES + 2 * CHUNK_S) + H * 4 + 256
+                               : (1 + p.split) * (W_BWD_BYTES + 16 * CHUNK_S) + A_BWD_BYTES + 2 * HP_BYTES + H * 4 + 256;
     const dim3 grid(2 * p.n_tiles, 2);
+#define RS_LAUNCH_BWD_R(VL_, DROP_, RC_)                                                                                \
+    do {                                                                                                                \
+        RS_CUDA_OK(cudaFuncSetAttribute(rec_bwd_pair_kernel<VL_, DROP_, RC_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
+        rec_bwd_pair_kernel<VL_, DROP_, RC_><<<grid, NUM_THREADS, smem, stream>>>(p);                                   \
+    } while (0)
 #define RS_LAUNCH_BWD(VL_, DROP_)                                                                                       \
     do {                                                                                                                \
-        RS_CUDA_OK(cudaFuncSetAttribute(rec_bwd_pair_kernel<VL_, DROP_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
-        rec_bwd_pair_kernel<VL_, DROP_><<<grid, NUM_THREADS, smem, stream>>>(p);                                        \
+        if (recompute) RS_LAUNCH_BWD_R(VL_, DROP_, true); else RS_LAUNCH_BWD_R(VL_, DROP_, false);                       \
     } while (0)
     if (lengths) { if (p.drop_bits) RS_LAUNCH_BWD(true, true); else RS_LAUNCH_BWD(true, false); }
     else { if (p.drop_bits) RS_LAUNCH_BWD(false, true); else RS_LAUNCH_BWD(false, false); }
 #undef RS_LAUNCH_BWD
+#undef RS_LAUNCH_BWD_R
     count_launch();
     RS_CUDA_OK(cudaGetLastError());
     return 0;

@@ -5,6 +5,7 @@ Per layer:   layer 0: fused K=2 input projection inside the recurrence kernel
                       with split (hi + lo) weights below 1024 traces: P = X W_ih^T + b by rs_blk_gemm_nt, then the recurrence
              recurrence forward                  rs_rec_fwd_bf16  (persistent CTA pairs, W_hh resident in shared memory)
 backward:    recurrence backward (BPTT)          rs_rec_bwd_bf16  -> dG (r | z | n | hn gate gradients); W_hn h recomputed
+                                                 layer 0 (I <= 2, unsplit): rs_rec_bwd_bf16_recompute, r, z, n recomputed too
              dW_ih, dW_hh, bias gradients        rs_blk_wgrad     (one launch per layer, 12 roles over dG)
              dX     = dG[r,z,n] W_ih             rs_blk_gemm_nt / rs_blk_gemm_nt_drop (x the dropout mask of the layer input)
 All per-timestep activations stay in the tile-major bf16 layout (roomslam_b200/layout.py); master weights and
@@ -36,6 +37,13 @@ def x_col(i: int, k: int) -> int:
 
 def x_steps(I: int) -> int:
     return (3 * I + 2 + 15) // 16
+
+
+def recompute_gates(padded_in: bool, split: int, I: int) -> bool:
+    """Layer 0 with unsplit weights and at most 2 inputs saves no gates: its backward kernel replays the forward MMA and
+    gets r, z and n bit for bit (rs_rec_bwd_bf16_recompute), instead of writing and reading 12 bytes per trace, step and
+    hidden unit pair of directions."""
+    return not padded_in and not split and I <= 2
 
 
 def _check_x_inputs(I: int):
@@ -185,7 +193,8 @@ class GRULayerBF16Fn(torch.autograd.Function):
             out_drop = L.empty_tm(B, T, 2 * H, dev, zero_pads=False) if drop is not None else None
             d_bits, d_scale = drop if drop is not None else (None, None)
             h_n = torch.empty(2, B, H, device=dev)
-            gates = torch.empty(tiles, T, 2, 48, L.TILE, 8, device=dev, dtype=torch.bfloat16) if need_grad else None   # r | z | n
+            recompute = recompute_gates(padded_in, split, Il)
+            gates = torch.empty(tiles, T, 2, 48, L.TILE, 8, device=dev, dtype=torch.bfloat16) if need_grad and not recompute else None   # r | z | n
             rec_flops = 2.0 * B * T * 2 * 3 * H * H
             X = None
             if not padded_in:
@@ -212,6 +221,7 @@ class GRULayerBF16Fn(torch.autograd.Function):
                 del P
                 saved_in = X
         ctx.meta = (padded_in, B, T, Il, split)
+        ctx.recompute = recompute
         ctx.drop = drop
         ctx.lengths = lengths
         # save_for_backward (not ctx attributes): `out` is an OUTPUT of this node; holding it in a plain attribute
@@ -226,7 +236,7 @@ class GRULayerBF16Fn(torch.autograd.Function):
     def backward(ctx, d_out, d_h_n):
         padded_in, B, T, Il, split = ctx.meta
         out, gates, saved_in, whhT_img, wt_dgrad, whh_img, b_hn = ctx.saved_tensors
-        if gates is None:
+        if gates is None and not ctx.recompute:
             raise RuntimeError("GRULayerBF16Fn: forward ran without saving activations (nothing required grad)")
         dev = out.device
         st = torch.cuda.current_stream(dev).cuda_stream
@@ -237,8 +247,14 @@ class GRULayerBF16Fn(torch.autograd.Function):
             dG = torch.empty(tiles, T + 2, 8 * H // 8, L.TILE, 8, device=dev, dtype=torch.bfloat16)
             with ktime("rec_bwd_pair_kernel", 2.0 * B * T * 2 * 3 * H * H):
                 d_bits, d_scale = ctx.drop if (ctx.drop is not None and ctx.mask_d_out) else (None, None)
-                _lib.call("rs_rec_bwd_bf16", _p(d_out), _p(d_h_n), _p(gates), _p(out), _p(whhT_img), _p(whh_img), whh_img.shape[1],
-                          _p(b_hn), _p(dG), _p(ctx.lengths), _p(d_bits), _p(d_scale), split, B, T, st)
+                if ctx.recompute:
+                    xpack = torch.empty(tiles, T, L.TILE, 8, device=dev, dtype=torch.bfloat16)
+                    _lib.call("rs_rec_bwd_bf16_recompute", _p(d_out), _p(d_h_n), _p(saved_in), Il, _p(xpack), _p(out), _p(whhT_img),
+                              _p(whh_img), whh_img.shape[1], _p(b_hn), _p(dG), _p(ctx.lengths), _p(d_bits), _p(d_scale), B, T, st)
+                    del xpack
+                else:
+                    _lib.call("rs_rec_bwd_bf16", _p(d_out), _p(d_h_n), _p(gates), _p(out), _p(whhT_img), _p(whh_img), whh_img.shape[1],
+                              _p(b_hn), _p(dG), _p(ctx.lengths), _p(d_bits), _p(d_scale), split, B, T, st)
             dW_ih, dW_hh, db_ih, db_hh, d_xin = grads_from_dG_128(dG, out, saved_in, padded_in, B, T, Il, split, wt_dgrad,
                                                                   ctx.in_drop, padded_in and ctx.needs_input_grad[0])
             dW_ih = dW_ih[:, :Il].contiguous() if not padded_in else dW_ih
